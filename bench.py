@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
     python bench.py --impl reference ...                     (the reference's CPU path: the oracle)
+    python bench.py ... --dump-outputs DIR                   (also write the outputs of the last timed step, to compare two builds)
 
 Workload (BASELINE.json configs[3]): synthetic 1024x1024 = 1 048 576 columns x 60 levels per GPU from
 the seeded CONUS-like convective domain of kid_b200/synth.py (about 30 % cloudy columns), dt = 10 s.
@@ -21,6 +22,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -100,6 +102,7 @@ class ClockSampler(threading.Thread):
         if self.proc is not None:
             try:
                 self.proc.terminate()
+                self.proc.wait(timeout=10)         # reaped here: no defunct nvidia-smi outlives the run
             except Exception:
                 pass
         inside = [r for t, r in self.rows if self.t0 is not None and self.t0 <= t <= (self.t1 or 1e99)]
@@ -122,6 +125,8 @@ def cpu_reference_run(ncol, steps, warmup, nthreads, col0=0):
     """The reference's CPU path (the C++ restatement under oracle/: no Fortran compiler exists here)
     on `ncol` columns of the bench domain, all host threads.  Returns (column-steps/s, ms/step, init_s)."""
     from kid_b200 import synth
+    # the oracle keeps its collection tables between runs; the tree may be read-only, so they go to a per-user temporary directory
+    os.environ.setdefault("KOR_CACHE_DIR", os.path.join(tempfile.gettempdir(), "kid_b200_oracle_cache_%d" % os.getuid()))
     from oracle.oracle import Oracle
     o = Oracle(set_Nc=100.0, iiwarm=False, l_sediment=True, nthreads=nthreads)
     st, p, dz = synth.make_domain(ncol, nz=NZ, col0=col0, nx=1024)
@@ -162,6 +167,23 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_COLUMNS = 24576                 # --dump-outputs: 2176 bytes a column (nine fields of 60 levels + 4 precipitation amounts) = 53.5 MB
+DUMP_SEED = 20261018
+
+
+def dump_outputs(out_dir, st, ppt, ncol):
+    """What the last timed step returned to the caller: the nine state fields (NZ, ncol) and the surface precipitation of the step
+    (4, ncol), as <out_dir>/<name>.npy in float32.  A domain of more than DUMP_COLUMNS columns is cut to a seeded sample of
+    columns (sorted, the same in every run), so that two builds of the project can be compared output for output."""
+    import torch
+    from kid_b200.kidmp import FIELDS
+    cols = np.arange(ncol) if ncol <= DUMP_COLUMNS else np.sort(np.random.default_rng(DUMP_SEED).choice(ncol, DUMP_COLUMNS, replace=False))
+    idx = torch.from_numpy(cols).to(ppt.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in [(k, st[k]) for k in FIELDS] + [("ppt", ppt)]:
+        np.save(os.path.join(out_dir, name + ".npy"), a.index_select(1, idx).cpu().numpy())
+
+
 def make_resident_domain(synth, ncol, col0, nx, dev, slab=1 << 20):
     """kid_b200/synth.py domain [col0, col0+ncol) on the device, generated slab by slab into preallocated tensors."""
     import torch
@@ -190,6 +212,8 @@ def main():
     ap.add_argument("--cpu-columns", type=int, default=262144, help="columns of the bounded CPU sample")
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned on rank 0 (state fields and "
+                    "surface precipitation, a fixed sample of %d columns) as DIR/<name>.npy" % DUMP_COLUMNS)
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "kidmp" else args.warmup
 
@@ -257,6 +281,8 @@ def main():
     ev[args.steps].record()
     torch.cuda.synchronize()
     sampler.mark(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, st, ppt, ncol)
     diag = torch.from_numpy(th.diag()).to(dev)          # the 8 domain sums accumulated over the K steps
     if world > 1:
         dist.all_reduce(diag)                           # the only collective: 64 bytes of diagnostics
