@@ -188,6 +188,9 @@ int kidmp_mp_gt_driver_aero(kidmp_handle* h, const kidmp_wrf_fields* w, const ki
  * "simple": 1 (default) = a column that holds no graupel and in which no fall speed can cross the thinnest layer in one step
  *   (every sub-step count of M:3242 is 0 or 1) skips the column kernel that settles those counts; 0 = every cloudy column
  *   goes through it.  KIDMP_SIMPLE.
+ * "classes": 1 (default) = every busy cell goes to the cell kernel specialised for its species set and temperature class;
+ *   0 = every busy cell goes to the general one.  The specialised kernels compute the same bits (tests/test_regimes.py): this
+ *   is their reference, not a tuning choice.
  * "lanes" (1..8, default 1, KIDMP_LANES), "lane_min" (columns, KIDMP_LANE_MIN), "stagger", "cell_blocks": a step over at least
  *   2 x lane_min columns is cut into launches that run side by side on `lanes` work sets and streams.  Measured on the
  *   bench domain: no gain over one lane (profiles/r02_ncu_step_kernels.md), so the default is one.

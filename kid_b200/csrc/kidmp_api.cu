@@ -81,9 +81,10 @@ struct kidmp_handle {
   // the same ("graphs" option, KIDMP_GRAPHS; KIDMP_GRAPH_MAX: largest domain): a small domain is launch-bound (fifteen kernels of
   // a few microseconds: 0.297 -> 0.277 ms for one column), the 1 048 576-column step loses its launch gaps (3.45 -> 3.425 ms)
   int graphs = 1; long graph_max_cols = 1L << 24;
-  struct StepGraph { cudaGraphExec_t exec = nullptr; StepArgs args{}; long key[6] = {}; long launches = 0; };
+  struct StepGraph { cudaGraphExec_t exec = nullptr; StepArgs args{}; long key[7] = {}; long launches = 0; };
   StepGraph graph_cache[8]; int graph_next = 0;        // a few steps at a time: the three rotating buffers of kidmp_step's pipeline, resident state, a caller's arrays
   int simple = 1;                                         // "simple" option: columns without sub-steps skip k_carries (kidmp_cells.cuh)
+  int classes = 1;                                        // "classes" option: 0 sends every busy cell to the general cell kernel (tests)
   int l2_window = 1;                                      // "l2_window" option: the cell kernels that gather from the tables carry the window
   int stagger = 0;                                        // "stagger" option: see launch_step
   int lanes_used = 1;                                     // work sets of the last step
@@ -443,7 +444,10 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
   }
   // One lane: replay the captured graph of this very step (all its chunks), or capture it now.
   const bool graphable = h->graphs && !h->timing && nchunks <= 64 && nl == 1 && a0.ncol <= h->graph_max_cols;
-  const long gkey[6] = {(long)(size_t)h->ws[0].d_scratch, h->ws[0].cols, (long)h->ws[0].nz, (long)h->simple, (long)(size_t)h->d_partial, (long)h->l2_window * 2 + chunk * 4};
+  // (a handle setting that a captured launch reads belongs in the key: a replay after the setting changed would run the old one.
+  // "stagger" and "cell_blocks" are not in it: they act only when a step runs on several lanes, which is never captured)
+  const long gkey[7] = {(long)(size_t)h->ws[0].d_scratch, h->ws[0].cols, (long)h->ws[0].nz, (long)h->simple, (long)(size_t)h->d_partial,
+                        (long)h->l2_window * 2 + chunk * 4, (long)h->classes};
   kidmp_handle::StepGraph* hit = nullptr;
   if (graphable)
     for (auto& g : h->graph_cache)
@@ -500,6 +504,7 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
     a.busy = (unsigned*)w.d_colwork; a.colint = w.d_colwork + 8 * w.cols; a.sub_list = w.d_colwork + 16 * w.cols; a.colvmax = w.d_colwork + 17 * w.cols;
     a.ws = w.d_ws; a.ws_cols = w.cols; a.n0a = w.d_n0a;
     a.coldiag = w.d_coldiag; a.diag_partial = h->d_partial + (size_t)ci * DIAG_BLOCKS * KIDMP_NDIAG; a.nsm = h->nsm; a.no_simple = h->simple ? 0 : 1;
+    a.no_classes = h->classes ? 0 : 1;
     // second stream of the launch; in timing mode everything runs on one stream, one kernel after the other
     const bool serial = h->timing == 1;
     cudaStream_t x = serial ? cs : w.aux;
@@ -1653,6 +1658,7 @@ int kidmp_set_option(kidmp_handle* h, const char* name, int value) {
   }
   if (!strcmp(name, "graphs")) { h->graphs = value != 0; return 0; }
   if (!strcmp(name, "simple")) { h->simple = value != 0; return 0; }
+  if (!strcmp(name, "classes")) { h->classes = value != 0; return 0; }
   if (!strcmp(name, "l2_window")) { h->l2_window = value != 0; return 0; }
   if (!strcmp(name, "stagger")) { h->stagger = value != 0; return 0; }
   if (!strcmp(name, "cell_blocks")) {

@@ -130,7 +130,7 @@ __global__ void __launch_bounds__(64) k_cell_offsets(StepArgs a) {
   const int t = threadIdx.x;
   const bool iiwarm = ck.iiwarm != 0;
   s_n[t] = a.cell_hist[t];
-  s_kc[t] = cell_kernel_class((unsigned)t & 31u, (t >> 5) != 0, iiwarm);
+  s_kc[t] = a.no_classes ? KC_FULL : cell_kernel_class((unsigned)t & 31u, (t >> 5) != 0, iiwarm);
   __syncthreads();
   int start = 0;
   for (int j = 0; j < 64; ++j) if (s_kc[j] < s_kc[t] || (s_kc[j] == s_kc[t] && j < t)) start += s_n[j];

@@ -171,6 +171,7 @@ struct StepArgs {
   const float* w;                        // [nz][ld] IN
   int nsm;                     // SMs of the device
   int no_simple;               // 1: every cloudy column goes through the counts of k_carries ("simple" option off: for A/B runs)
+  int no_classes;              // 1: every busy cell goes to k_cells<KC_FULL> ("classes" option off: the class kernels' reference)
 };
 
 // device tables (kidmp_tables.cuh fills them)

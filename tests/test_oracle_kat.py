@@ -357,18 +357,8 @@ def test_saturation_over_ice_not_above_liquid():
 def test_cell_class_rule_covers_every_species_set():
     """The rule of cell_kernel_class (kid_b200/csrc/kidmp_column.cuh): every (species set, cold, iiwarm) combination goes to a
     class whose kernel may hold those species (CellTraits of kidmp_cells.cuh)."""
-    QC, QI, QR, QS, QG = 1, 2, 4, 8, 16
+    from regimes import QC, QI, QR, QS, QG, kernel_class as rule
     allowed = {"WARM": QC | QR, "ICE": QI | QS, "MIXNR": QC | QI | QS | QG, "FULL": 31}
-
-    def rule(sp, cold, iiwarm):
-        ice = bool(sp & (QI | QS | QG))
-        if iiwarm:
-            return "FULL" if ice else "WARM"
-        if not cold and not ice:
-            return "WARM"
-        if cold and not (sp & (QC | QR | QG)):
-            return "ICE"
-        return "FULL" if sp & QR else "MIXNR"
     for sp in range(32):
         for cold in (False, True):
             for iiwarm in (False, True):
