@@ -149,8 +149,10 @@ typedef struct kidmp_kid_columns {
 } kidmp_kid_columns;
 int kidmp_kid_interface(kidmp_handle* h, const kidmp_kid_columns* c, float dt, float p0, float r_on_cp);
 
-/* The WRF / MPAS-facing entry: what mp_gt_driver (M:806-1143) does for a tile of ni x nj columns of nk levels.
- * 3-D arrays are WRF's (i,k,j) order, a[i + ni*(k + nk*j)]; 2-D arrays are (i,j), a[i + ni*j].  INOUT: the nine
+/* The WRF / MPAS-facing entry: what mp_gt_driver (M:806-1143) does for ni x nj columns of nk levels.
+ * ni, nk, nj are the MEMORY dimensions of the arrays.  3-D arrays are WRF's (i,k,j) order, a[i + ni*(k + nk*j)]; 2-D arrays
+ * are (i,j), a[i + ni*j].  kidmp_mp_gt_driver steps the whole box; a host whose arrays carry halo points or spare levels
+ * (WRF and MPAS allocate kme = kte + 1) names the cells to step with kidmp_mp_gt_driver_tile below.  INOUT: the nine
  * prognostic fields with potential temperature `th` (T = th*pii goes into the step, th = T/pii comes back, M:941,
  * M:1022); IN: pii (Exner function), p, dz (per-column layer depths, M:944).  RAINNC / SNOWNC / GRAUPELNC are
  * accumulated, RAINNCV / SNOWNCV / GRAUPELNCV / SR overwritten (M:991-1003); the snow and graupel pairs may be NULL
@@ -176,6 +178,26 @@ typedef struct kidmp_wrf_aerosols {
   const float* nwfa2d;
 } kidmp_wrf_aerosols;
 int kidmp_mp_gt_driver_aero(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_aerosols* ae, float dt_in);
+
+/* The same step for one tile inside the memory box of kidmp_wrf_fields, in place: w->ni, w->nk, w->nj are the memory
+ * dimensions ime-ims+1, kme-kms+1, jme-jms+1, and the tile is given by 0-based offsets and extents,
+ *   i0 = its-ims, ni = ite-its+1,  k0 = kts-kms, nk = kte-kts+1,  j0 = jts-jms, nj = jte-jts+1.
+ * Tile cell (i,k,j) is memory cell (i0+i, k0+k, j0+j); its 2-D cell is (i0+i, j0+j).  The call reads and writes only cells
+ * of the tile box: halo points, the spare top level and every other cell of every array are neither read nor written, so
+ * the tiles of one patch may run at the same time (one handle each).  A tile outside the memory box, nk < 2 or an empty
+ * extent is rejected (non-zero return, kidmp_last_error) before anything is copied or launched.  ae == NULL is
+ * is_aerosol_aware = .false. (kidmp_mp_gt_driver), else kidmp_mp_gt_driver_aero.  Everything else as those two:
+ * radii only with all three re_* given, optional snow and graupel accumulators, the handle's process-rate buffer on
+ * the non-aerosol path, a multi-device handle steps the tile on its first device.
+ * kidmp_mp_gt_driver_tile takes HOST arrays and returns when they hold the result; only the tile rows travel.
+ * kidmp_mp_gt_driver_tile_device takes DEVICE arrays of the handle's GPU and is enqueued on `stream` (a cudaStream_t passed
+ * as void*; NULL = the handle's stream) without synchronising; the step runs on the handle's resident state, ordered against
+ * kidmp_diag and the next call by an event.  It needs a single-device handle. */
+typedef struct kidmp_wrf_tile { int i0, ni, k0, nk, j0, nj; } kidmp_wrf_tile;
+int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const kidmp_wrf_aerosols* ae,
+                            float dt_in);
+int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t,
+                                   const kidmp_wrf_aerosols* ae, float dt_in, void* stream);
 
 /* Tuning knobs; results do not depend on them.
  * "chunk": columns per launch of the step kernels (default 1 048 576, or the KIDMP_CHUNK environment variable): the work
@@ -206,8 +228,9 @@ int kidmp_set_option(kidmp_handle* h, const char* name, int value);
 /* Multi-device handles (kidmp_config::ndev > 1).  kidmp_step, kidmp_kid_interface and the resident-state calls cut the
  * host arrays into one contiguous column range per device (columns are independent, I:54: no exchange on the data path) and
  * run the devices side by side; results are bit-identical to a single-device handle, column by column.  kidmp_column and
- * kidmp_mp_gt_driver run on the first device.  The entry points that take or return DEVICE pointers (kidmp_step_device,
- * kidmp_set_rates_buffer, kidmp_device_state, kidmp_stream) need a single-device handle.  NCCL (libnccl.so.2, or the file
+ * kidmp_mp_gt_driver[_aero,_tile] run on the first device.  The entry points that take or return DEVICE pointers
+ * (kidmp_step_device, kidmp_mp_gt_driver_tile_device, kidmp_set_rates_buffer, kidmp_device_state, kidmp_stream) need a
+ * single-device handle.  NCCL (libnccl.so.2, or the file
  * named by the KIDMP_NCCL_LIB environment variable) is loaded when such a handle is created, not before. */
 int kidmp_num_devices(const kidmp_handle* h);
 

@@ -1525,116 +1525,211 @@ int kidmp_diag(kidmp_handle* h, double out[KIDMP_NDIAG]) {
   return 0;
 }
 
-// mp_gt_driver, M:806-1143 (see kidmp_wrf.cuh)
-static int wrf_driver(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_aerosols* ae, float dt_in);
-int kidmp_mp_gt_driver(kidmp_handle* h, const kidmp_wrf_fields* w, float dt_in) { return wrf_driver(h, w, nullptr, dt_in); }
+// mp_gt_driver, M:806-1143 (see kidmp_wrf.cuh).  Every entry is one tile of the caller's memory box; the packed entries
+// step the whole box.  One set of kernels serves both sides: the device entry runs them on the caller's arrays, the host
+// entry stages the tile rows through the pinned buffer and runs them on the packed tile (a box of its own).
+int kidmp_mp_gt_driver(kidmp_handle* h, const kidmp_wrf_fields* w, float dt_in) {
+  if (!h) return 1;
+  if (!w) return fail(h, "mp_gt_driver: null argument");
+  const kidmp_wrf_tile t{0, w->ni, 0, w->nk, 0, w->nj};
+  return kidmp_mp_gt_driver_tile(h, w, &t, nullptr, dt_in);
+}
 int kidmp_mp_gt_driver_aero(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_aerosols* ae, float dt_in) {
   if (!h) return 1;
-  if (!ae || !ae->nc || !ae->nwfa || !ae->nifa || !ae->w) return fail(h, "mp_gt_driver_aero: null aerosol array");
-  return wrf_driver(h, w, ae, dt_in);
-}
-static int wrf_driver(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_aerosols* ae, float dt_in) {
-  if (!h) return 1;
-  if (h->multi) return wrf_driver(h->multi->dev[0], w, ae, dt_in) ? fail(h, "%s", h->multi->dev[0]->err.c_str()) : 0;   // one tile, one device
+  if (!ae) return fail(h, "mp_gt_driver_aero: null aerosol array");
   if (!w) return fail(h, "mp_gt_driver: null argument");
-  if (w->ni < 1 || w->nj < 1 || w->nk < 2) return fail(h, "mp_gt_driver: bad dimensions %d x %d x %d", w->ni, w->nk, w->nj);
-  float* const io[9] = {w->qv, w->qc, w->qi, w->qr, w->qs, w->qg, w->ni_, w->nr, w->th};      // state-field order
-  for (int q = 0; q < 9; ++q) if (!io[q]) return fail(h, "mp_gt_driver: null field %d", q);
-  if (!w->pii || !w->p || !w->dz || !w->rainnc || !w->rainncv || !w->sr) return fail(h, "mp_gt_driver: null array");
-  if (!(dt_in > 0.f)) return fail(h, "mp_gt_driver: dt must be positive");
-  const bool radii = w->re_cloud && w->re_ice && w->re_snow;
-  const long ncol = (long)w->ni * w->nj;
-  if (kidmp_state_alloc(h, ncol, w->nk)) return 1;
-  DevGuard guard_(h->device);
-  const size_t n = (size_t)ncol * w->nk, n2 = (size_t)ncol;
-  // device staging: 12 three-dimensional inputs, the per-column dz in step layout, 3 radii, 7 two-dimensional arrays
-  const size_t dfloats = (12 + 1 + 3) * n + 7 * n2;
-  if (h->kid_floats < dfloats) {
-    if (h->d_kid) cudaFree(h->d_kid);
-    h->d_kid = nullptr; h->kid_floats = 0;
-    CK(h, cudaMalloc((void**)&h->d_kid, dfloats * 4));
-    h->kid_floats = dfloats;
+  const kidmp_wrf_tile t{0, w->ni, 0, w->nk, 0, w->nj};
+  return kidmp_mp_gt_driver_tile(h, w, &t, ae, dt_in);
+}
+
+// Every check of a tile call, before anything is copied or launched: a rejected call leaves every array as it was.
+static int wrf_check(kidmp_handle* h, const char* who, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t,
+                     const kidmp_wrf_aerosols* ae, float dt_in) {
+  if (!w || !t) return fail(h, "%s: null argument", who);
+  if (w->ni < 1 || w->nj < 1 || w->nk < 2) return fail(h, "%s: bad memory dimensions %d x %d x %d", who, w->ni, w->nk, w->nj);
+  if (t->ni < 1 || t->nj < 1 || t->nk < 2 || t->nk > 256)
+    return fail(h, "%s: bad tile extents %d x %d x %d (ni, nj >= 1, 2 <= nk <= 256)", who, t->ni, t->nk, t->nj);
+  if (t->i0 < 0 || t->k0 < 0 || t->j0 < 0 || (long)t->i0 + t->ni > w->ni || (long)t->k0 + t->nk > w->nk || (long)t->j0 + t->nj > w->nj)
+    return fail(h, "%s: tile i %d+%d, k %d+%d, j %d+%d does not lie inside the memory box %d x %d x %d", who, t->i0, t->ni,
+                t->k0, t->nk, t->j0, t->nj, w->ni, w->nk, w->nj);
+  if (t->nj > 65535) return fail(h, "%s: tile nj = %d, at most 65535", who, t->nj);
+  const float* const io[9] = {w->qv, w->qc, w->qi, w->qr, w->qs, w->qg, w->ni_, w->nr, w->th};
+  for (int q = 0; q < 9; ++q) if (!io[q]) return fail(h, "%s: null field %d", who, q);
+  if (!w->pii || !w->p || !w->dz || !w->rainnc || !w->rainncv || !w->sr) return fail(h, "%s: null array", who);
+  if (!(dt_in > 0.f)) return fail(h, "%s: dt must be positive", who);
+  if (ae) {
+    if (!ae->nc || !ae->nwfa || !ae->nifa || !ae->w) return fail(h, "%s: null aerosol array", who);
+    if (h->d_rates || h->rates_on) return fail(h, "%s: the process-rate buffer is not available in an aerosol-aware step", who);
   }
-  const size_t hfloats = 12 * n + 7 * n2;            // one pinned buffer, one copy each way (as kidmp_kid_interface)
+  return 0;
+}
+
+static int ensure_dev(kidmp_handle* h, float** p, size_t* have, size_t need) {
+  if (*have >= need) return 0;
+  if (*p) cudaFree(*p);
+  *p = nullptr; *have = 0;
+  CK(h, cudaMalloc((void**)p, need * 4));
+  *have = need;
+  return 0;
+}
+
+// The kernels of one call on device arrays that a.t addresses, on stream s: the tile into the resident planes, the step,
+// the planes back into the tile, the accumulators.  ae4: nc nwfa nifa w of an aerosol-aware call (else NULL), nwfa2d or NULL,
+// with their planes in h->d_aero.  The caller sets a.t, the tile's arrays and a.dz_col; a.f, a.p, a.ppt are set here.
+static int wrf_kernels(kidmp_handle* h, WrfArgs& a, float* const* ae4, const float* nwfa2d, float dt_in, cudaStream_t s) {
+  const long ncol = (long)a.t.ni * a.t.nj;
+  const size_t n = (size_t)ncol * a.t.nk;
+  if (ae4 && ensure_wev_table(h)) return 1;
+  for (int q = 0; q < KIDMP_NFIELDS; ++q) a.f[q] = field_ptr(h, q);
+  a.p = field_ptr(h, KIDMP_NFIELDS);
+  a.ppt = h->d_ppt;
+  CK(h, cudaStreamWaitEvent(s, h->ev_done, 0));         // the resident planes and staging may serve a step on another stream
+  const dim3 b(128), g((unsigned)((a.t.ni + 127) / 128), (unsigned)a.t.nk, (unsigned)a.t.nj);
+  const dim3 g2(g.x, 1, g.z);
+  WrfBox t2 = a.t;                                      // the (i,j) arrays: a box of one level
+  t2.nk = 1; t2.nk_m = 1; t2.k0 = 0;
+  k_wrf_gather<<<g, b, 0, s>>>(a);
+  if (s == h->stream) CK(h, cudaEventRecord(h->ev0, s));
+  StepArgs sa = resident_args(h, dt_in);
+  sa.dz_col = a.dz_col;
+  float* const d_ae = h->d_aero;                         // aerosol-aware run: 4 planes and the nwfa2d plane
+  if (ae4) {
+    for (int q = 0; q < 4; ++q) k_ikj_planes<<<g, b, 0, s>>>(ae4[q], d_ae + n * q, a.t, 1);
+    if (nwfa2d) k_ikj_planes<<<g2, b, 0, s>>>(const_cast<float*>(nwfa2d), d_ae + 4 * n, t2, 1);   // (read only)
+    sa.nc = d_ae; sa.nwfa = d_ae + n; sa.nifa = d_ae + 2 * n; sa.w = d_ae + 3 * n;
+    a.nc_plane = sa.nc;
+    h->launches += nwfa2d ? 5 : 4;
+  }
+  if (launch_step(h, sa, s)) return 1;
+  if (ae4 && nwfa2d) { k_nwfa_surface<<<(unsigned)((ncol + 255) / 256), 256, 0, s>>>(sa.nwfa, d_ae + 4 * n, ncol, dt_in); ++h->launches; }   // M:1001
+  if (s == h->stream) CK(h, cudaEventRecord(h->ev1, s));
+  k_wrf_scatter<<<g, b, 0, s>>>(a, h->kc.Nt_c);
+  if (ae4) {
+    for (int q = 0; q < 3; ++q) k_ikj_planes<<<g, b, 0, s>>>(ae4[q], d_ae + n * q, a.t, 0);
+    h->launches += 3;
+  }
+  k_wrf_accumulate<<<(unsigned)((ncol + 255) / 256), 256, 0, s>>>(a);
+  h->launches += 3;
+  CK(h, cudaGetLastError());
+  CK(h, cudaEventRecord(h->ev_done, s));                 // the next call or kidmp_diag reuses the planes, maybe on another stream
+  return 0;
+}
+
+// the tile rows of one array between the caller's memory box `mem` (ni_m x nk_m x ...) and the packed tile `tile`.  A row is
+// ni floats at memory (i0, k0+k, j0+j); rows that follow each other in memory (a tile as wide as the box) move as one block.
+// A 2-D array is the box with nk = nk_m = 1, k0 = 0.
+static void tile_rows(float* tile, float* mem, const kidmp_wrf_tile& t, long ni_m, long nk_m, bool to_tile) {
+  long run = t.ni;
+  int nkr = t.nk, njr = t.nj;
+  if (t.ni == ni_m) { run *= t.nk; nkr = 1; if (t.nk == nk_m) { run *= t.nj; njr = 1; } }
+  for (int j = 0; j < njr; ++j)
+    for (int k = 0; k < nkr; ++k) {
+      float* const m = mem + t.i0 + ni_m * (t.k0 + k + nk_m * (long)(t.j0 + j));
+      float* const p = tile + ((long)k + (long)t.nk * j) * t.ni;
+      if (to_tile) memcpy(p, m, run * 4); else memcpy(m, p, run * 4);
+    }
+}
+
+int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const kidmp_wrf_aerosols* ae,
+                            float dt_in) {
+  if (!h) return 1;
+  if (h->multi) return kidmp_mp_gt_driver_tile(h->multi->dev[0], w, t, ae, dt_in) ? fail(h, "%s", h->multi->dev[0]->err.c_str()) : 0;   // one tile, one device
+  if (wrf_check(h, ae ? "mp_gt_driver_aero" : "mp_gt_driver", w, t, ae, dt_in)) return 1;
+  const bool radii = w->re_cloud && w->re_ice && w->re_snow;
+  const long ncol = (long)t->ni * t->nj;
+  if (kidmp_state_alloc(h, ncol, t->nk)) return 1;
+  DevGuard guard_(h->device);
+  const size_t n = (size_t)ncol * t->nk, n2 = (size_t)ncol;
+  // device staging: 12 three-dimensional inputs, the per-column dz in step layout, 3 radii, 7 two-dimensional arrays
+  if (ensure_dev(h, &h->d_kid, &h->kid_floats, (12 + 1 + 3) * n + 7 * n2)) return 1;
+  // one pinned buffer, one copy each way (as kidmp_kid_interface): the tile of the 12 inputs, 7 accumulators, 4 aerosol arrays + nwfa2d
+  const size_t hfloats = 12 * n + 7 * n2 + (ae ? 4 * n + n2 : 0);
   if (h->h_kid_floats < hfloats) {
     if (h->h_kid) cudaFreeHost(h->h_kid);
     h->h_kid = nullptr; h->h_kid_floats = 0;
     CK(h, cudaHostAlloc((void**)&h->h_kid, hfloats * 4, cudaHostAllocDefault));
     h->h_kid_floats = hfloats;
   }
-  WrfArgs a{};
-  a.ni = w->ni; a.nk = w->nk; a.nj = w->nj;
+  // aerosol-aware: planes (4 n + n2) for wrf_kernels, then the packed tile of the 4 arrays and nwfa2d
+  if (ae && ensure_dev(h, &h->d_aero, &h->aero_floats, 2 * (4 * n + n2))) return 1;
+  const long ni_m = w->ni, nk_m = w->nk;
+  const kidmp_wrf_tile t2{t->i0, t->ni, 0, 1, t->j0, t->nj};
+  CK(h, cudaStreamWaitEvent(h->stream, h->ev_done, 0));  // (the device staging may still serve a call on another stream)
+  float* const io[9] = {w->qv, w->qc, w->qi, w->qr, w->qs, w->qg, w->ni_, w->nr, w->th};      // state-field order
   const float* const in3[12] = {w->qv, w->qc, w->qi, w->qr, w->qs, w->qg, w->ni_, w->nr, w->th, w->pii, w->p, w->dz};
-  for (int q = 0; q < 12; ++q) memcpy(h->h_kid + n * q, in3[q], n * 4);
+  for (int q = 0; q < 12; ++q) tile_rows(h->h_kid + n * q, const_cast<float*>(in3[q]), *t, ni_m, nk_m, true);   // (read only)
+  float* const h_2d = h->h_kid + n * 12;
+  float* const acc[7] = {w->rainnc, w->rainncv, w->sr, w->snownc, w->snowncv, w->graupelnc, w->graupelncv};
+  for (int q = 0; q < 7; ++q) if (acc[q]) tile_rows(h_2d + n2 * q, acc[q], t2, ni_m, 1, true);
+  float* const h_ae = h_2d + 7 * n2;
+  if (ae) {
+    const float* const in4[4] = {ae->nc, ae->nwfa, ae->nifa, ae->w};
+    for (int q = 0; q < 4; ++q) tile_rows(h_ae + n * q, const_cast<float*>(in4[q]), *t, ni_m, nk_m, true);
+    if (ae->nwfa2d) tile_rows(h_ae + 4 * n, const_cast<float*>(ae->nwfa2d), t2, ni_m, 1, true);
+  }
+  // on the device the packed tile is a memory box of its own
+  WrfArgs a{};
+  a.t = WrfBox{t->ni, t->nk, t->nj, 0, 0, 0, t->ni, t->nk};
   for (int q = 0; q < 9; ++q) a.a3[q] = h->d_kid + n * q;
   a.pii = h->d_kid + n * 9; a.p3 = h->d_kid + n * 10; a.dz3 = h->d_kid + n * 11;
   a.dz_col = h->d_kid + n * 12;
   float* const d_re = h->d_kid + n * 13;
   if (radii) { a.re_cloud = d_re; a.re_ice = d_re + n; a.re_snow = d_re + 2 * n; }
   float* const d_2d = h->d_kid + n * 16;
-  float* const h_2d = h->h_kid + n * 12;
-  float* const acc[7] = {w->rainnc, w->rainncv, w->sr, w->snownc, w->snowncv, w->graupelnc, w->graupelncv};
-  for (int q = 0; q < 7; ++q) if (acc[q]) memcpy(h_2d + n2 * q, acc[q], n2 * 4);
   a.rainnc = d_2d; a.rainncv = d_2d + n2; a.sr = d_2d + 2 * n2;
   if (w->snownc && w->snowncv) { a.snownc = d_2d + 3 * n2; a.snowncv = d_2d + 4 * n2; }
   if (w->graupelnc && w->graupelncv) { a.graupelnc = d_2d + 5 * n2; a.graupelncv = d_2d + 6 * n2; }
-  for (int q = 0; q < KIDMP_NFIELDS; ++q) a.f[q] = field_ptr(h, q);
-  a.p = field_ptr(h, KIDMP_NFIELDS);
-  a.ppt = h->d_ppt;
+  float* const d_aet = ae ? h->d_aero + 4 * n + n2 : nullptr;
   CK(h, cudaMemcpyAsync(h->d_kid, h->h_kid, 12 * n * 4, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpyAsync(d_2d, h_2d, 7 * n2 * 4, cudaMemcpyHostToDevice, h->stream));
-  const dim3 b(128), g((unsigned)((w->ni + 127) / 128), (unsigned)w->nk, (unsigned)w->nj);
-  k_wrf_gather<<<g, b, 0, h->stream>>>(a);
-  CK(h, cudaEventRecord(h->ev0, h->stream));
-  StepArgs sa = resident_args(h, dt_in);
-  sa.dz_col = a.dz_col;
-  float* d_ae = nullptr;                                // aerosol-aware run: 4 (i,k,j) arrays, their 4 planes, nwfa2d
-  if (ae) {
-    if (sa.rates) return fail(h, "mp_gt_driver_aero: the process-rate buffer is not available in an aerosol-aware step");
-    if (ensure_wev_table(h)) return 1;
-    if (h->aero_floats < 8 * n + n2) {
-      if (h->d_aero) cudaFree(h->d_aero);
-      h->d_aero = nullptr; h->aero_floats = 0;
-      CK(h, cudaMalloc((void**)&h->d_aero, (8 * n + n2) * 4));
-      h->aero_floats = 8 * n + n2;
-    }
-    d_ae = h->d_aero;
-    const float* const in4[4] = {ae->nc, ae->nwfa, ae->nifa, ae->w};
-    for (int q = 0; q < 4; ++q) {
-      CK(h, cudaMemcpyAsync(d_ae + n * q, in4[q], n * 4, cudaMemcpyHostToDevice, h->stream));
-      k_ikj_planes<<<g, b, 0, h->stream>>>(d_ae + n * q, d_ae + n * (4 + q), w->ni, w->nk, w->nj, 1);
-    }
-    if (ae->nwfa2d) CK(h, cudaMemcpyAsync(d_ae + 8 * n, ae->nwfa2d, n2 * 4, cudaMemcpyHostToDevice, h->stream));
-    sa.nc = d_ae + 4 * n; sa.nwfa = d_ae + 5 * n; sa.nifa = d_ae + 6 * n; sa.w = d_ae + 7 * n;
-    a.nc_plane = sa.nc;
-    h->launches += 4;
-  }
-  if (launch_step(h, sa, h->stream)) return 1;
-  if (ae && ae->nwfa2d) { k_nwfa_surface<<<(unsigned)((ncol + 255) / 256), 256, 0, h->stream>>>(sa.nwfa, d_ae + 8 * n, ncol, dt_in); ++h->launches; }   // M:1001
-  CK(h, cudaEventRecord(h->ev1, h->stream));
-  k_wrf_scatter<<<g, b, 0, h->stream>>>(a, h->kc.Nt_c);
-  if (ae) {
-    float* const out3[3] = {ae->nc, ae->nwfa, ae->nifa};
-    for (int q = 0; q < 3; ++q) {
-      k_ikj_planes<<<g, b, 0, h->stream>>>(d_ae + n * q, d_ae + n * (4 + q), w->ni, w->nk, w->nj, 0);
-      CK(h, cudaMemcpyAsync(out3[q], d_ae + n * q, n * 4, cudaMemcpyDeviceToHost, h->stream));   // (synchronised with the stream below)
-    }
-    h->launches += 3;
-  }
-  k_wrf_accumulate<<<(unsigned)((ncol + 255) / 256), 256, 0, h->stream>>>(a);
-  h->launches += 3;
-  CK(h, cudaGetLastError());
+  if (ae) CK(h, cudaMemcpyAsync(d_aet, h_ae, (4 * n + n2) * 4, cudaMemcpyHostToDevice, h->stream));
+  float* const ae4[4] = {d_aet, d_aet + n, d_aet + 2 * n, d_aet + 3 * n};
+  if (wrf_kernels(h, a, ae ? ae4 : nullptr, ae && ae->nwfa2d ? d_aet + 4 * n : nullptr, dt_in, h->stream)) return 1;
   CK(h, cudaMemcpyAsync(h->h_kid, h->d_kid, 9 * n * 4, cudaMemcpyDeviceToHost, h->stream));
   float* const h_re = h->h_kid + n * 9;               // pii, p, dz slots of the pinned buffer are free again
   if (radii) CK(h, cudaMemcpyAsync(h_re, d_re, 3 * n * 4, cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaMemcpyAsync(h_2d, d_2d, 7 * n2 * 4, cudaMemcpyDeviceToHost, h->stream));
+  if (ae) CK(h, cudaMemcpyAsync(h_ae, d_aet, 3 * n * 4, cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
-  for (int q = 0; q < 9; ++q) memcpy(io[q], h->h_kid + n * q, n * 4);
-  if (radii) { memcpy(w->re_cloud, h_re, n * 4); memcpy(w->re_ice, h_re + n, n * 4); memcpy(w->re_snow, h_re + 2 * n, n * 4); }
-  memcpy(w->rainnc, h_2d, n2 * 4); memcpy(w->rainncv, h_2d + n2, n2 * 4); memcpy(w->sr, h_2d + 2 * n2, n2 * 4);
-  if (a.snownc) { memcpy(w->snownc, h_2d + 3 * n2, n2 * 4); memcpy(w->snowncv, h_2d + 4 * n2, n2 * 4); }
-  if (a.graupelnc) { memcpy(w->graupelnc, h_2d + 5 * n2, n2 * 4); memcpy(w->graupelncv, h_2d + 6 * n2, n2 * 4); }
+  for (int q = 0; q < 9; ++q) tile_rows(h->h_kid + n * q, io[q], *t, ni_m, nk_m, false);
+  if (radii) {
+    float* const re[3] = {w->re_cloud, w->re_ice, w->re_snow};
+    for (int q = 0; q < 3; ++q) tile_rows(h_re + n * q, re[q], *t, ni_m, nk_m, false);
+  }
+  for (int q = 0; q < 3; ++q) tile_rows(h_2d + n2 * q, acc[q], t2, ni_m, 1, false);
+  if (a.snownc) for (int q = 3; q < 5; ++q) tile_rows(h_2d + n2 * q, acc[q], t2, ni_m, 1, false);
+  if (a.graupelnc) for (int q = 5; q < 7; ++q) tile_rows(h_2d + n2 * q, acc[q], t2, ni_m, 1, false);
+  if (ae) {
+    float* const out3[3] = {ae->nc, ae->nwfa, ae->nifa};
+    for (int q = 0; q < 3; ++q) tile_rows(h_ae + n * q, out3[q], *t, ni_m, nk_m, false);
+  }
   return 0;
+}
+
+int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t,
+                                   const kidmp_wrf_aerosols* ae, float dt_in, void* stream) {
+  if (!h) return 1;
+  if (h->multi) return fail(h, "mp_gt_driver_tile_device: device pointers belong to one device; use a single-device handle per GPU");
+  if (wrf_check(h, "mp_gt_driver_tile_device", w, t, ae, dt_in)) return 1;
+  const long ncol = (long)t->ni * t->nj;
+  if (kidmp_state_alloc(h, ncol, t->nk)) return 1;
+  DevGuard guard_(h->device);
+  const size_t n = (size_t)ncol * t->nk, n2 = (size_t)ncol;
+  if (ensure_dev(h, &h->d_kid, &h->kid_floats, n)) return 1;          // the per-column dz in step layout
+  if (ae && ensure_dev(h, &h->d_aero, &h->aero_floats, 4 * n + n2)) return 1;
+  WrfArgs a{};
+  a.t = WrfBox{t->ni, t->nk, t->nj, t->i0, t->k0, t->j0, w->ni, w->nk};
+  float* const io[9] = {w->qv, w->qc, w->qi, w->qr, w->qs, w->qg, w->ni_, w->nr, w->th};
+  for (int q = 0; q < 9; ++q) a.a3[q] = io[q];
+  a.pii = w->pii; a.p3 = w->p; a.dz3 = w->dz;
+  a.dz_col = h->d_kid;
+  if (w->re_cloud && w->re_ice && w->re_snow) { a.re_cloud = w->re_cloud; a.re_ice = w->re_ice; a.re_snow = w->re_snow; }
+  a.rainnc = w->rainnc; a.rainncv = w->rainncv; a.sr = w->sr;
+  if (w->snownc && w->snowncv) { a.snownc = w->snownc; a.snowncv = w->snowncv; }
+  if (w->graupelnc && w->graupelncv) { a.graupelnc = w->graupelnc; a.graupelncv = w->graupelncv; }
+  cudaStream_t s = stream ? (cudaStream_t)stream : h->stream;
+  float* const ae4[4] = {ae ? ae->nc : nullptr, ae ? ae->nwfa : nullptr, ae ? ae->nifa : nullptr, ae ? const_cast<float*>(ae->w) : nullptr};
+  return wrf_kernels(h, a, ae ? ae4 : nullptr, ae ? ae->nwfa2d : nullptr, dt_in, s);
 }
 
 int kidmp_set_option(kidmp_handle* h, const char* name, int value) {

@@ -4,8 +4,10 @@
 // RAINNC / RAINNCV / SNOWNC / SNOWNCV / GRAUPELNC / GRAUPELNCV / SR (M:991-1003) and the effective radii of cloud
 // water, cloud ice and snow (calc_effectRad, M:4834-4935; clamps M:1118-1122).
 //
-// A WRF array a(i,k,j) sits at a[i + ni*(k + nk*j)]; the step's layout is [k][col] with col = i + ni*j, so a row of ni
-// floats moves as a whole and both sides of every copy are coalesced.
+// A WRF array a(i,k,j) of the caller's memory box (ni_m x nk_m x nj_m, halo and spare levels included) sits at
+// a[i + ni_m*(k + nk_m*j)], a 2-D one at a[i + ni_m*j].  A call steps one tile of it: tile cell (i,k,j) is memory cell
+// (i0+i, k0+k, j0+j) and column i + ni*j of the step's [k][col] planes, so a row of ni floats moves as a whole and both
+// sides of every copy are coalesced.  Nothing outside the tile is read or written.
 //
 // The is_aerosol_aware branches (M:950-956, M:999-1007, M:4875) are served by kidmp_mp_gt_driver_aero: nc, nwfa, nifa and w
 // travel through k_ikj_planes, the surface emission is k_nwfa_surface, the cloud radius reads the prognostic droplet number.
@@ -18,11 +20,21 @@
 
 namespace kidmp {
 
+// the tile of a call inside the memory box of its arrays (the host checks that it lies inside)
+struct WrfBox {
+  int ni, nk, nj;        // tile extents
+  int i0, k0, j0;        // tile origin in the memory box
+  int ni_m, nk_m;        // memory extents of i and k (the strides)
+  __device__ long at(int i, int k, int j) const { return (long)(i0 + i) + (long)ni_m * ((long)(k0 + k) + (long)nk_m * (j0 + j)); }
+  __device__ long at2(int i, int j) const { return (long)(i0 + i) + (long)ni_m * (j0 + j); }
+  __device__ long plane(int i, int k, int j) const { return (long)k * ni * nj + (long)j * ni + i; }
+};
+
 struct WrfArgs {
-  int ni, nk, nj;
+  WrfBox t;
   float* a3[9];                 // qv qc qi qr qs qg ni nr th, (i,k,j), in state-field order
   const float *pii, *p3, *dz3;  // (i,k,j)
-  float* f[KIDMP_NFIELDS];      // state [nk][ni*nj]
+  float* f[KIDMP_NFIELDS];      // state [nk][ni*nj] of the tile
   float *p, *dz_col;            // [nk][ni*nj]
   const float* ppt;             // [4][ni*nj] rain, ice, snow, graupel of this step
   float *rainnc, *rainncv, *sr, *snownc, *snowncv, *graupelnc, *graupelncv;   // (i,j); the last four may be NULL
@@ -30,20 +42,19 @@ struct WrfArgs {
   const float* nc_plane;                // [nk][ni*nj] prognostic droplet number of an aerosol-aware run, else NULL (nc = Nt_c, M:4875)
 };
 
-// one (i,k,j) array <-> one [k][col] plane of the step (col = i + ni*j); x: i, y: k, z: j
-__global__ void k_ikj_planes(float* a3, float* plane, int ni, int nk, int nj, int to_planes) {
+// one (i,k,j) array <-> one [k][col] plane of the step; x: i, y: k, z: j.  A 2-D (i,j) array is the box with nk = nk_m = 1.
+__global__ void k_ikj_planes(float* a3, float* plane, WrfBox t, int to_planes) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x, k = blockIdx.y, j = blockIdx.z;
-  if (i >= ni) return;
-  const long x = (long)i + (long)ni * (k + (long)nk * j), y = (long)k * ni * nj + (long)j * ni + i;
+  if (i >= t.ni) return;
+  const long x = t.at(i, k, j), y = t.plane(i, k, j);
   if (to_planes) plane[y] = a3[x]; else a3[x] = plane[y];
 }
 
 // one thread per cell; x: i, y: k, z: j
 __global__ void k_wrf_gather(WrfArgs a) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x, k = blockIdx.y, j = blockIdx.z;
-  if (i >= a.ni) return;
-  const long src = (long)i + (long)a.ni * (k + (long)a.nk * j);
-  const long dst = (long)k * a.ni * a.nj + (long)j * a.ni + i;
+  if (i >= a.t.ni) return;
+  const long src = a.t.at(i, k, j), dst = a.t.plane(i, k, j);
 #pragma unroll
   for (int q = 0; q < 8; ++q) a.f[q][dst] = a.a3[q][src];
   a.f[8][dst] = a.a3[8][src] * a.pii[src];                 // t1d = th*pii, M:941
@@ -56,9 +67,8 @@ __device__ __constant__ float c_g_ratio[15] = {24, 60, 120, 210, 336, 504, 720, 
 
 __global__ void k_wrf_scatter(WrfArgs a, float Nt_c) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x, k = blockIdx.y, j = blockIdx.z;
-  if (i >= a.ni) return;
-  const long dst = (long)i + (long)a.ni * (k + (long)a.nk * j);
-  const long src = (long)k * a.ni * a.nj + (long)j * a.ni + i;
+  if (i >= a.t.ni) return;
+  const long dst = a.t.at(i, k, j), src = a.t.plane(i, k, j);
   const float qv1d = a.f[0][src], qc1d = a.f[1][src], qi1d = a.f[2][src], qs1d = a.f[4][src], ni1d = a.f[6][src];
   const float t1d = a.f[8][src];
 #pragma unroll
@@ -100,17 +110,19 @@ __global__ void k_wrf_scatter(WrfArgs a, float Nt_c) {
   }
 }
 
-// M:986-1003, one thread per column
+// M:986-1003, one thread per column of the tile (c = i + ni*j)
 __global__ void k_wrf_accumulate(WrfArgs a) {
-  const long c = (long)blockIdx.x * blockDim.x + threadIdx.x, ncol = (long)a.ni * a.nj;
+  const long c = (long)blockIdx.x * blockDim.x + threadIdx.x, ncol = (long)a.t.ni * a.t.nj;
   if (c >= ncol) return;
+  const int j = (int)(c / a.t.ni), i = (int)(c - (long)j * a.t.ni);
+  const long m = a.t.at2(i, j);
   const float pptrain = a.ppt[c], pptice = a.ppt[ncol + c], pptsnow = a.ppt[2 * ncol + c], pptgraul = a.ppt[3 * ncol + c];
   const float rncv = pptrain + pptsnow + pptgraul + pptice;
-  a.rainncv[c] = rncv;
-  a.rainnc[c] = a.rainnc[c] + pptrain + pptsnow + pptgraul + pptice;
-  if (a.snowncv && a.snownc) { a.snowncv[c] = pptsnow + pptice; a.snownc[c] = a.snownc[c] + pptsnow + pptice; }
-  if (a.graupelncv && a.graupelnc) { a.graupelncv[c] = pptgraul; a.graupelnc[c] = a.graupelnc[c] + pptgraul; }
-  a.sr[c] = (pptsnow + pptgraul + pptice) / (rncv + 1.e-12f);
+  a.rainncv[m] = rncv;
+  a.rainnc[m] = a.rainnc[m] + pptrain + pptsnow + pptgraul + pptice;
+  if (a.snowncv && a.snownc) { a.snowncv[m] = pptsnow + pptice; a.snownc[m] = a.snownc[m] + pptsnow + pptice; }
+  if (a.graupelncv && a.graupelnc) { a.graupelncv[m] = pptgraul; a.graupelnc[m] = a.graupelnc[m] + pptgraul; }
+  a.sr[m] = (pptsnow + pptgraul + pptice) / (rncv + 1.e-12f);
 }
 
 }  // namespace kidmp

@@ -43,7 +43,8 @@ module mphys_thompson09n
      type(c_ptr) :: ppt
   end type kidmp_kid_columns
 
-  ! include/kidmp.h :: kidmp_wrf_fields, (i,k,j) arrays as c_loc of (ims:ime,kms:kme,jms:jme) arrays
+  ! include/kidmp.h :: kidmp_wrf_fields, (i,k,j) arrays as c_loc of (ims:ime,kms:kme,jms:jme) arrays; ni, nk, nj are the memory
+  ! dimensions (kidmp_mp_gt_driver steps the whole box: a host with halos or kme = kte+1 uses kidmp_mp_gt_driver_tile)
   type, bind(C) :: kidmp_wrf_fields
      integer(c_int) :: ni, nk, nj
      type(c_ptr) :: qv, qc, qr, qi, qs, qg, ni_, nr, th, pii, p, dz
@@ -54,6 +55,16 @@ module mphys_thompson09n
   type, bind(C) :: kidmp_wrf_aerosols
      type(c_ptr) :: nc, nwfa, nifa, w, nwfa2d
   end type kidmp_wrf_aerosols
+  ! include/kidmp.h :: kidmp_wrf_tile, the tile to step inside the memory box of kidmp_wrf_fields (0-based offsets, extents).
+  ! A WRF / MPAS caller passes the memory dimensions in kidmp_wrf_fields and its tile here:
+  !   w%ni = ime-ims+1;  w%nk = kme-kms+1;  w%nj = jme-jms+1          (c_loc of the (ims:ime,kms:kme,jms:jme) arrays)
+  !   t%i0 = its-ims;    t%ni = ite-its+1
+  !   t%k0 = kts-kms;    t%nk = kte-kts+1                              (kme = kte+1: the spare top level stays out)
+  !   t%j0 = jts-jms;    t%nj = jte-jts+1
+  ! The call reads and writes only the tile, so the OpenMP tiles of one patch may step at the same time (one handle each).
+  type, bind(C) :: kidmp_wrf_tile
+     integer(c_int) :: i0, ni, k0, nk, j0, nj
+  end type kidmp_wrf_tile
 
   interface
      integer(c_int) function kidmp_init(cfg, handle) bind(C, name='kidmp_init')
@@ -109,6 +120,26 @@ module mphys_thompson09n
        type(kidmp_wrf_aerosols), intent(in) :: ae
        real(c_float), value :: dt_in
      end function kidmp_mp_gt_driver_aero
+     ! one tile of the memory box, host arrays; ae = c_null_ptr: is_aerosol_aware = .false., else c_loc of a kidmp_wrf_aerosols
+     integer(c_int) function kidmp_mp_gt_driver_tile(handle, w, t, ae, dt_in) bind(C, name='kidmp_mp_gt_driver_tile')
+       import :: c_int, c_ptr, c_float, kidmp_wrf_fields, kidmp_wrf_tile
+       type(c_ptr), value :: handle
+       type(kidmp_wrf_fields), intent(in) :: w
+       type(kidmp_wrf_tile), intent(in) :: t
+       type(c_ptr), value :: ae
+       real(c_float), value :: dt_in
+     end function kidmp_mp_gt_driver_tile
+     ! ... the same on device arrays (e.g. OpenACC / CUDA Fortran device data), enqueued on `stream` (c_null_ptr = the handle's)
+     integer(c_int) function kidmp_mp_gt_driver_tile_device(handle, w, t, ae, dt_in, stream) &
+          bind(C, name='kidmp_mp_gt_driver_tile_device')
+       import :: c_int, c_ptr, c_float, kidmp_wrf_fields, kidmp_wrf_tile
+       type(c_ptr), value :: handle
+       type(kidmp_wrf_fields), intent(in) :: w
+       type(kidmp_wrf_tile), intent(in) :: t
+       type(c_ptr), value :: ae
+       real(c_float), value :: dt_in
+       type(c_ptr), value :: stream
+     end function kidmp_mp_gt_driver_tile_device
   end interface
 
   !Logical switches

@@ -94,6 +94,17 @@ class WrfAerosols(C.Structure):
 
 SYMBOLS["kidmp_mp_gt_driver"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields), C.c_float])
 SYMBOLS["kidmp_mp_gt_driver_aero"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields), C.POINTER(WrfAerosols), C.c_float])
+
+
+class WrfTile(C.Structure):
+    """kidmp_wrf_tile of include/kidmp.h: 0-based offsets and extents of the tile inside the memory box."""
+    _fields_ = [(n, C.c_int) for n in ("i0", "ni", "k0", "nk", "j0", "nj")]
+
+
+SYMBOLS["kidmp_mp_gt_driver_tile"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields), C.POINTER(WrfTile), C.POINTER(WrfAerosols),
+                                                C.c_float])
+SYMBOLS["kidmp_mp_gt_driver_tile_device"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields), C.POINTER(WrfTile),
+                                                       C.POINTER(WrfAerosols), C.c_float, C.c_void_p])
 SYMBOLS["kidmp_kid_interface"] = (C.c_int, [C.c_void_p, C.POINTER(KidColumns), C.c_float, C.c_float, C.c_float])
 HYD_PLANES = ("qc", "qr", "nr", "qi", "ni", "qs", "qg")
 
@@ -281,24 +292,57 @@ class Thompson:
         """kidmp_set_option: tuning knobs that do not change results ("chunk": columns per launch, "timing": 0 / 1)."""
         self._ck(self._L.kidmp_set_option(self.h, name.encode(), int(value)))
 
-    def mp_gt_driver(self, dt, f3, pii, p, dz, acc, radii=True, aerosols=None):
+    def mp_gt_driver(self, dt, f3, pii, p, dz, acc, radii=True, aerosols=None, tile=None):
         """mp_gt_driver (M:806-1143) through kidmp_mp_gt_driver.  f3: dict qv qc qr qi qs qg ni nr th of (nj, nk, ni)
         float32 arrays (C order = WRF's (i,k,j) Fortran order), updated in place; pii, p, dz the same shape; acc: dict
         rainnc rainncv sr [snownc snowncv graupelnc graupelncv] of (nj, ni) arrays, updated in place.
         aerosols: dict nc nwfa nifa w of (nj, nk, ni) arrays [+ nwfa2d (nj, ni)]: is_aerosol_aware = .true. through
         kidmp_mp_gt_driver_aero (nc, nwfa, nifa updated in place).
+        tile: (i0, ni, k0, nk, j0, nj) steps only that tile of the arrays, which are then the memory box (halo points and
+        spare levels included), through kidmp_mp_gt_driver_tile; nothing outside the tile is read or written.
+        radii: True = new zero arrays of the memory box's shape, returned (outside a tile they stay zero); a dict of
+        re_cloud re_ice re_snow arrays = those, filled in place; False = no radii.
         Returns dict re_cloud re_ice re_snow (empty when radii is False)."""
         nj, nk, ni = f3["qv"].shape
+        w, ae, re, keep = self._wrf_structs(f3, pii, p, dz, acc, radii, aerosols, (nj, nk, ni), lambda a: _f32c(a).ctypes.data_as(_fp))
+        if tile is not None:
+            t = WrfTile(*[int(x) for x in tile])
+            self._ck(self._L.kidmp_mp_gt_driver_tile(self.h, C.byref(w), C.byref(t), C.byref(ae) if ae is not None else None,
+                                                     float(dt)))
+        elif ae is not None:
+            self._ck(self._L.kidmp_mp_gt_driver_aero(self.h, C.byref(w), C.byref(ae), float(dt)))
+        else:
+            self._ck(self._L.kidmp_mp_gt_driver(self.h, C.byref(w), float(dt)))
+        return re
+
+    def mp_gt_driver_device(self, dt, f3, pii, p, dz, acc, tile=None, radii=None, aerosols=None, stream=None):
+        """kidmp_mp_gt_driver_tile_device: the same step on device arrays (anything with data_ptr(), e.g. contiguous float32
+        CUDA tensors of the shapes of mp_gt_driver), enqueued on `stream` (a torch.cuda.Stream, a cudaStream_t as int, or
+        None = the handle's stream) without synchronising.  tile None = the whole memory box.  radii: dict re_cloud re_ice
+        re_snow of device arrays (filled inside the tile) or None."""
+        nj, nk, ni = f3["qv"].shape
+        w, ae, _, keep = self._wrf_structs(f3, pii, p, dz, acc, radii or False, aerosols, (nj, nk, ni),
+                                           lambda a: C.cast(C.c_void_p(int(a.data_ptr())), _fp))
+        t = WrfTile(*[int(x) for x in (tile if tile is not None else (0, ni, 0, nk, 0, nj))])
+        s = getattr(stream, "cuda_stream", stream)
+        self._ck(self._L.kidmp_mp_gt_driver_tile_device(self.h, C.byref(w), C.byref(t), C.byref(ae) if ae is not None else None,
+                                                        float(dt), C.c_void_p(int(s)) if s else None))
+
+    @staticmethod
+    def _wrf_structs(f3, pii, p, dz, acc, radii, aerosols, shape3, addr):
+        """kidmp_wrf_fields / kidmp_wrf_aerosols over the arrays; addr(a) gives an array's address."""
+        nj, nk, ni = shape3
         w = WrfFields()
         w.ni, w.nk, w.nj = ni, nk, nj
         keep = []
 
         def ptr(a, shape):
-            a = _f32c(a)
-            if a.shape != shape:
-                raise ValueError("array shape %r, expected %r" % (a.shape, shape))
+            if tuple(a.shape) != shape:
+                raise ValueError("array shape %r, expected %r" % (tuple(a.shape), shape))
+            if hasattr(a, "is_contiguous") and (not a.is_contiguous() or str(a.dtype) != "torch.float32"):
+                raise ValueError("float32 contiguous tensor required")
             keep.append(a)
-            return a.ctypes.data_as(_fp)
+            return addr(a)
         for name, key in (("qv", "qv"), ("qc", "qc"), ("qr", "qr"), ("qi", "qi"), ("qs", "qs"), ("qg", "qg"),
                           ("ni_", "ni"), ("nr", "nr"), ("th", "th")):
             setattr(w, name, ptr(f3[key], (nj, nk, ni)))
@@ -308,19 +352,20 @@ class Thompson:
         for name in ("snownc", "snowncv", "graupelnc", "graupelncv"):
             if acc.get(name) is not None:
                 setattr(w, name, ptr(acc[name], (nj, ni)))
-        re = {k: np.zeros((nj, nk, ni), np.float32) for k in ("re_cloud", "re_ice", "re_snow")} if radii else {}
+        if radii is True:
+            re = {k: np.zeros((nj, nk, ni), np.float32) for k in ("re_cloud", "re_ice", "re_snow")}
+        else:
+            re = dict(radii) if radii else {}
         for name, a in re.items():
             setattr(w, name, ptr(a, (nj, nk, ni)))
+        ae = None
         if aerosols is not None:
             ae = WrfAerosols()
             for name in ("nc", "nwfa", "nifa", "w"):
                 setattr(ae, name, ptr(aerosols[name], (nj, nk, ni)))
             if aerosols.get("nwfa2d") is not None:
                 ae.nwfa2d = ptr(aerosols["nwfa2d"], (nj, ni))
-            self._ck(self._L.kidmp_mp_gt_driver_aero(self.h, C.byref(w), C.byref(ae), float(dt)))
-            return re
-        self._ck(self._L.kidmp_mp_gt_driver(self.h, C.byref(w), float(dt)))
-        return re
+        return w, ae, re, keep
 
     def kid_interface(self, kid, dt, p0=1.0e5, r_on_cp=287.05 / 1005.0):
         """mphys_thompson09_interfacen (I:28-246) without save_dg.  kid: dict of float32 (nx, nz) arrays 'theta',
