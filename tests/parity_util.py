@@ -17,6 +17,10 @@ FLIP_FRACTION = 2e-4
 # compared absolutely
 FLOOR = {"qv": 1e-10, "qc": 1e-12, "qi": 1e-12, "qr": 1e-12, "qs": 1e-12, "qg": 1e-12, "ni": 1e-3, "nr": 1e-3,
          "t": 1.0, "nc": 1e-3, "nwfa": 1e-3, "nifa": 1e-3}
+# the constants of thompson_init (M:374-797) that the device keeps and the oracle exports: compared bit for bit
+INIT_CONSTANTS = ("cre", "crg", "cse", "csg", "cge", "cgg", "cie", "cig", "cce1", "cce2", "cce3", "cce4", "cce5",
+                  "ccg1", "ccg2", "ccg3", "ccg4", "ccg5", "ocg1", "ocg2", "scalars", "offsets",
+                  "Dc", "Di", "Dr", "Ds", "Dg", "t_Nc", "dtc", "dti", "dtr", "dts", "dtg")
 
 
 def compare_field(name, got, ref):

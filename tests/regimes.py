@@ -10,11 +10,14 @@ run in too few cells for a domain-wide outlier allowance to notice.  Every case 
 Each case has two kinds of column: PROBE columns (a few busy levels in an otherwise clear column: sedimentation carries the
 result into idle cells below) and UNIFORM columns (every level in the regime).  The values spread over the columns include
 the exact f32 threshold and np.nextafter on each side of it.  tests/test_regimes.py checks the claims on the CPU and
-compares the CUDA step with the oracle case by case on the GPU.  M: = module_mp_thompson09n.f90.
+compares the CUDA step with the oracle case by case on the GPU; tests/test_configurations.py does the same under every handle
+configuration.  The device-step helpers and the cell-by-cell outlier reports both use are at the end of this module.
+M: = module_mp_thompson09n.f90.
 """
 import numpy as np
 
 from oracle import oracle as orc
+from parity_util import FLOOR, REL_TOL
 
 F = np.float32
 FIELDS = ("qv", "qc", "qi", "qr", "qs", "qg", "ni", "nr", "t")
@@ -555,6 +558,94 @@ def oracle_run(o, case, with_rates=True):
             r = o.column(dt, *[st[k][:, j] for k in FIELDS], p[:, j], dz, want_rates=True)
             rates[:, :, j] = r["rates"]
     return st, p, dz, dt, out, ppt, rates
+
+
+def bench_like(ncol, dz):
+    """Columns of the bench domain (kid_b200/synth.py, 60 levels of depth dz): (state, p, dz)."""
+    from kid_b200 import synth
+    st, p, dzv = synth.make_domain(ncol, nz=60, nx=1024, dz=dz, col0=300000)
+    return {k: v.numpy().copy() for k, v in st.items()}, p.numpy().copy(), dzv.numpy().copy()
+
+
+# ---- the CUDA step against the oracle, cell by cell (GPU tests) --------------------------------------------------------
+RATE_TOL = 1e-5
+
+
+def cell_outliers(got, ref, fields, cls):
+    """One line per cell of `fields` where got and ref differ by more than REL_TOL (relative to max(|ref|, FLOOR))."""
+    out = []
+    for f in fields:
+        a, b = got[f].astype(np.float64), ref[f].astype(np.float64)
+        rel = np.abs(a - b) / np.maximum(np.abs(b), FLOOR.get(f, 1e-30))
+        rel = np.where(a == b, 0.0, rel)
+        for k, j in np.argwhere(~(rel <= REL_TOL)):
+            out.append("col %d level %d %s: gpu %.9g oracle %.9g (rel %.2e, class %s)" % (j, k, f, a[k, j], b[k, j], rel[k, j],
+                                                                                          cls[k, j] or "idle"))
+    return out
+
+
+def rate_outliers(got, ref, names, cls):
+    """One line per (rate, cell) where the device rate differs from the oracle's (rounded to f32) by more than RATE_TOL."""
+    out = []
+    ref32 = ref.astype(np.float32).astype(np.float64)
+    got = got.astype(np.float64)
+    rel = np.abs(got - ref32) / np.maximum(np.abs(ref32), 1e-30)
+    rel = np.where(got == ref32, 0.0, rel)
+    for q, k, j in np.argwhere(~(rel <= RATE_TOL)):
+        out.append("col %d level %d %s: gpu %.9g oracle %.9g (class %s)" % (j, k, names[q], got[q, k, j], ref32[q, k, j],
+                                                                             cls[k, j] or "idle"))
+    return out
+
+
+class Device:
+    """Device copies of one input, allocated once: every run() starts from the same inputs at the same addresses, so that a
+    handle with CUDA graphs on replays its capture of the previous run unless a setting in the graph key changed."""
+
+    def __init__(self, st, p, dz, dt, rates=True):
+        import torch
+        self.nz, self.ncol = st["t"].shape
+        self.dt = dt
+        self.src = {k: torch.from_numpy(st[k].copy()).cuda() for k in FIELDS}
+        self.dev = {k: v.clone() for k, v in self.src.items()}
+        self.p, self.dz = torch.from_numpy(p).cuda(), torch.from_numpy(dz).cuda()
+        self.ppt = torch.zeros((4, self.ncol), dtype=torch.float32, device="cuda")
+        self.rates = torch.empty((36, self.nz, self.ncol), dtype=torch.float32, device="cuda") if rates else None
+
+    def run(self, th):
+        """One step; returns (state, ppt, rates or None, diag, step_stats)."""
+        import torch
+        for k in FIELDS:
+            self.dev[k].copy_(self.src[k])
+        if self.rates is not None:
+            self.rates.fill_(float("nan"))
+        th.set_rates_buffer(self.rates.data_ptr() if self.rates is not None else 0)
+        th.diag()
+        torch.cuda.synchronize()
+        try:
+            th.step_device(self.ncol, self.nz, self.dt, [self.dev[k].data_ptr() for k in FIELDS], self.p.data_ptr(),
+                           self.dz.data_ptr(), self.ppt.data_ptr())
+            th.sync()
+        finally:
+            th.set_rates_buffer(0)
+        return ({k: self.dev[k].cpu().numpy() for k in FIELDS}, self.ppt.cpu().numpy(),
+                self.rates.cpu().numpy() if self.rates is not None else None, th.diag(), th.step_stats())
+
+
+def aero_step(th, st, p, dz, dt, nc, nwfa, nifa, w):
+    """kidmp_step_device_aero on device copies of the inputs: (state with nc nwfa nifa, ppt)."""
+    import torch
+    nz, ncol = st["t"].shape
+    dev = {k: torch.from_numpy(st[k].copy()).cuda() for k in FIELDS}
+    dnc, dnwfa, dnifa, dw = (torch.from_numpy(x.copy()).cuda() for x in (nc, nwfa, nifa, w))
+    dp, ddz = torch.from_numpy(p).cuda(), torch.from_numpy(dz).cuda()
+    ppt = torch.zeros((4, ncol), dtype=torch.float32, device="cuda")
+    torch.cuda.synchronize()
+    th.step_device_aero(ncol, nz, dt, [dev[k].data_ptr() for k in FIELDS], dnc.data_ptr(), dnwfa.data_ptr(), dnifa.data_ptr(),
+                        dp.data_ptr(), dw.data_ptr(), ddz.data_ptr(), ppt.data_ptr())
+    th.sync()
+    out = {k: dev[k].cpu().numpy() for k in FIELDS}
+    out.update(nc=dnc.cpu().numpy(), nwfa=dnwfa.cpu().numpy(), nifa=dnifa.cpu().numpy())
+    return out, ppt.cpu().numpy()
 
 
 def aero_inputs(st, p, seed=0):

@@ -9,7 +9,7 @@ import os
 import numpy as np
 import pytest
 
-from parity_util import assert_parity, compare_states, FIELDS
+from parity_util import assert_parity, compare_states, FIELDS, INIT_CONSTANTS
 
 pytestmark = pytest.mark.gpu
 
@@ -32,9 +32,7 @@ def _both(g, o, dt, st, p, dz, layout="col_fastest"):
 
 # ---- thompson_init: constants and lookup tables (M:374-797, M:3698-4343) ------------------------------
 def test_init_constants_bit_exact(gpu_mixed, oracle_mixed):
-    for name in ("cre", "crg", "cse", "csg", "cge", "cgg", "cie", "cig", "cce1", "cce2", "cce3", "cce4", "cce5",
-                 "ccg1", "ccg2", "ccg3", "ccg4", "ccg5", "ocg1", "ocg2", "scalars", "offsets",
-                 "Dc", "Di", "Dr", "Ds", "Dg", "t_Nc", "dtc", "dti", "dtr", "dts", "dtg"):
+    for name in INIT_CONSTANTS:
         assert np.array_equal(gpu_mixed.get(name), oracle_mixed.get(name).ravel()), name
 
 
@@ -679,7 +677,8 @@ def test_wrf_driver_entry(gpu_mixed, oracle_mixed):
     for k, (lo, hi) in lim.items():
         assert ra[k].min() >= np.float32(lo) and ra[k].max() <= np.float32(hi), k
         assert (ra[k] > np.float32(lo) * 1.01).any(), k
-        # where the state agrees to the bit the radius must too (up to the f32 rounding of one power)
+        # where the state agrees to the bit the radius must too (up to the f32 rounding of one power); the bit-exact check of
+        # the radii against calc_effectRad of the returned state is tests/test_effective_radii.py
         np.testing.assert_allclose(ra[k], rb[k], rtol=2e-5, err_msg=k)
     # optional arguments absent: snow / graupel accumulators and radii are simply not produced
     a4 = {k: v.copy() for k, v in f3.items()}
@@ -865,7 +864,7 @@ def test_wrf_driver_entry_aerosol_aware(gpu_mixed, oracle_mixed):
     tot = ppt.sum(0).reshape(nj, ni)
     np.testing.assert_allclose(aa["rainncv"], tot, rtol=1e-4, atol=1e-9)
     # the cloud radius follows the prognostic droplet number: equal to the oracle's calc_effectRad fed with nc, and
-    # different from what the fixed Nt_c gives
+    # different from what the fixed Nt_c gives (bit for bit, on the state the step returns: tests/test_effective_radii.py)
     rc_want = np.zeros((nk, nj * ni), np.float32)
     rc_fixed = np.zeros((nk, nj * ni), np.float32)
     for c in range(0, nj * ni, 7):

@@ -10,11 +10,9 @@ import numpy as np
 import pytest
 
 import regimes as R
-from parity_util import FLOOR, REL_TOL
 
 FIELDS = R.FIELDS
 AERO_FIELDS = FIELDS + ("nc", "nwfa", "nifa")
-RATE_TOL = 1e-5
 
 # Outliers allowed per (case, handle); every other case allows none.  Keep each a fixed count with its cause.
 # sediment: dt = 120 s with hundreds of sedimentation sub-steps takes nearly all the graupel (rain: its number) out of the lowest
@@ -79,66 +77,8 @@ def test_thresholds_sit_on_both_sides_of_their_f32_values():
 
 
 # ---- GPU ---------------------------------------------------------------------------------------------------------------
-def _cell_outliers(got, ref, fields, cls):
-    out = []
-    for f in fields:
-        a, b = got[f].astype(np.float64), ref[f].astype(np.float64)
-        rel = np.abs(a - b) / np.maximum(np.abs(b), FLOOR.get(f, 1e-30))
-        rel = np.where(a == b, 0.0, rel)
-        for k, j in np.argwhere(~(rel <= REL_TOL)):
-            out.append("col %d level %d %s: gpu %.9g oracle %.9g (rel %.2e, class %s)" % (j, k, f, a[k, j], b[k, j], rel[k, j],
-                                                                                          cls[k, j] or "idle"))
-    return out
-
-
-def _rate_outliers(got, ref, names, cls):
-    out = []
-    ref32 = ref.astype(np.float32).astype(np.float64)
-    got = got.astype(np.float64)
-    rel = np.abs(got - ref32) / np.maximum(np.abs(ref32), 1e-30)
-    rel = np.where(got == ref32, 0.0, rel)
-    for q, k, j in np.argwhere(~(rel <= RATE_TOL)):
-        out.append("col %d level %d %s: gpu %.9g oracle %.9g (class %s)" % (j, k, names[q], got[q, k, j], ref32[q, k, j],
-                                                                             cls[k, j] or "idle"))
-    return out
-
-
-class _Device:
-    """Device copies of one input, allocated once: every run() starts from the same inputs at the same addresses, so that a
-    handle with CUDA graphs on replays its capture of the previous run unless a setting in the graph key changed."""
-
-    def __init__(self, st, p, dz, dt, rates=True):
-        import torch
-        self.nz, self.ncol = st["t"].shape
-        self.dt = dt
-        self.src = {k: torch.from_numpy(st[k].copy()).cuda() for k in FIELDS}
-        self.dev = {k: v.clone() for k, v in self.src.items()}
-        self.p, self.dz = torch.from_numpy(p).cuda(), torch.from_numpy(dz).cuda()
-        self.ppt = torch.zeros((4, self.ncol), dtype=torch.float32, device="cuda")
-        self.rates = torch.empty((36, self.nz, self.ncol), dtype=torch.float32, device="cuda") if rates else None
-
-    def run(self, th):
-        """One step; returns (state, ppt, rates or None, diag, step_stats)."""
-        import torch
-        for k in FIELDS:
-            self.dev[k].copy_(self.src[k])
-        if self.rates is not None:
-            self.rates.fill_(float("nan"))
-        th.set_rates_buffer(self.rates.data_ptr() if self.rates is not None else 0)
-        th.diag()
-        torch.cuda.synchronize()
-        try:
-            th.step_device(self.ncol, self.nz, self.dt, [self.dev[k].data_ptr() for k in FIELDS], self.p.data_ptr(),
-                           self.dz.data_ptr(), self.ppt.data_ptr())
-            th.sync()
-        finally:
-            th.set_rates_buffer(0)
-        return ({k: self.dev[k].cpu().numpy() for k in FIELDS}, self.ppt.cpu().numpy(),
-                self.rates.cpu().numpy() if self.rates is not None else None, th.diag(), th.step_stats())
-
-
 def _device_step(th, st, p, dz, dt, rates=True):
-    return _Device(st, p, dz, dt, rates).run(th)
+    return R.Device(st, p, dz, dt, rates).run(th)
 
 
 @pytest.mark.gpu
@@ -150,11 +90,11 @@ def test_case_parity_with_the_oracle(case, handle, gpu_mixed, gpu_warm, oracle_m
     st, p, dz, dt, ref, ppt_ref, rates_ref = _oracle(o, case, handle)
     got, ppt, rates, _, _ = _device_step(th, st, p, dz, dt)
     cls, _ = R.cell_classes(st, p, iiwarm=handle == "warm")
-    bad = _cell_outliers(got, ref, FIELDS, cls)
+    bad = R.cell_outliers(got, ref, FIELDS, cls)
     # clear-sky columns: the kernel leaves the buffer alone; every other column gets all of its levels
     active = np.isfinite(rates).all(axis=(0, 1))
     assert not rates_ref[:, :, ~active].any()
-    rbad = _rate_outliers(rates[:, :, active], rates_ref[:, :, active], o.rate_names, cls[:, active])
+    rbad = R.rate_outliers(rates[:, :, active], rates_ref[:, :, active], o.rate_names, cls[:, active])
     print("REGIME %s/%s: %d state outliers, %d rate outliers" % (case.name, handle, len(bad), len(rbad)))
     assert len(bad) <= STATE_ALLOW.get((case.name, handle), 0), "%s/%s state:\n  %s" % (case.name, handle, "\n  ".join(bad[:20]))
     assert len(rbad) <= RATE_ALLOW.get((case.name, handle), 0), "%s/%s rates:\n  %s" % (case.name, handle, "\n  ".join(rbad[:20]))
@@ -173,12 +113,6 @@ def _same(a, b, what):
     assert np.allclose(da[:6], db[:6], rtol=1e-12, atol=0), what
 
 
-def _bench_like(ncol, dz):
-    from kid_b200 import synth
-    st, p, dzv = synth.make_domain(ncol, nz=60, nx=1024, dz=dz, col0=300000)
-    return {k: v.numpy().copy() for k, v in st.items()}, p.numpy().copy(), dzv.numpy().copy()
-
-
 @pytest.mark.gpu
 def test_class_kernels_compute_what_the_general_kernel_computes():
     """Every class kernel computes bit for bit what k_cells<KC_FULL> computes for the same cell (kidmp_cells.cuh): the
@@ -189,9 +123,9 @@ def test_class_kernels_compute_what_the_general_kernel_computes():
     try:
         inputs = [("regimes",) + R.regime_domain(), ("sediment",) + R.build("sediment")]
         for dt in (10.0, 60.0):
-            inputs.append(("bench-like dt=%g" % dt,) + _bench_like(40000, 100.0) + (dt,))
+            inputs.append(("bench-like dt=%g" % dt,) + R.bench_like(40000, 100.0) + (dt,))
         for name, st, p, dz, dt in inputs:
-            d = _Device(st, p, dz, dt)
+            d = R.Device(st, p, dz, dt)
             runs = {}
             for classes in (1, 0, 1):
                 th.set_option("classes", classes)
@@ -215,7 +149,7 @@ def test_class_kernels_of_the_warm_handle():
     from kid_b200.kidmp import Thompson
     th = Thompson(set_Nc=50.0, iiwarm=True, l_sediment=True)
     try:
-        d = _Device(*R.regime_domain())
+        d = R.Device(*R.regime_domain())
         runs = {}
         for classes in (1, 0):
             th.set_option("classes", classes)
@@ -226,22 +160,6 @@ def test_class_kernels_of_the_warm_handle():
         assert s0["cells_full"] == s0["busy_cells"] == s1["busy_cells"], s0
     finally:
         th.close()
-
-
-def _aero_step(th, st, p, dz, dt, nc, nwfa, nifa, w):
-    import torch
-    nz, ncol = st["t"].shape
-    dev = {k: torch.from_numpy(st[k].copy()).cuda() for k in FIELDS}
-    dnc, dnwfa, dnifa, dw = (torch.from_numpy(x.copy()).cuda() for x in (nc, nwfa, nifa, w))
-    dp, ddz = torch.from_numpy(p).cuda(), torch.from_numpy(dz).cuda()
-    ppt = torch.zeros((4, ncol), dtype=torch.float32, device="cuda")
-    torch.cuda.synchronize()
-    th.step_device_aero(ncol, nz, dt, [dev[k].data_ptr() for k in FIELDS], dnc.data_ptr(), dnwfa.data_ptr(), dnifa.data_ptr(),
-                        dp.data_ptr(), dw.data_ptr(), ddz.data_ptr(), ppt.data_ptr())
-    th.sync()
-    out = {k: dev[k].cpu().numpy() for k in FIELDS}
-    out.update(nc=dnc.cpu().numpy(), nwfa=dnwfa.cpu().numpy(), nifa=dnifa.cpu().numpy())
-    return out, ppt.cpu().numpy()
 
 
 AERO_CASES = [c for c in R.CASES if c.aero]
@@ -257,7 +175,7 @@ def test_aerosol_aware_class_kernels_compute_what_the_general_kernel_computes():
         runs = {}
         for classes in (1, 0):
             th.set_option("classes", classes)
-            runs[classes] = _aero_step(th, st, p, dz, dt, *ae)
+            runs[classes] = R.aero_step(th, st, p, dz, dt, *ae)
         for k in AERO_FIELDS:
             assert np.array_equal(runs[1][0][k], runs[0][0][k]), k
         assert np.array_equal(runs[1][1], runs[0][1])
@@ -295,10 +213,10 @@ def test_aerosol_aware_case_parity_with_the_oracle(case, gpu_mixed, oracle_mixed
     ref = {k: v.copy() for k, v in st.items()}
     rnc, rnwfa, rnifa = nc.copy(), nwfa.copy(), nifa.copy()
     ppt_ref = oracle_mixed.step_aero(dt, ref, rnc, rnwfa, rnifa, p, w, dz)
-    got, ppt = _aero_step(gpu_mixed, st, p, dz, dt, nc, nwfa, nifa, w)
+    got, ppt = R.aero_step(gpu_mixed, st, p, dz, dt, nc, nwfa, nifa, w)
     ref.update(nc=rnc, nwfa=rnwfa, nifa=rnifa)
     cls, _ = R.cell_classes(st, p)
-    bad = _cell_outliers(got, ref, AERO_FIELDS, cls)
+    bad = R.cell_outliers(got, ref, AERO_FIELDS, cls)
     print("REGIME aero %s: %d state outliers" % (case.name, len(bad)))
     assert len(bad) <= AERO_ALLOW.get(case.name, 0), "aero %s:\n  %s" % (case.name, "\n  ".join(bad[:20]))
     np.testing.assert_allclose(ppt, ppt_ref, rtol=1e-5, atol=1e-10, err_msg="aero %s ppt" % case.name)
