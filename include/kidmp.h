@@ -204,7 +204,7 @@ int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, c
  * buffers (128-byte hand-off records, cell lists) are sized for one chunk, whatever the size of the domain.
  * "timing": 1 = run the kernels of a launch one after the other with an event after each (kidmp_last_kernel_ms), 2 = the
  *   normal schedule (second stream in use) with the same events on the main stream, 0 = normal.
- * "graphs": 1 (default, KIDMP_GRAPHS) = the launches of a step (up to 64 chunks on one lane) are captured once in a CUDA graph (a cache of eight) and replayed
+ * "graphs": 1 (default, KIDMP_GRAPHS) = the launches of a step (up to 64 chunks) are captured once in a CUDA graph (a cache of eight) and replayed
  *   while the arguments stay the same (KiD's own cases of 1 to 14 400 columns are launch-bound; the 1 048 576-column step loses its
  *   launch gaps); 0 = plain launches.
  * "simple": 1 (default) = a column that holds no graupel and in which no fall speed can cross the thinnest layer in one step
@@ -213,16 +213,10 @@ int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, c
  * "classes": 1 (default) = every busy cell goes to the cell kernel specialised for its species set and temperature class;
  *   0 = every busy cell goes to the general one.  The specialised kernels compute the same bits (tests/test_regimes.py): this
  *   is their reference, not a tuning choice.
- * "lanes" (1..8, default 1, KIDMP_LANES), "lane_min" (columns, KIDMP_LANE_MIN), "stagger", "cell_blocks": a step over at least
- *   2 x lane_min columns is cut into launches that run side by side on `lanes` work sets and streams.  Measured on the
- *   bench domain: no gain over one lane (profiles/r02_ncu_step_kernels.md), so the default is one.
- * "l2_window": the cell kernels that gather from the collection tables carry an L2 access-policy window over the table slab;
- *   only has an effect when the handle was created with KIDMP_L2_WINDOW=1 in the environment (the L2 set-aside is made at
- *   init).  Measured: the step slows from 3.5 to 5.1 ms, so it is off.
- * "fuse", "units": knobs of the round-1 kernels, accepted and ignored.
- * Environment only: KIDMP_PIPE_CHUNK (columns per chunk of kidmp_step's host pipeline), KIDMP_ZEROCOPY=0 (copy whole chunks
- *   back instead of writing the changed columns into pinned host arrays), KIDMP_PIPE_TRACE=1 (device timeline of every chunk
- *   of kidmp_step on stderr). */
+ * Any other name is refused ("unknown option").
+ * Environment only: KIDMP_PIPE_CHUNK (columns per chunk of kidmp_step's host pipeline; a smaller "chunk" takes its place,
+ *   so that every pipeline chunk is one launch), KIDMP_ZEROCOPY=0 (copy whole chunks back instead of writing the changed
+ *   columns into pinned host arrays), KIDMP_PIPE_TRACE=1 (device timeline of every chunk of kidmp_step on stderr). */
 int kidmp_set_option(kidmp_handle* h, const char* name, int value);
 
 /* Multi-device handles (kidmp_config::ndev > 1).  kidmp_step, kidmp_kid_interface and the resident-state calls cut the
@@ -236,7 +230,7 @@ int kidmp_num_devices(const kidmp_handle* h);
 
 /* bookkeeping for benchmarks */
 long kidmp_gpu_launches(const kidmp_handle* h);         /* kernels launched so far          */
-/* counts of the last launch of the step kernels on every work set the last step used (waits for it): 0 cloudy columns, 1 busy
+/* counts of the last launch of the step kernels in the last step (waits for it): 0 cloudy columns, 1 busy
  * cells, 2-5 busy cells of the warm / ice / mixed-without-rain / full cell kernels, 6 columns with sedimentation sub-steps,
  * 7 whether the last kidmp_step returned only the changed columns (pinned host arrays, see kidmp_step) */
 int kidmp_step_stats(kidmp_handle* h, long out[8]);

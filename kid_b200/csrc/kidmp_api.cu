@@ -24,7 +24,6 @@ using namespace kidmp;
 // kernel groups of one launch, in launch order (kidmp_kernel_names / kidmp_last_kernel_ms)
 enum { KT_CLASSIFY = 0, KT_LISTS, KT_N0, KT_WARM, KT_ICE, KT_MIXNR, KT_FULL, KT_CARRIES, KT_SUBSTEPS, KT_FINISH, KT_DIAG, KT_N };
 
-constexpr int MAX_LANES = 8;
 struct WorkSet {
   float* d_scratch = nullptr;                             // [nz*cols][SC_REC] hand-off records of the busy cells
   unsigned char* d_cls = nullptr;                         // [nz][cols] class byte of every cell
@@ -38,11 +37,10 @@ struct WorkSet {
   double* d_coldiag = nullptr;                            // [2][cols] per-column water paths for the ordered domain sums
   int* d_colwork = nullptr;                               // [8 busy words | 8 colint | sub list | 2 colvmax][cols] of the column kernels
   long cols = 0; int nz = 0;
-  cudaStream_t s = nullptr;                               // this lane's stream (a single-lane step runs on the caller's stream instead)
   cudaStream_t aux = nullptr;                             // second stream of a launch: k_n0_sweep, k_substeps
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_dag[4] = {}, ev_done = nullptr;
-  cudaEvent_t ev_lists = nullptr;                         // the cell list of this set's current launch is complete (its cell kernels come next)
-  bool used = false;                                      // by the last step
+  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+  cudaEvent_t ev_lists_done = nullptr;                    // the work list is complete: k_n0_sweep may start
+  cudaEvent_t ev_n0_done = nullptr;                       // k_n0_sweep is done: the cell kernels with graupel may start
 };
 
 struct kidmp_handle {
@@ -58,7 +56,6 @@ struct kidmp_handle {
   char* d_tables = nullptr; size_t tables_bytes = 0;   // the slab behind tabs
   double* d_tnc_wev = nullptr;                          // table_dropEvap (M:4400-4439), made by the first aerosol-aware step
   float* d_aero = nullptr; size_t aero_floats = 0;      // staging of kidmp_mp_gt_driver_aero
-  size_t l2_window_bytes = 0; float l2_hit_ratio = 0.f; // L2 access-policy window over the slab (0: none)
   float table_ms = 0.f;
   bool tables_from_cache = false;
   long launches = 0;
@@ -70,14 +67,9 @@ struct kidmp_handle {
   float* d_ppt = nullptr;        // [4][ncol]
   float* d_stage = nullptr;      // staging for layout conversion, [nz][ncol]
   double* d_partial = nullptr; long partial_chunks = 0;   // [chunks of one step][DIAG_BLOCKS][KIDMP_NDIAG] block sums of the domain diagnostics
-  // Work buffers of one launch (a chunk of at most chunk_cols columns), sized for the worst case of the chunk.  A step over a
-  // large domain is cut into sub-chunks that run on `lanes` work sets, each with its own streams: the HBM-bound kernels of
-  // one sub-chunk (classification, lists, carries, finish) run beside the issue-bound cell kernels of another.
-  WorkSet ws[MAX_LANES];
-  int lanes = 1;                                          // work sets used side by side ("lanes" option, KIDMP_LANES)
-  long lane_min_cols = 131072;                            // no sub-chunk smaller than this ("lane_min" option)
-  int cell_blocks = 0;                                    // blocks per SM of the cell kernels when several lanes run (0: the kernel's own)
-  // The launches of a step that is one chunk on one lane are captured once in a CUDA graph and replayed while the arguments stay
+  // Work buffers of one launch (a chunk of at most chunk_cols columns), sized for the worst case of the chunk
+  WorkSet ws;
+  // The launches of a step of up to 64 chunks are captured once in a CUDA graph and replayed while the arguments stay
   // the same ("graphs" option, KIDMP_GRAPHS; KIDMP_GRAPH_MAX: largest domain): a small domain is launch-bound (fifteen kernels of
   // a few microseconds: 0.297 -> 0.277 ms for one column), the 1 048 576-column step loses its launch gaps (3.45 -> 3.425 ms)
   int graphs = 1; long graph_max_cols = 1L << 24;
@@ -85,10 +77,6 @@ struct kidmp_handle {
   StepGraph graph_cache[8]; int graph_next = 0;        // a few steps at a time: the three rotating buffers of kidmp_step's pipeline, resident state, a caller's arrays
   int simple = 1;                                         // "simple" option: columns without sub-steps skip k_carries (kidmp_cells.cuh)
   int classes = 1;                                        // "classes" option: 0 sends every busy cell to the general cell kernel (tests)
-  int l2_window = 1;                                      // "l2_window" option: the cell kernels that gather from the tables carry the window
-  int stagger = 0;                                        // "stagger" option: see launch_step
-  int lanes_used = 1;                                     // work sets of the last step
-  cudaEvent_t ev_start = nullptr;                         // the lanes of a step start after this point of the caller's stream
   // "timing" option: the kernels of a launch run one after the other on one stream with an event after each
   bool last_zero_copy = false;                            // the last kidmp_step wrote the changed columns straight into pinned host arrays
   int timing = 0; bool timing_valid = false;             // 1: kernels serialised on one stream; 2: the normal schedule, events on the main stream only
@@ -291,27 +279,14 @@ void free_work(WorkSet& w) {
   w.d_scratch = nullptr; w.d_cls = nullptr; w.d_colflag = nullptr; w.d_work = nullptr; w.d_cells = nullptr;
   w.d_cellmeta = nullptr; w.d_coldiag = nullptr; w.d_colwork = nullptr; w.d_cellidx = nullptr; w.d_ws = nullptr; w.d_n0a = nullptr; w.cols = 0; w.nz = 0;
 }
-// The streams of the work sets are made at init, before the host makes its own: measured on the bench (a PyTorch stream made
-// after kidmp_init), a second stream made at the first step instead left k_substeps running 0.2 ms past k_finish.
-int ensure_streams(kidmp_handle* h, WorkSet& w, bool own_stream) {
-  if (own_stream && !w.s) CK(h, cudaStreamCreateWithFlags(&w.s, cudaStreamNonBlocking));
-  if (!w.aux) {
-    bool ok = cudaStreamCreateWithFlags(&w.aux, cudaStreamNonBlocking) == cudaSuccess &&
-              cudaEventCreateWithFlags(&w.ev_fork, cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&w.ev_join, cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&w.ev_done, cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&w.ev_lists, cudaEventDisableTiming) == cudaSuccess;
-    for (int q = 0; q < 4 && ok; ++q) ok = cudaEventCreateWithFlags(&w.ev_dag[q], cudaEventDisableTiming) == cudaSuccess;
-    if (!ok) return fail(h, "stream/event creation failed");
-  }
-  return 0;
-}
-int ensure_work(kidmp_handle* h, WorkSet& w, long cols, int nz, bool own_stream) {
-  if (ensure_streams(h, w, own_stream)) return 1;
+int ensure_work(kidmp_handle* h, long cols, int nz) {
+  WorkSet& w = h->ws;
   if (cols <= w.cols && nz <= w.nz) return 0;
   const long C = cols > w.cols ? cols : w.cols;
   const int Z = nz > w.nz ? nz : w.nz;
-  CK(h, cudaDeviceSynchronize());                    // nothing may still be reading the buffers that go away
+  // Only this handle's steps use the buffers that go away, and each has ended at ev_done (the k_scatter_host that follows a
+  // pipelined step is waited for before step_pipelined returns).  A device-wide wait would also fail another thread's capture.
+  CK(h, cudaEventSynchronize(h->ev_done));
   free_work(w);
   const size_t cells = (size_t)C * Z;
   const long ngroups = (C + 31) / 32, lblocks = (C + LIST_TILE - 1) / LIST_TILE;
@@ -369,8 +344,6 @@ int ensure_work(kidmp_handle* h, WorkSet& w, long cols, int nz, bool own_stream)
 #define KC_FULL_BARS 11
 #endif
 
-// `bps`: blocks per SM (0: as many as the kernel's launch bounds allow).  With several lanes a cell kernel that left no
-// register of an SM free would keep the other lanes' HBM-bound kernels out until its last block retires.
 #ifndef KC_AERO_WARM_B
 #define KC_AERO_WARM_B 3
 #endif
@@ -381,73 +354,48 @@ int ensure_work(kidmp_handle* h, WorkSet& w, long cols, int nz, bool own_stream)
 #define KC_AERO_MIX_B 2
 #endif
 template <bool RATES, bool AERO>
-void launch_cells(kidmp_handle* h, const StepArgs& a, int nsm, cudaStream_t s, cudaEvent_t n0_done, int bps) {
+void launch_cells(kidmp_handle* h, const StepArgs& a, int nsm, cudaStream_t s, cudaEvent_t n0_done) {
   auto mark = [&](int q) { if (h->timing) cudaEventRecord(h->ev_k[q + 1], s); };
-  auto grid = [&](int own) { return (unsigned)(nsm * (bps > 0 && bps < own ? bps : own)); };
   // (the aerosol-aware instantiations carry more live values: one block per SM less keeps them out of local memory)
   constexpr int WB = AERO ? KC_AERO_WARM_B : KC_WARM_B, IB = AERO ? KC_AERO_ICE_B : KC_ICE_B, MB = AERO ? KC_AERO_MIX_B : KC_MIXNR_B,
                 FB = AERO ? KC_AERO_MIX_B : KC_FULL_B;
-  k_cells<KC_WARM, KC_WARM_T, WB, KC_WARM_BARS, RATES, AERO><<<grid(WB), KC_WARM_T, 0, s>>>(a);
+  k_cells<KC_WARM, KC_WARM_T, WB, KC_WARM_BARS, RATES, AERO><<<nsm * WB, KC_WARM_T, 0, s>>>(a);
   mark(KT_WARM);
-  k_cells<KC_ICE, KC_ICE_T, IB, KC_ICE_BARS, RATES, AERO><<<grid(IB), KC_ICE_T, 0, s>>>(a);
+  k_cells<KC_ICE, KC_ICE_T, IB, KC_ICE_BARS, RATES, AERO><<<nsm * IB, KC_ICE_T, 0, s>>>(a);
   mark(KT_ICE);
   if (n0_done) cudaStreamWaitEvent(s, n0_done, 0);     // only the classes with graupel read the intercept minima of k_n0_sweep
-  // The two classes that gather from the big tables (qcfz / iaus: mixed; racs, racg, qrfz: full) run with an L2
-  // access-policy window over the table slab: table lines persist, the streamed state and records do not evict them.
-  cudaLaunchAttribute att[1];
-  att[0].id = cudaLaunchAttributeAccessPolicyWindow;
-  att[0].val.accessPolicyWindow.base_ptr = h->d_tables;
-  att[0].val.accessPolicyWindow.num_bytes = h->l2_window_bytes;
-  att[0].val.accessPolicyWindow.hitRatio = h->l2_hit_ratio;
-  att[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-  att[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-  cudaLaunchConfig_t cfg{};
-  cfg.blockDim = dim3(KC_MIXNR_T); cfg.gridDim = dim3(grid(MB)); cfg.dynamicSmemBytes = 0; cfg.stream = s;
-  cfg.attrs = att; cfg.numAttrs = (h->l2_window_bytes && h->l2_window) ? 1 : 0;
-  cudaLaunchKernelEx(&cfg, k_cells<KC_MIXNR, KC_MIXNR_T, MB, KC_MIXNR_BARS, RATES, AERO>, a);
+  k_cells<KC_MIXNR, KC_MIXNR_T, MB, KC_MIXNR_BARS, RATES, AERO><<<nsm * MB, KC_MIXNR_T, 0, s>>>(a);
   mark(KT_MIXNR);
-  cfg.blockDim = dim3(KC_FULL_T); cfg.gridDim = dim3(grid(FB));
-  cudaLaunchKernelEx(&cfg, k_cells<KC_FULL, KC_FULL_T, FB, KC_FULL_BARS, RATES, AERO>, a);
+  k_cells<KC_FULL, KC_FULL_T, FB, KC_FULL_BARS, RATES, AERO><<<nsm * FB, KC_FULL_T, 0, s>>>(a);
   mark(KT_FULL);
 }
 
-// One step over [ncol] columns whose arrays have row stride ld, in launches of at most chunk_cols columns (the work
-// buffers are sized for one launch: 29 hand-off planes would otherwise grow with the domain).  Columns are independent,
-// so the chunking changes no result.  A large domain is cut into at least `lanes` launches that run on as many work sets
-// and streams: the kernels of a launch alternate between HBM-bound (classification, carries, finish) and issue-bound
-// (cells), and side by side they fill each other's idle resource.  A small domain or a timing-mode step is one launch
-// after the other on the caller's stream.
+// One step over [ncol] columns whose arrays have row stride ld, in launches of at most chunk_cols columns on the caller's
+// stream (the work buffers are sized for one launch: 29 hand-off planes would otherwise grow with the domain).  Columns are
+// independent, so the chunking changes no result.
 int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
   if (a0.nz < 2 || a0.nz > 256) return fail(h, "nz=%d outside [2,256]", a0.nz);
   if (a0.ncol < 1) return fail(h, "ncol=%ld", a0.ncol);
   if (!(a0.dt > 0.f)) return fail(h, "dt must be positive");
-  long chunk = h->chunk_cols;
-  if (!h->timing && h->lanes > 1 && a0.ncol >= 2 * h->lane_min_cols) {
-    long sub = (a0.ncol + h->lanes - 1) / h->lanes;
-    sub = (sub + 1023) / 1024 * 1024;                  // launches start on whole 128-byte lines of the caller's rows
-    if (sub < h->lane_min_cols) sub = h->lane_min_cols;
-    if (sub < chunk) chunk = sub;
-  }
+  const long chunk = h->chunk_cols;
   const long cap = a0.ncol < chunk ? a0.ncol : chunk;
   const long nchunks = (a0.ncol + chunk - 1) / chunk;
-  const int nl = (h->timing || h->lanes <= 1 || nchunks < 2) ? 1 : (int)(nchunks < h->lanes ? nchunks : h->lanes);
   if (cap > (1L << 24)) return fail(h, "chunk of %ld columns: at most 16 777 216 per launch (set_option \"chunk\")", cap);
   if ((double)cap * a0.nz >= 4.0e9) return fail(h, "chunk of %ld columns x %d levels does not fit the 32-bit cell index", cap, a0.nz);
-  for (int l = 0; l < nl; ++l) if (ensure_work(h, h->ws[l], cap, a0.nz, l > 0)) return 1;   // (lane 0 runs on the caller's stream)
-  // the work sets are the handle's: a step on another stream than the last one starts after it
+  if (ensure_work(h, cap, a0.nz)) return 1;
+  // the work set is the handle's: a step on another stream than the last one starts after it
   CK(h, cudaStreamWaitEvent(s, h->ev_done, 0));
   if (ensure_constants(h, s)) return 1;
   if (h->partial_chunks < nchunks) {
-    if (h->d_partial) { CK(h, cudaDeviceSynchronize()); cudaFree(h->d_partial); h->d_partial = nullptr; h->partial_chunks = 0; }
+    if (h->d_partial) { CK(h, cudaEventSynchronize(h->ev_done)); cudaFree(h->d_partial); h->d_partial = nullptr; h->partial_chunks = 0; }
     CK(h, cudaMalloc((void**)&h->d_partial, (size_t)nchunks * DIAG_BLOCKS * KIDMP_NDIAG * 8));
     h->partial_chunks = nchunks;
   }
-  // One lane: replay the captured graph of this very step (all its chunks), or capture it now.
-  const bool graphable = h->graphs && !h->timing && nchunks <= 64 && nl == 1 && a0.ncol <= h->graph_max_cols;
-  // (a handle setting that a captured launch reads belongs in the key: a replay after the setting changed would run the old one.
-  // "stagger" and "cell_blocks" are not in it: they act only when a step runs on several lanes, which is never captured)
-  const long gkey[7] = {(long)(size_t)h->ws[0].d_scratch, h->ws[0].cols, (long)h->ws[0].nz, (long)h->simple, (long)(size_t)h->d_partial,
-                        (long)h->l2_window * 2 + chunk * 4, (long)h->classes};
+  // Replay the captured graph of this very step (all its chunks), or capture it now.
+  const bool graphable = h->graphs && !h->timing && nchunks <= 64 && a0.ncol <= h->graph_max_cols;
+  // (a handle setting that a captured launch reads belongs in the key: a replay after the setting changed would run the old one)
+  const long gkey[7] = {(long)(size_t)h->ws.d_scratch, h->ws.cols, (long)h->ws.nz, (long)h->simple, (long)(size_t)h->d_partial,
+                        chunk, (long)h->classes};
   kidmp_handle::StepGraph* hit = nullptr;
   if (graphable)
     for (auto& g : h->graph_cache)
@@ -455,8 +403,6 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
   if (hit) {
     CK(h, cudaGraphLaunch(hit->exec, s));
     h->launches += hit->launches;
-    for (int l = 0; l < MAX_LANES; ++l) h->ws[l].used = l == 0;
-    h->lanes_used = 1;
     h->timing_valid = false;
     CK(h, cudaEventRecord(h->ev_done, s));
     h->last_on_own_stream = (s == h->stream);
@@ -475,19 +421,11 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
     cudaStream_t s; bool* on;
     ~CaptureGuard() { if (*on) { cudaGraph_t g = nullptr; cudaStreamEndCapture(s, &g); if (g) cudaGraphDestroy(g); cudaGetLastError(); } }
   } capture_guard{s, &capturing};
-  if (nl > 1) {
-    CK(h, cudaEventRecord(h->ev_start, s));
-    for (int l = 1; l < nl; ++l) CK(h, cudaStreamWaitEvent(h->ws[l].s, h->ev_start, 0));
-  }
   // the handle's own rate buffer starts every step at zero: clear-sky columns have no process at all
   if (a0.rates && a0.rates == h->d_rates_own) CK(h, cudaMemsetAsync(h->d_rates_own, 0, (size_t)KIDMP_NRATES * a0.nz * a0.ld * 4, s));
-  for (int l = 0; l < MAX_LANES; ++l) h->ws[l].used = l < nl;
-  h->lanes_used = nl;
-  const int bps = nl > 1 ? h->cell_blocks : 0;
+  const WorkSet& w = h->ws;
   long ci = 0;
   for (long c0 = 0; c0 < a0.ncol; c0 += chunk, ++ci) {
-    WorkSet& w = h->ws[ci % nl];
-    cudaStream_t cs = (ci % nl) ? w.s : s;
     StepArgs a = a0;
     a.ncol = (a0.ncol - c0 < chunk) ? (a0.ncol - c0) : chunk;
     for (int q = 0; q < KIDMP_NFIELDS; ++q) a.f[q] = a0.f[q] + c0;
@@ -507,64 +445,55 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
     a.no_classes = h->classes ? 0 : 1;
     // second stream of the launch; in timing mode everything runs on one stream, one kernel after the other
     const bool serial = h->timing == 1;
-    cudaStream_t x = serial ? cs : w.aux;
-    auto mark = [&](int q) { if (h->timing) cudaEventRecord(h->ev_k[q + 1], cs); };
+    cudaStream_t x = serial ? s : w.aux;
+    auto mark = [&](int q) { if (h->timing) cudaEventRecord(h->ev_k[q + 1], s); };
     auto fork = [&](cudaEvent_t e, cudaStream_t from, cudaStream_t to) {
       if (from != to) { cudaEventRecord(e, from); cudaStreamWaitEvent(to, e, 0); }
     };
-    // Stagger the lanes: a launch starts its classification when the launch before it (on the neighbouring lane) has
-    // its cell list, i.e. its HBM-bound front runs beside that launch's cell kernels instead of beside its front.
-    if (nl > 1 && ci > 0 && h->stagger) CK(h, cudaStreamWaitEvent(cs, h->ws[(ci - 1) % nl].ev_lists, 0));
-    CK(h, cudaMemsetAsync(w.d_cellmeta, 0, 128 * 4, cs));
-    if (h->timing) CK(h, cudaEventRecord(h->ev_k[0], cs));
-    k_classify<<<(unsigned)((a.ncol + 127) / 128), 128, 0, cs>>>(a);
-    CK(h, cudaMemsetAsync(a.colvmax, 0, (size_t)2 * w.cols * 4, cs));
+    CK(h, cudaMemsetAsync(w.d_cellmeta, 0, 128 * 4, s));
+    if (h->timing) CK(h, cudaEventRecord(h->ev_k[0], s));
+    k_classify<<<(unsigned)((a.ncol + 127) / 128), 128, 0, s>>>(a);
+    CK(h, cudaMemsetAsync(a.colvmax, 0, (size_t)2 * w.cols * 4, s));
     mark(KT_CLASSIFY);
     // The classification left the key histogram of the busy cells: first entry of every key and class, the work list of
     // the cloudy columns, then the list of the busy cells.  Second stream: the graupel intercept sweep (needs the work list
     // only; the cell kernels with graupel wait for it).
-    k_cell_offsets<<<1, 64, 0, cs>>>(a);
-    k_list_scan<<<1, 1024, 0, cs>>>(a.work_mask, (int)ngroups, a.work_offset, a.work_count);
-    k_list_fill<<<(unsigned)((ngroups * 32 + 255) / 256), 256, 0, cs>>>(a.work_mask, a.work_offset, (int)ngroups, a.work_list);
+    k_cell_offsets<<<1, 64, 0, s>>>(a);
+    k_list_scan<<<1, 1024, 0, s>>>(a.work_mask, (int)ngroups, a.work_offset, a.work_count);
+    k_list_fill<<<(unsigned)((ngroups * 32 + 255) / 256), 256, 0, s>>>(a.work_mask, a.work_offset, (int)ngroups, a.work_list);
     if (serial) {
-      k_cell_fill<<<(unsigned)lblocks, LIST_TILE, 0, cs>>>(a);
+      k_cell_fill<<<(unsigned)lblocks, LIST_TILE, 0, s>>>(a);
       mark(KT_LISTS);
-      if (!h->kc.iiwarm) k_n0_sweep<<<(unsigned)((a.ncol + 127) / 128), 128, 0, cs>>>(a);
+      if (!h->kc.iiwarm) k_n0_sweep<<<(unsigned)((a.ncol + 127) / 128), 128, 0, s>>>(a);
       mark(KT_N0);
     } else {
-      fork(w.ev_dag[2], cs, x);                      // (recorded after k_list_fill)
+      fork(w.ev_lists_done, s, x);                   // (recorded after k_list_fill)
       // the number of cloudy columns is only known on the device: grids for the worst case, surplus blocks leave at once
       if (!h->kc.iiwarm) k_n0_sweep<<<(unsigned)((a.ncol + 127) / 128), 128, 0, x>>>(a);
-      k_cell_fill<<<(unsigned)lblocks, LIST_TILE, 0, cs>>>(a);
-      CK(h, cudaEventRecord(w.ev_dag[3], x));        // the sweep runs beside k_cell_fill and the warm and ice cell kernels
+      k_cell_fill<<<(unsigned)lblocks, LIST_TILE, 0, s>>>(a);
+      CK(h, cudaEventRecord(w.ev_n0_done, x));       // the sweep runs beside k_cell_fill and the warm and ice cell kernels
       mark(KT_LISTS); mark(KT_N0);
     }
-    if (nl > 1) CK(h, cudaEventRecord(w.ev_lists, cs));
-    cudaEvent_t n0_done = serial ? nullptr : w.ev_dag[3];
+    cudaEvent_t n0_done = serial ? nullptr : w.ev_n0_done;
     const bool aero = a.nc != nullptr;                  // (an aerosol-aware step has no process-rate buffer: checked by its entry point)
-    if (aero) launch_cells<false, true>(h, a, h->nsm, cs, n0_done, bps);
-    else if (a.rates) launch_cells<true, false>(h, a, h->nsm, cs, n0_done, bps);
-    else launch_cells<false, false>(h, a, h->nsm, cs, n0_done, bps);
-    k_carries<<<(unsigned)((a.ncol + 63) / 64), 64, 0, cs>>>(a);
+    if (aero) launch_cells<false, true>(h, a, h->nsm, s, n0_done);
+    else if (a.rates) launch_cells<true, false>(h, a, h->nsm, s, n0_done);
+    else launch_cells<false, false>(h, a, h->nsm, s, n0_done);
+    k_carries<<<(unsigned)((a.ncol + 63) / 64), 64, 0, s>>>(a);
     mark(KT_CARRIES);
     // the columns with sedimentation sub-steps on the second stream, the others on this one: disjoint columns
-    fork(w.ev_fork, cs, x);
+    fork(w.ev_fork, s, x);
     const unsigned sgrid = (unsigned)(ngroups < h->nsm * 16 ? ngroups : h->nsm * 16);
     if (aero) k_substeps<false, true><<<sgrid, 32, 0, x>>>(a);
     else if (a.rates) k_substeps<true, false><<<sgrid, 32, 0, x>>>(a); else k_substeps<false, false><<<sgrid, 32, 0, x>>>(a);
     mark(KT_SUBSTEPS);
-    if (aero) k_finish<false, true><<<(unsigned)ngroups, 32, 0, cs>>>(a);
-    else if (a.rates) k_finish<true, false><<<(unsigned)ngroups, 32, 0, cs>>>(a); else k_finish<false, false><<<(unsigned)ngroups, 32, 0, cs>>>(a);
+    if (aero) k_finish<false, true><<<(unsigned)ngroups, 32, 0, s>>>(a);
+    else if (a.rates) k_finish<true, false><<<(unsigned)ngroups, 32, 0, s>>>(a); else k_finish<false, false><<<(unsigned)ngroups, 32, 0, s>>>(a);
     mark(KT_FINISH);
-    fork(w.ev_join, x, cs);
-    k_diag_columns<<<DIAG_BLOCKS, 256, 0, cs>>>(a, (a.ncol + DIAG_BLOCKS - 1) / DIAG_BLOCKS);
+    fork(w.ev_join, x, s);
+    k_diag_columns<<<DIAG_BLOCKS, 256, 0, s>>>(a, (a.ncol + DIAG_BLOCKS - 1) / DIAG_BLOCKS);
     h->launches += h->kc.iiwarm ? 13 : 14;
   }
-  if (nl > 1)
-    for (int l = 1; l < nl; ++l) {
-      CK(h, cudaEventRecord(h->ws[l].ev_done, h->ws[l].s));
-      CK(h, cudaStreamWaitEvent(s, h->ws[l].ev_done, 0));
-    }
   // the block sums of all launches, in column order
   k_diag_reduce<<<KIDMP_NDIAG, 256, 0, s>>>(h->d_partial, (int)(nchunks * DIAG_BLOCKS), h->d_diag);
   ++h->launches;
@@ -882,10 +811,6 @@ int kidmp_init(const kidmp_config* cfg, kidmp_handle** out) {
   h->device = dev1;
   if (getenv("KIDMP_CHUNK") && atol(getenv("KIDMP_CHUNK")) >= 32) h->chunk_cols = atol(getenv("KIDMP_CHUNK"));
   if (dev1 >= MAX_DEVICES) { delete h; return fail(nullptr, "kidmp_init: device ordinal %d not supported", dev1); }
-  if (getenv("KIDMP_LANES")) { const int v = atoi(getenv("KIDMP_LANES")); h->lanes = v < 1 ? 1 : v > MAX_LANES ? MAX_LANES : v; }
-  if (getenv("KIDMP_LANE_MIN") && atol(getenv("KIDMP_LANE_MIN")) >= 1024) h->lane_min_cols = atol(getenv("KIDMP_LANE_MIN"));
-  if (getenv("KIDMP_CELL_BLOCKS")) h->cell_blocks = atoi(getenv("KIDMP_CELL_BLOCKS"));
-  if (getenv("KIDMP_STAGGER")) h->stagger = atoi(getenv("KIDMP_STAGGER"));
   if (getenv("KIDMP_SIMPLE")) h->simple = atoi(getenv("KIDMP_SIMPLE")) != 0;
   if (getenv("KIDMP_GRAPHS")) h->graphs = atoi(getenv("KIDMP_GRAPHS")) != 0;
   if (getenv("KIDMP_GRAPH_MAX") && atol(getenv("KIDMP_GRAPH_MAX")) > 0) h->graph_max_cols = atol(getenv("KIDMP_GRAPH_MAX"));
@@ -899,13 +824,19 @@ int kidmp_init(const kidmp_config* cfg, kidmp_handle** out) {
   cudaGetDeviceProperties(&prop, h->device);
   h->nsm = prop.multiProcessorCount;
   if (prop.major < 10) { fail(h, "kidmp_init: built for sm_100a, device is sm_%d%d", prop.major, prop.minor); return bail(1); }
+  // The second stream of a launch is made here, before the host makes its own: measured on the bench (a PyTorch stream made
+  // after kidmp_init), a second stream made at the first step instead left k_substeps running 0.2 ms past k_finish.
+  WorkSet& w = h->ws;
   if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaEventCreate(&h->ev0) != cudaSuccess || cudaEventCreate(&h->ev1) != cudaSuccess ||
       cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&h->ev_start, cudaEventDisableTiming) != cudaSuccess) {
+      cudaStreamCreateWithFlags(&w.aux, cudaStreamNonBlocking) != cudaSuccess ||
+      cudaEventCreateWithFlags(&w.ev_fork, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&w.ev_join, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&w.ev_lists_done, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&w.ev_n0_done, cudaEventDisableTiming) != cudaSuccess) {
     h->err = "stream/event creation failed"; return bail(1);
   }
-  for (int l = 0; l < h->lanes; ++l) if (ensure_streams(h, h->ws[l], l > 0)) return bail(1);
   for (int q = 0; q <= KT_N; ++q) if (cudaEventCreate(&h->ev_k[q]) != cudaSuccess) {
     h->err = "stream/event creation failed"; return bail(1);
   }
@@ -916,7 +847,7 @@ int kidmp_init(const kidmp_config* cfg, kidmp_handle** out) {
   h->kc.t_Nc1 = h->hb.t_Nc[0];
   publish_constants(h);
   {
-    // one slab for all lookup tables (the gathered ones first): one L2 access-policy window covers them
+    // one slab for all lookup tables: one allocation, freed in one call
     size_t total = 0;
     for (auto& a : table_allocs(h)) total += (a.bytes + 255) / 256 * 256;
     if (cudaMalloc((void**)&h->d_tables, total) != cudaSuccess || cudaMemset(h->d_tables, 0, total) != cudaSuccess) {
@@ -925,22 +856,6 @@ int kidmp_init(const kidmp_config* cfg, kidmp_handle** out) {
     h->tables_bytes = total;
     size_t off = 0;
     for (auto& a : table_allocs(h)) { *a.p = h->d_tables + off; off += (a.bytes + 255) / 256 * 256; }
-    // L2 set-aside for the window (north_star: "lookup tables staged in ... L2-persisting windows"): as much of the slab as
-    // the device allows.  Only the cell kernels that gather from the collection / freezing tables carry the window.
-    int max_persist = 0, max_window = 0;
-    cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, h->device);
-    cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, h->device);
-    size_t want = total < (size_t)max_persist ? total : (size_t)max_persist;
-    // MEASURED (profiles/r02_ncu_step_kernels.md, "What did not pay"): with the set-aside (the device grants ~3/5 of L2) the step goes from 3.51 to 5.1 ms -
-    // k_finish 0.68 -> 1.46 ms, k_carries 0.33 -> 0.62, even k_cells<FULL> 0.35 -> 0.48: the records and the state stream
-    // through what is left of L2, and only ~2 % of the busy cells gather from the big tables.  So the window is OFF unless
-    // KIDMP_L2_WINDOW=1 asks for it at init.
-    if (!(getenv("KIDMP_L2_WINDOW") && atoi(getenv("KIDMP_L2_WINDOW")) != 0)) want = 0;
-    if (want && max_window > 0 && cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
-      h->l2_window_bytes = total < (size_t)max_window ? total : (size_t)max_window;
-      h->l2_hit_ratio = h->l2_window_bytes <= want ? 1.0f : (float)want / (float)h->l2_window_bytes;
-    }
-    cudaGetLastError();
   }
   if (cudaMalloc((void**)&h->d_diag, KIDMP_NDIAG * 8) != cudaSuccess || cudaMemset(h->d_diag, 0, KIDMP_NDIAG * 8) != cudaSuccess) {
     h->err = "diag allocation failed"; return bail(1);
@@ -974,7 +889,9 @@ int kidmp_finalize(kidmp_handle* h) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (g_const_owner[h->device] == h) g_const_owner[h->device] = nullptr;
   }
-  cudaDeviceSynchronize();                           // steps may have run on caller streams
+  // what this handle enqueued: steps end at ev_done (on whatever stream they ran), copies and staging on its own streams
+  if (h->ev_done) cudaEventSynchronize(h->ev_done);
+  for (cudaStream_t s : {h->stream, h->copy_in, h->copy_out}) if (s) cudaStreamSynchronize(s);
   free_state(h);
   for (auto& g : h->graph_cache) if (g.exec) cudaGraphExecDestroy(g.exec);
   if (h->d_tables) cudaFree(h->d_tables);
@@ -984,17 +901,9 @@ int kidmp_finalize(kidmp_handle* h) {
   if (h->d_diag) cudaFree(h->d_diag);
   if (h->d_kid) cudaFree(h->d_kid);
   if (h->h_kid) cudaFreeHost(h->h_kid);
-  for (WorkSet& w : h->ws) {
-    free_work(w);
-    if (w.ev_fork) cudaEventDestroy(w.ev_fork);
-    if (w.ev_join) cudaEventDestroy(w.ev_join);
-    if (w.ev_done) cudaEventDestroy(w.ev_done);
-    if (w.ev_lists) cudaEventDestroy(w.ev_lists);
-    for (int q = 0; q < 4; ++q) if (w.ev_dag[q]) cudaEventDestroy(w.ev_dag[q]);
-    if (w.aux) cudaStreamDestroy(w.aux);
-    if (w.s) cudaStreamDestroy(w.s);
-  }
-  if (h->ev_start) cudaEventDestroy(h->ev_start);
+  free_work(h->ws);
+  for (cudaEvent_t e : {h->ws.ev_fork, h->ws.ev_join, h->ws.ev_lists_done, h->ws.ev_n0_done}) if (e) cudaEventDestroy(e);
+  if (h->ws.aux) cudaStreamDestroy(h->ws.aux);
   for (int q = 0; q <= KT_N; ++q) if (h->ev_k[q]) cudaEventDestroy(h->ev_k[q]);
   if (h->ev_done) cudaEventDestroy(h->ev_done);
   if (h->d_pipe) cudaFree(h->d_pipe);
@@ -1190,7 +1099,7 @@ int kidmp_enable_rates(kidmp_handle* h, int on) {
   }
   DevGuard guard_(h->device);
   h->rates_on = on != 0;
-  if (!h->rates_on && h->d_rates_own) { CK(h, cudaDeviceSynchronize()); cudaFree(h->d_rates_own); h->d_rates_own = nullptr; }
+  if (!h->rates_on && h->d_rates_own) { CK(h, cudaEventSynchronize(h->ev_done)); cudaFree(h->d_rates_own); h->d_rates_own = nullptr; }
   if (h->rates_on && !h->d_rates_own && h->d_state)
     CK(h, cudaMalloc((void**)&h->d_rates_own, (size_t)h->ncol * h->nz * KIDMP_NRATES * 4));
   return 0;
@@ -1286,7 +1195,8 @@ int kidmp_download(kidmp_handle* h, int layout, float* const fields[KIDMP_NFIELD
 // of the same arrays.
 static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* const fields[KIDMP_NFIELDS],
                           const float* p, const float* dz, float* ppt, long hld) {
-  const long chunk = h->pipe_chunk;
+  // (no larger than a launch chunk: then every pipeline chunk is one launch of launch_step, whose column flags k_scatter_host reads)
+  const long chunk = h->pipe_chunk < h->chunk_cols ? h->pipe_chunk : h->chunk_cols;
   const int NB = 3;
   // (streams are made when they are first needed: the device has few hardware queues, and streams that share one
   // serialise kernels that could run side by side)
@@ -1359,7 +1269,7 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
       HostFields hc = hf;
       for (int q = 0; q < KIDMP_NFIELDS; ++q) hc.f[q] += c0;
       StepArgs sa = a;
-      sa.colflag = h->ws[0].d_colflag;               // (of this chunk, a single launch on work set 0: the next chunk's kernels follow on the same stream)
+      sa.colflag = h->ws.d_colflag;                  // (this chunk's flags: it was one launch, and the next chunk's kernels follow on this stream)
       k_scatter_host<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(sa, hc, hld);
       ++h->launches;
       CK(h, cudaEventRecord(h->pipe_ev[b][1], h->stream));
@@ -1743,25 +1653,10 @@ int kidmp_set_option(kidmp_handle* h, const char* name, int value) {
     if (value < 32) return fail(h, "set_option: chunk must be at least 32 columns");
     h->chunk_cols = value; return 0;
   }
-  if (!strcmp(name, "lanes")) {
-    if (value < 1 || value > MAX_LANES) return fail(h, "set_option: lanes must be 1..%d", MAX_LANES);
-    h->lanes = value; return 0;
-  }
-  if (!strcmp(name, "lane_min")) {
-    if (value < 1024) return fail(h, "set_option: lane_min must be at least 1024 columns");
-    h->lane_min_cols = value; return 0;
-  }
   if (!strcmp(name, "graphs")) { h->graphs = value != 0; return 0; }
   if (!strcmp(name, "simple")) { h->simple = value != 0; return 0; }
   if (!strcmp(name, "classes")) { h->classes = value != 0; return 0; }
-  if (!strcmp(name, "l2_window")) { h->l2_window = value != 0; return 0; }
-  if (!strcmp(name, "stagger")) { h->stagger = value != 0; return 0; }
-  if (!strcmp(name, "cell_blocks")) {
-    if (value < 0 || value > 8) return fail(h, "set_option: cell_blocks must be 0..8");
-    h->cell_blocks = value; return 0;
-  }
   if (!strcmp(name, "timing")) { h->timing = value < 0 ? 0 : value > 2 ? 2 : value; h->timing_valid = false; return 0; }
-  if (!strcmp(name, "fuse") || !strcmp(name, "units")) return 0;      // knobs of the round-1 kernels: accepted, no effect
   return fail(h, "set_option: unknown option '%s'", name);
 }
 
@@ -1798,14 +1693,13 @@ int kidmp_step_stats(kidmp_handle* h, long out[8]) {
   for (int q = 0; q < 8; ++q) out[q] = 0;
   DevGuard guard_(h->device);
   CK(h, cudaEventSynchronize(h->ev_done));
-  for (const WorkSet& w : h->ws) {                     // the last launch of every work set the last step used
-    if (!w.used || !w.d_cellmeta) continue;
+  if (h->ws.d_cellmeta) {                               // the last launch of the last step
     int meta[8], cloudy = 0;
-    CK(h, cudaMemcpy(meta, w.d_cellmeta, sizeof meta, cudaMemcpyDeviceToHost));
-    CK(h, cudaMemcpy(&cloudy, w.d_work, 4, cudaMemcpyDeviceToHost));
-    out[0] += cloudy; out[1] += meta[KC_N];
-    for (int q = 0; q < KC_N; ++q) out[2 + q] += meta[q];
-    out[6] += meta[5];
+    CK(h, cudaMemcpy(meta, h->ws.d_cellmeta, sizeof meta, cudaMemcpyDeviceToHost));
+    CK(h, cudaMemcpy(&cloudy, h->ws.d_work, 4, cudaMemcpyDeviceToHost));
+    out[0] = cloudy; out[1] = meta[KC_N];
+    for (int q = 0; q < KC_N; ++q) out[2 + q] = meta[q];
+    out[6] = meta[5];
   }
   out[7] = h->last_zero_copy ? 1 : 0;
   return 0;
