@@ -10,7 +10,6 @@
 #include <string>
 #include <vector>
 #include <map>
-#include <mutex>
 #include "kidmp_internal.h"
 #include "kidmp_hostinit.h"
 #include "kidmp_tables.cuh"
@@ -50,6 +49,8 @@ struct kidmp_handle {
   int device = 0;
   cudaStream_t stream = nullptr, copy_in = nullptr, copy_out = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  // The scalars of thompson_init.  Every kernel that reads them gets this copy as a launch parameter (a captured graph keeps
+  // its own), so handles on one device share nothing: several may step at the same time, from different threads.
   KConst kc;
   HostBins hb;
   TableSet tabs{};
@@ -101,7 +102,6 @@ struct kidmp_handle {
 namespace {
 
 std::string g_init_error;
-std::mutex g_mu;
 
 // Every entry point leaves the caller's current CUDA device as it found it (the host may be PyTorch or KiD's own code).
 struct DevGuard {
@@ -255,24 +255,6 @@ int build_device_tables(kidmp_handle* h, const hostinit::Prep& pp) {
   return 0;
 }
 
-// The scalars of thompson_init live in ONE __constant__ block per device (`ck`) and one __device__ double (the graupel
-// intercept constant): the handle that ran last on a device owns them.  A change of owner is ordered on the device: the
-// new owner's stream first waits for the previous owner's last step, then uploads on that same stream, so neither
-// handle's kernels can see the other's constants.
-constexpr int MAX_DEVICES = 64;
-kidmp_handle* g_const_owner[MAX_DEVICES] = {};
-int ensure_constants(kidmp_handle* h, cudaStream_t s) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  kidmp_handle*& owner = g_const_owner[h->device];
-  if (owner != h) {
-    if (owner && owner->ev_done) CK(h, cudaStreamWaitEvent(s, owner->ev_done, 0));
-    CK(h, cudaMemcpyToSymbolAsync(ck, &h->kc, sizeof(KConst), 0, cudaMemcpyHostToDevice, s));
-    k_n0_lo<<<1, 1, 0, s>>>();                       // the per-run graupel intercept constant (kidmp_column.cuh)
-    owner = h;
-  }
-  return 0;
-}
-
 void free_work(WorkSet& w) {
   void* old[] = {w.d_scratch, w.d_cls, w.d_colflag, w.d_work, w.d_cells, w.d_cellmeta, w.d_coldiag, w.d_colwork, w.d_cellidx, w.d_ws, w.d_n0a};
   for (void* q : old) if (q) cudaFree(q);
@@ -359,14 +341,14 @@ void launch_cells(kidmp_handle* h, const StepArgs& a, int nsm, cudaStream_t s, c
   // (the aerosol-aware instantiations carry more live values: one block per SM less keeps them out of local memory)
   constexpr int WB = AERO ? KC_AERO_WARM_B : KC_WARM_B, IB = AERO ? KC_AERO_ICE_B : KC_ICE_B, MB = AERO ? KC_AERO_MIX_B : KC_MIXNR_B,
                 FB = AERO ? KC_AERO_MIX_B : KC_FULL_B;
-  k_cells<KC_WARM, KC_WARM_T, WB, KC_WARM_BARS, RATES, AERO><<<nsm * WB, KC_WARM_T, 0, s>>>(a);
+  k_cells<KC_WARM, KC_WARM_T, WB, KC_WARM_BARS, RATES, AERO><<<nsm * WB, KC_WARM_T, 0, s>>>(a, h->kc);
   mark(KT_WARM);
-  k_cells<KC_ICE, KC_ICE_T, IB, KC_ICE_BARS, RATES, AERO><<<nsm * IB, KC_ICE_T, 0, s>>>(a);
+  k_cells<KC_ICE, KC_ICE_T, IB, KC_ICE_BARS, RATES, AERO><<<nsm * IB, KC_ICE_T, 0, s>>>(a, h->kc);
   mark(KT_ICE);
   if (n0_done) cudaStreamWaitEvent(s, n0_done, 0);     // only the classes with graupel read the intercept minima of k_n0_sweep
-  k_cells<KC_MIXNR, KC_MIXNR_T, MB, KC_MIXNR_BARS, RATES, AERO><<<nsm * MB, KC_MIXNR_T, 0, s>>>(a);
+  k_cells<KC_MIXNR, KC_MIXNR_T, MB, KC_MIXNR_BARS, RATES, AERO><<<nsm * MB, KC_MIXNR_T, 0, s>>>(a, h->kc);
   mark(KT_MIXNR);
-  k_cells<KC_FULL, KC_FULL_T, FB, KC_FULL_BARS, RATES, AERO><<<nsm * FB, KC_FULL_T, 0, s>>>(a);
+  k_cells<KC_FULL, KC_FULL_T, FB, KC_FULL_BARS, RATES, AERO><<<nsm * FB, KC_FULL_T, 0, s>>>(a, h->kc);
   mark(KT_FULL);
 }
 
@@ -385,7 +367,6 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
   if (ensure_work(h, cap, a0.nz)) return 1;
   // the work set is the handle's: a step on another stream than the last one starts after it
   CK(h, cudaStreamWaitEvent(s, h->ev_done, 0));
-  if (ensure_constants(h, s)) return 1;
   if (h->partial_chunks < nchunks) {
     if (h->d_partial) { CK(h, cudaEventSynchronize(h->ev_done)); cudaFree(h->d_partial); h->d_partial = nullptr; h->partial_chunks = 0; }
     CK(h, cudaMalloc((void**)&h->d_partial, (size_t)nchunks * DIAG_BLOCKS * KIDMP_NDIAG * 8));
@@ -393,7 +374,9 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
   }
   // Replay the captured graph of this very step (all its chunks), or capture it now.
   const bool graphable = h->graphs && !h->timing && nchunks <= 64 && a0.ncol <= h->graph_max_cols;
-  // (a handle setting that a captured launch reads belongs in the key: a replay after the setting changed would run the old one)
+  // (a handle setting that a captured launch reads belongs in the key: a replay after the setting changed would run the old one.
+  // The constants h->kc, which every graph carries as launch parameters, need no place in it: they are fixed by kidmp_init
+  // except tnc_wev, which only the aerosol-aware kernels read and which is set before the first of them is launched or captured.)
   const long gkey[7] = {(long)(size_t)h->ws.d_scratch, h->ws.cols, (long)h->ws.nz, (long)h->simple, (long)(size_t)h->d_partial,
                         chunk, (long)h->classes};
   kidmp_handle::StepGraph* hit = nullptr;
@@ -458,18 +441,18 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
     // The classification left the key histogram of the busy cells: first entry of every key and class, the work list of
     // the cloudy columns, then the list of the busy cells.  Second stream: the graupel intercept sweep (needs the work list
     // only; the cell kernels with graupel wait for it).
-    k_cell_offsets<<<1, 64, 0, s>>>(a);
+    k_cell_offsets<<<1, 64, 0, s>>>(a, h->kc);
     k_list_scan<<<1, 1024, 0, s>>>(a.work_mask, (int)ngroups, a.work_offset, a.work_count);
     k_list_fill<<<(unsigned)((ngroups * 32 + 255) / 256), 256, 0, s>>>(a.work_mask, a.work_offset, (int)ngroups, a.work_list);
     if (serial) {
       k_cell_fill<<<(unsigned)lblocks, LIST_TILE, 0, s>>>(a);
       mark(KT_LISTS);
-      if (!h->kc.iiwarm) k_n0_sweep<<<(unsigned)((a.ncol + 127) / 128), 128, 0, s>>>(a);
+      if (!h->kc.iiwarm) k_n0_sweep<<<(unsigned)((a.ncol + 127) / 128), 128, 0, s>>>(a, h->kc);
       mark(KT_N0);
     } else {
       fork(w.ev_lists_done, s, x);                   // (recorded after k_list_fill)
       // the number of cloudy columns is only known on the device: grids for the worst case, surplus blocks leave at once
-      if (!h->kc.iiwarm) k_n0_sweep<<<(unsigned)((a.ncol + 127) / 128), 128, 0, x>>>(a);
+      if (!h->kc.iiwarm) k_n0_sweep<<<(unsigned)((a.ncol + 127) / 128), 128, 0, x>>>(a, h->kc);
       k_cell_fill<<<(unsigned)lblocks, LIST_TILE, 0, s>>>(a);
       CK(h, cudaEventRecord(w.ev_n0_done, x));       // the sweep runs beside k_cell_fill and the warm and ice cell kernels
       mark(KT_LISTS); mark(KT_N0);
@@ -479,16 +462,17 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
     if (aero) launch_cells<false, true>(h, a, h->nsm, s, n0_done);
     else if (a.rates) launch_cells<true, false>(h, a, h->nsm, s, n0_done);
     else launch_cells<false, false>(h, a, h->nsm, s, n0_done);
-    k_carries<<<(unsigned)((a.ncol + 63) / 64), 64, 0, s>>>(a);
+    k_carries<<<(unsigned)((a.ncol + 63) / 64), 64, 0, s>>>(a, h->kc);
     mark(KT_CARRIES);
     // the columns with sedimentation sub-steps on the second stream, the others on this one: disjoint columns
     fork(w.ev_fork, s, x);
     const unsigned sgrid = (unsigned)(ngroups < h->nsm * 16 ? ngroups : h->nsm * 16);
-    if (aero) k_substeps<false, true><<<sgrid, 32, 0, x>>>(a);
-    else if (a.rates) k_substeps<true, false><<<sgrid, 32, 0, x>>>(a); else k_substeps<false, false><<<sgrid, 32, 0, x>>>(a);
+    if (aero) k_substeps<false, true><<<sgrid, 32, 0, x>>>(a, h->kc);
+    else if (a.rates) k_substeps<true, false><<<sgrid, 32, 0, x>>>(a, h->kc); else k_substeps<false, false><<<sgrid, 32, 0, x>>>(a, h->kc);
     mark(KT_SUBSTEPS);
-    if (aero) k_finish<false, true><<<(unsigned)ngroups, 32, 0, s>>>(a);
-    else if (a.rates) k_finish<true, false><<<(unsigned)ngroups, 32, 0, s>>>(a); else k_finish<false, false><<<(unsigned)ngroups, 32, 0, s>>>(a);
+    if (aero) k_finish<false, true><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
+    else if (a.rates) k_finish<true, false><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
+    else k_finish<false, false><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
     mark(KT_FINISH);
     fork(w.ev_join, x, s);
     k_diag_columns<<<DIAG_BLOCKS, 256, 0, s>>>(a, (a.ncol + DIAG_BLOCKS - 1) / DIAG_BLOCKS);
@@ -810,7 +794,6 @@ int kidmp_init(const kidmp_config* cfg, kidmp_handle** out) {
   h->cfg = *cfg;
   h->device = dev1;
   if (getenv("KIDMP_CHUNK") && atol(getenv("KIDMP_CHUNK")) >= 32) h->chunk_cols = atol(getenv("KIDMP_CHUNK"));
-  if (dev1 >= MAX_DEVICES) { delete h; return fail(nullptr, "kidmp_init: device ordinal %d not supported", dev1); }
   if (getenv("KIDMP_SIMPLE")) h->simple = atoi(getenv("KIDMP_SIMPLE")) != 0;
   if (getenv("KIDMP_GRAPHS")) h->graphs = atoi(getenv("KIDMP_GRAPHS")) != 0;
   if (getenv("KIDMP_GRAPH_MAX") && atol(getenv("KIDMP_GRAPH_MAX")) > 0) h->graph_max_cols = atol(getenv("KIDMP_GRAPH_MAX"));
@@ -868,6 +851,16 @@ int kidmp_init(const kidmp_config* cfg, kidmp_handle** out) {
       h->err = "math table upload failed"; return bail(1);
     }
   }
+  {
+    // KConst::n0_lo, the graupel intercept constant: it goes through the device's dlog / dexp, so the device evaluates it
+    double* d = nullptr;
+    cudaError_t e = cudaMalloc((void**)&d, sizeof(double));
+    if (e == cudaSuccess) { k_n0_lo<<<1, 1, 0, h->stream>>>(d); e = cudaGetLastError(); }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&h->kc.n0_lo, d, sizeof(double), cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    if (d) cudaFree(d);
+    if (e != cudaSuccess) { fail(h, "n0_lo: %s", cudaGetErrorString(e)); return bail(1); }
+  }
   bool loaded = false;
   if (cfg->reuse_tables && !h->cache_path.empty()) loaded = load_cache(h) == 0;   // l_reuse_thompson_lookup, M:3720
   h->tables_from_cache = loaded;
@@ -885,10 +878,6 @@ int kidmp_finalize(kidmp_handle* h) {
   if (!h) return 0;
   if (h->multi) { multi_finalize(h); return 0; }
   DevGuard guard_(h->device);
-  {
-    std::lock_guard<std::mutex> lk(g_mu);
-    if (g_const_owner[h->device] == h) g_const_owner[h->device] = nullptr;
-  }
   // what this handle enqueued: steps end at ev_done (on whatever stream they ran), copies and staging on its own streams
   if (h->ev_done) cudaEventSynchronize(h->ev_done);
   for (cudaStream_t s : {h->stream, h->copy_in, h->copy_out}) if (s) cudaStreamSynchronize(s);
@@ -1349,7 +1338,7 @@ int kidmp_step_device(kidmp_handle* h, long ncol, int nz, float dt, float* const
 // table_dropEvap, M:4400-4439: number of the cloud droplets smaller than D-star for every (D-star bin, cloud water node,
 // droplet number node).  Only an aerosol-aware run reads it (M:2850): built by the first such step - slope and intercept of the
 // 3 700 spectra on the host (two powers each, like the per-node scalars of the other tables), the 370 000 bin sums by
-// k_table_wev - and the constants re-published.
+// k_table_wev - and its pointer set in the handle's constants.
 int ensure_wev_table(kidmp_handle* h) {
   if (h->d_tnc_wev) return 0;
   const HostBins& b = h->hb;
@@ -1383,8 +1372,6 @@ int ensure_wev_table(kidmp_handle* h) {
   for (void* q : keep) cudaFree(q);
   if (e != cudaSuccess) { if (h->d_tnc_wev) { cudaFree(h->d_tnc_wev); h->d_tnc_wev = nullptr; } return fail(h, "table_dropEvap: %s", cudaGetErrorString(e)); }
   h->kc.tnc_wev = h->d_tnc_wev;
-  std::lock_guard<std::mutex> lk(g_mu);
-  if (g_const_owner[h->device] == h) g_const_owner[h->device] = nullptr;      // the next step uploads the constants again
   return 0;
 }
 
@@ -1513,7 +1500,7 @@ static int wrf_kernels(kidmp_handle* h, WrfArgs& a, float* const* ae4, const flo
   if (launch_step(h, sa, s)) return 1;
   if (ae4 && nwfa2d) { k_nwfa_surface<<<(unsigned)((ncol + 255) / 256), 256, 0, s>>>(sa.nwfa, d_ae + 4 * n, ncol, dt_in); ++h->launches; }   // M:1001
   if (s == h->stream) CK(h, cudaEventRecord(h->ev1, s));
-  k_wrf_scatter<<<g, b, 0, s>>>(a, h->kc.Nt_c);
+  k_wrf_scatter<<<g, b, 0, s>>>(a, h->kc);
   if (ae4) {
     for (int q = 0; q < 3; ++q) k_ikj_planes<<<g, b, 0, s>>>(ae4[q], d_ae + n * q, a.t, 0);
     h->launches += 3;

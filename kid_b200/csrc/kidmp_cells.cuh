@@ -86,7 +86,7 @@ __device__ __forceinline__ RecA load_rec_a(const StepArgs& a, unsigned idx, unsi
 }
 
 // M:1649-1653 for a given intercept (the running minimum already taken)
-__device__ __forceinline__ void graupel_slope(double N0_exp, float rg, double& ilamg, double& N0_g) {
+__device__ __forceinline__ void graupel_slope(const KConst& ck, double N0_exp, float rg, double& ilamg, double& N0_g) {
   const double lam_exp = sqrt(sqrt(N0_exp * (double)ck.am_g * (double)ck.cgg[0] / (double)rg));   // **oge1, oge1 = 1/4
   const double lamg = lam_exp * (double)ck.lamg_fac;
   ilamg = (double)1.f / lamg;
@@ -125,7 +125,7 @@ template <int KC> struct CellTraits {
 // k_classify (kidmp_column.cuh) counts the keys per 32-column group and per launch while it writes the class bytes;
 // k_cell_offsets: first entry of every key and class; k_cell_fill: the entries, and the busy bits of every cloudy column
 // for the column kernels.
-__global__ void __launch_bounds__(64) k_cell_offsets(StepArgs a) {
+__global__ void __launch_bounds__(64) k_cell_offsets(StepArgs a, const __grid_constant__ KConst ck) {
   __shared__ int s_n[64], s_kc[64];
   const int t = threadIdx.x;
   const bool iiwarm = ck.iiwarm != 0;
@@ -195,7 +195,7 @@ __global__ void __launch_bounds__(LIST_TILE) k_cell_fill(StepArgs a) {
 // ---- running minimum of the graupel intercept of S4 (M:1633-1648), only for columns that hold graupel: the slope and
 // intercept it feeds (M:1649-1653) are read by graupel processes alone.  One thread per cloudy column, top-down; the value
 // of every graupel cell goes to n0a[k][slot].  Needs the work list only: runs beside the cell-list kernels.  The rain of S1 is needed for the supercooled-drop test of M:1640.
-__global__ void __launch_bounds__(128) k_n0_sweep(StepArgs a) {
+__global__ void __launch_bounds__(128) k_n0_sweep(StepArgs a, const __grid_constant__ KConst ck) {
   const int slot = blockIdx.x * 128 + threadIdx.x;
   const int count = *a.work_count;
   if (slot >= count || ck.iiwarm) return;
@@ -204,7 +204,7 @@ __global__ void __launch_bounds__(128) k_n0_sweep(StepArgs a) {
   const int nz = a.nz;
   const long ld = a.ld;
   float* const n0a = a.n0a + slot;                         // [nz][count], read by the cell kernels for graupel cells
-  const double n0_empty = g_n0_lo;
+  const double n0_empty = ck.n0_lo;
   bool warm_a = false;                                    // a level at or above this one has T >= 270.65 K (k_0, M:1635)
   double n0_min = (double)KP_GONV_MAX;
   constexpr int B = 6;                                    // levels loaded per batch: the walk is a chain of dependent steps,
@@ -234,8 +234,8 @@ __global__ void __launch_bounds__(128) k_n0_sweep(StepArgs a) {
         if (cold_rain) {                                  // the rain of S1 (M:1445-1466) for the xslw1 of M:1640
           const float rr = qr1d * rho;
           float nr = fmaxf(R2, a.f[F_NR][g] * rho);
-          if (nr <= R2) { mvd_r = 1.0E-3f; nr = nr_from_mvd(rr, mvd_r); }
-          const double lamr = rain_lam(nr, rr);
+          if (nr <= R2) { mvd_r = 1.0E-3f; nr = nr_from_mvd(ck, rr, mvd_r); }
+          const double lamr = rain_lam(ck, nr, rr);
           mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr);
           if (mvd_r > 2.5E-3f) mvd_r = 2.5E-3f;
           else if (mvd_r < D0r * 0.75f) mvd_r = D0r * 0.75f;
@@ -259,7 +259,7 @@ __global__ void __launch_bounds__(128) k_n0_sweep(StepArgs a) {
 // AERO: is_aerosol_aware = .true. (M:28): cloud droplet number, water-friendly and ice-friendly aerosol numbers are prognostic
 // (a.nc, a.nwfa, a.nifa), a.w feeds the droplet activation; every aerosol block is compiled out of the default kernels.
 template <int KC, int THREADS, int MINB, int BARS, bool RATES, bool AERO>
-__global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
+__global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a, const __grid_constant__ KConst ck) {
   using TR = CellTraits<KC>;
   constexpr bool LOCK = BARS != 0;
   const int n = a.cell_count[KC];
@@ -274,7 +274,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
   const float odt = 1.f / DT, odts = 1.f / DT;
   const float Nt_c = ck.Nt_c;
   const bool iiwarm = ck.iiwarm != 0;
-  const double n0_empty = g_n0_lo;
+  const double n0_empty = ck.n0_lo;
 #define LOCKBAR(i) do { if (LOCK && ((BARS >> (i)) & 1)) { __syncwarp(); asm volatile("bar.sync 1, %0;" ::"r"(lock_threads) : "memory"); } } while (0)
 #pragma unroll 1
   for (int base = blockIdx.x * THREADS; base < n; base += gridDim.x * THREADS) {
@@ -357,7 +357,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
         ni = (float)fmin(499.E3, (double)(ck.cig[0] * ck.oig2 * ri / ck.am_i) * cube_d(lami));
       }
       L_qi = true;
-      lami = ice_lam(ni, ri);
+      lami = ice_lam(ck, ni, ri);
       ilami = (double)1.f / lami;
       const float xDi = (float)((double)(3.f + 0.f + 1.f) * ilami);
       if (xDi < 5.E-6f) {
@@ -375,12 +375,12 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
     if (TR::R && qr1d > R1) {
       rr = qr1d * rho;
       nr = fmaxf(R2, nr1d * rho);
-      if (nr <= R2) { mvd_r = 1.0E-3f; nr = nr_from_mvd(rr, mvd_r); }
+      if (nr <= R2) { mvd_r = 1.0E-3f; nr = nr_from_mvd(ck, rr, mvd_r); }
       L_qr = true;
-      lamr = rain_lam(nr, rr);
+      lamr = rain_lam(ck, nr, rr);
       mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr);
-      if (mvd_r > 2.5E-3f) { mvd_r = 2.5E-3f; nr = nr_from_mvd(rr, mvd_r); lamr_stale = true; }
-      else if (mvd_r < D0r * 0.75f) { mvd_r = D0r * 0.75f; nr = nr_from_mvd(rr, mvd_r); lamr_stale = true; }
+      if (mvd_r > 2.5E-3f) { mvd_r = 2.5E-3f; nr = nr_from_mvd(ck, rr, mvd_r); lamr_stale = true; }
+      else if (mvd_r < D0r * 0.75f) { mvd_r = D0r * 0.75f; nr = nr_from_mvd(ck, rr, mvd_r); lamr_stale = true; }
     } else {
       qr1d = 0.0f; nr1d = 0.0f; rr = R1; nr = R2; L_qr = false;
     }
@@ -428,12 +428,12 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
         smof = field_moment(tc0, ck.cse[15], smo2);
       }
       // ---- S4, M:1633-1654 graupel intercept: the running minimum of M:1648 comes from k_n0_sweep -----------
-      if (TR::G && L_qg) graupel_slope((double)a.n0a[(size_t)k * count + slot], rg, ilamg, N0_g);
+      if (TR::G && L_qg) graupel_slope(ck, (double)a.n0a[(size_t)k * count + slot], rg, ilamg, N0_g);
     }
     // M:1661-1666 rain slope and intercept.  Without rain (rr = R1, nr = R2) every reader of lamr, ilamr, N0_r
     // and mvd_r is switched off (L_qr at M:1676, M:1724, M:2880; rr >= r_r(1) at M:1818, M:1964, M:2028, M:2188)
     if (TR::R && L_qr) {
-      if (lamr_stale) { lamr = rain_lam(nr, rr); mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr); }
+      if (lamr_stale) { lamr = rain_lam(ck, nr, rr); mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr); }
       ilamr = (double)1.f / lamr;
       N0_r = (double)(nr * ck.org2) * lamr;                                // lamr**cre(2), cre(2) = 1
     }
@@ -503,24 +503,24 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
       int idx_t = (int)((tempc - 2.5f) / 5.f) - 1;
       idx_t = max(1, -idx_t);
       idx_t = min(idx_t, (int)NTB_T);
-      const int idx_c = (TR::C && rc > ck.r_c1) ? decade_idx_f(rc, ck.nic2, NTB_C) : 1;
-      const int idx_i = (ri > ck.r_i1) ? decade_idx_f(ri, ck.nii2, NTB_I) : 1;
-      const int idx_i1 = (ni > ck.Nt_i1) ? decade_idx_f(ni, ck.nii3, NTB_I1) : 1;
+      const int idx_c = (TR::C && rc > ck.r_c1) ? decade_idx_f(ck, rc, ck.nic2, NTB_C) : 1;
+      const int idx_i = (ri > ck.r_i1) ? decade_idx_f(ck, ri, ck.nii2, NTB_I) : 1;
+      const int idx_i1 = (ni > ck.Nt_i1) ? decade_idx_f(ck, ni, ck.nii3, NTB_I1) : 1;
       int idx_r = 1, idx_r1 = NTB_R1, idx_s = 1, idx_g = 1, idx_g1 = NTB_G1;
       if (TR::R && rr > ck.r_r1) {
-        idx_r = decade_idx_f(rr, ck.nir2, NTB_R);
+        idx_r = decade_idx_f(ck, rr, ck.nir2, NTB_R);
         lamr = (double)1.f / ilamr;
         const double lam_exp = lamr * (double)ck.n0r_fac;
         const double N0_exp = (double)(ck.org1 * rr / ck.am_r) * sq_d(sq_d(lam_exp));   // **cre(1), cre(1) = 4
-        idx_r1 = decade_idx_d(N0_exp, ck.nir3, NTB_R1);
+        idx_r1 = decade_idx_d(ck, N0_exp, ck.nir3, NTB_R1);
       }
-      if (TR::R) idx_s = (rs > ck.r_s1) ? decade_idx_f(rs, ck.nis2, NTB_S) : 1;          // only the rain-snow tables read it
+      if (TR::R) idx_s = (rs > ck.r_s1) ? decade_idx_f(ck, rs, ck.nis2, NTB_S) : 1;      // only the rain-snow tables read it
       if (TR::R && TR::G && rg > ck.r_g1) {                                              // only the rain-graupel tables read them
-        idx_g = decade_idx_f(rg, ck.nig2, NTB_G);
+        idx_g = decade_idx_f(ck, rg, ck.nig2, NTB_G);
         const double lamg = (double)1.f / ilamg;
         const double lam_exp = lamg * (double)ck.n0g_fac;
         const double N0_exp = (double)(ck.ogg1 * rg / ck.am_g) * sq_d(sq_d(lam_exp));   // **cge(1), cge(1) = 4
-        idx_g1 = decade_idx_d(N0_exp, ck.nig3, NTB_G1);
+        idx_g1 = decade_idx_d(ck, N0_exp, ck.nig3, NTB_G1);
       }
 
       // M:1884-1900 sublimation/deposition prefactor
@@ -701,7 +701,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
         // M:2116-2149 deposition / sublimation of cloud ice, ice -> snow
         float oxmi = 0.f, xDi = 0.f;
         if (L_qi) {
-          if (lami_stale) lami = ice_lam(ni, ri);
+          if (lami_stale) lami = ice_lam(ck, ni, ri);
           ilami = (double)1.f / lami;
           xDi = (float)fmax((double)ck.D0i, (double)(3.f + 0.f + 1.f) * ilami);
           const float xmi = ck.am_i * cube_f(xDi);
@@ -947,7 +947,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
       const float xri = fmaxf(R1, (qi1d + qit * DT) * rho);
       float xni = fmaxf(R2, (ni1d + nit * DT) * rho);
       if (TR::I9 && xri > R1) {
-        lami = ice_lam(xni, xri);
+        lami = ice_lam(ck, xni, xri);
         ilami = (double)1.f / lami;
         const float xD = (float)((double)(3.f + 0.f + 1.f) * ilami);
         if (xD < 5.E-6f) {
@@ -970,15 +970,15 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
       const float xrr = fmaxf(R1, (qr1d + qrt * DT) * rho);
       float xnr = fmaxf(R2, (nr1d + nrt * DT) * rho);
       if (TR::R9 && xrr > R1) {
-        lamr = rain_lam(xnr, xrr);
+        lamr = rain_lam(ck, xnr, xrr);
         mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr);
         if (mvd_r > 2.5E-3f) {
           mvd_r = 2.5E-3f;
-          xnr = nr_from_mvd(xrr, mvd_r);
+          xnr = nr_from_mvd(ck, xrr, mvd_r);
           nrt = (xnr - nr1d * rho) * odts * orho;
         } else if (mvd_r < D0r * 0.75f) {
           mvd_r = D0r * 0.75f;
-          xnr = nr_from_mvd(xrr, mvd_r);
+          xnr = nr_from_mvd(ck, xrr, mvd_r);
           nrt = (xnr - nr1d * rho) * odts * orho;
         }
       } else {
@@ -1040,11 +1040,11 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
         rr = (qr1d + qrt * DT) * rho;
         nr = fmaxf(R2, (nr1d + nrt * DT) * rho);
         L_qr = true;
-        lamr = rain_lam(nr, rr);
+        lamr = rain_lam(ck, nr, rr);
         lamr_stale = false;
         mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr);
-        if (mvd_r > 2.5E-3f) { mvd_r = 2.5E-3f; nr = nr_from_mvd(rr, mvd_r); lamr_stale = true; }
-        else if (mvd_r < D0r * 0.75f) { mvd_r = D0r * 0.75f; nr = nr_from_mvd(rr, mvd_r); lamr_stale = true; }
+        if (mvd_r > 2.5E-3f) { mvd_r = 2.5E-3f; nr = nr_from_mvd(ck, rr, mvd_r); lamr_stale = true; }
+        else if (mvd_r < D0r * 0.75f) { mvd_r = D0r * 0.75f; nr = nr_from_mvd(ck, rr, mvd_r); lamr_stale = true; }
       } else { rr = R1; nr = R2; L_qr = false; }
       if (TR::S9 && (qs1d + qst * DT) > R1) { rs = (qs1d + qst * DT) * rho; L_qs = true; } else { rs = R1; L_qs = false; }
       if (TR::G9 && (qg1d + qgt * DT) > R1) { rg = (qg1d + qgt * DT) * rho; L_qg = true; } else { rg = R1; L_qg = false; }
@@ -1069,7 +1069,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
       n0b_slw = (TR::R9 && !warm9 && L_qr && mvd_r > 100.E-6f) ? graupel_n0_exp(4.01f + log10_f(mvd_r), rg) : n0b_lo;
     }
     if (TR::R9 && L_qr) {                                                   // M:2750-2755, as at M:1661
-      if (lamr_stale) { lamr = rain_lam(nr, rr); mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr); lamr_stale = false; }
+      if (lamr_stale) { lamr = rain_lam(ck, nr, rr); mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr); lamr_stale = false; }
       ilamr = (double)1.f / lamr;
       N0_r = (double)(nr * ck.org2) * lamr;
     }
@@ -1113,7 +1113,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
           const int idx_d = max(1, min((int)(1.E6 * Dc_star), (int)NBINS));
           int idx_n = nint_d(1.0 + (double)(float)NBINS * dlog((double)nc / ck.t_Nc1) / (double)ck.nic1);
           idx_n = max(1, min(idx_n, (int)NBINS));
-          const int idx_c = (rc > ck.r_c1) ? decade_idx_f(rc, ck.nic2, NTB_C) : 1;
+          const int idx_c = (rc > ck.r_c1) ? decade_idx_f(ck, rc, ck.nic2, NTB_C) : 1;
           prw_vcd = fmax((double)(-rc * 0.99f * orho * odt), prw_vcd);
           const double tnc = ck.tnc_wev[(size_t)(idx_d - 1) + (size_t)NBINS * ((idx_c - 1) + (size_t)NTB_C * (idx_n - 1))];
           pnc_wcd = fmax((double)(-nc * 0.99f * orho * odt), (double)(-tnc * (double)orho * (double)odt));
@@ -1200,7 +1200,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
     rhof = sqrtf(ck.rho_not / rho);
     float v_r = 0.f, v_nr = 0.f, v_i = 0.f, v_ni = 0.f, vts_h = 0.f;
     if (TR::R9 && rr > R1) {
-      if (!L_qr || lamr_stale) lamr = rain_lam(nr, rr);                   // M:3227: same nr, rr as at M:2750 otherwise
+      if (!L_qr || lamr_stale) lamr = rain_lam(ck, nr, rr);               // M:3227: same nr, rr as at M:2750 otherwise
       const double lf = lamr + (double)KP_FV_R;
       const double l2 = lamr * lamr, lf2 = lf * lf;
       // lamr**cre(3) * (lamr+fv_r)**(-cre(6)), cre(3) = 4, cre(6) = 5
@@ -1210,7 +1210,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a) {
     }
     if (TR::ICEPROC && !iiwarm) {
       if (TR::I9 && ri > R1) {
-        lami = ice_lam(ni, ri);
+        lami = ice_lam(ck, ni, ri);
         ilami = (double)1.f / lami;
         v_i = (float)((double)(rhof * KP_AV_I * ck.cig[2] * ck.oig2) * ilami);               // ilami**bv_i, bv_i = 1
         v_ni = (float)((double)(rhof * KP_AV_I * ck.cig[5] / ck.cig[6]) * ilami);
@@ -1312,7 +1312,7 @@ __device__ __forceinline__ void sed_substeps(float* __restrict__ r, float* __res
 // that rule, M:3301, M:3328), the sub-step counts and top sedimenting levels (M:3242, M:3208).  One thread per cloudy
 // column; all the values of a busy cell are loaded in one batch (one memory round trip per level).  Leaves colint
 // [8][count] and the list of the columns that need sedimentation sub-steps.
-__global__ void __launch_bounds__(64, 16) k_carries(StepArgs a) {
+__global__ void __launch_bounds__(64, 16) k_carries(StepArgs a, const __grid_constant__ KConst ck) {
   const int slot = blockIdx.x * 64 + threadIdx.x;
   const int count = *a.work_count;
   if (slot >= count) return;
@@ -1322,7 +1322,7 @@ __global__ void __launch_bounds__(64, 16) k_carries(StepArgs a) {
   const long cs = count;
   const float DT = a.dt;
   const bool iiwarm = ck.iiwarm != 0;
-  const double n0_empty = g_n0_lo;
+  const double n0_empty = ck.n0_lo;
   const unsigned* const cidx = a.cellidx + slot;
   const float* const dzp = a.dz_col ? a.dz_col + col : a.dz;     // one vector shared by all columns (KiD) or this column's own (WRF entry)
   const long dzs = a.dz_col ? ld : 1;
@@ -1377,7 +1377,7 @@ __global__ void __launch_bounds__(64, 16) k_carries(StepArgs a) {
         if (rg > R1) {
           const float rhof = sqrtf(ck.rho_not / rho);
           double ilamg = 0., N0_g = 0.;
-          graupel_slope(n0_min, rg, ilamg, N0_g);
+          graupel_slope(ck, n0_min, rg, ilamg, N0_g);
           const float vtg = (float)((double)(rhof * KP_AV_G * ck.cgg[5] * ck.ogg3) * pow_d(ilamg, (double)KP_BV_G));
           v_g = (s15 > 0.f) ? fmaxf(vtg, v_r) : vtg;         // temp > T_0 is what makes the S15 factor positive
           sc[SC_VTG] = v_g;
@@ -1426,7 +1426,7 @@ __device__ __forceinline__ SedCounts sed_counts(const int* ci, long cs, int nz) 
 }
 
 // the record of an idle cell: all rates zero, state unchanged, contents R1 / R2 (speeds: those of the level above)
-__device__ __forceinline__ void idle_record(float temp, float pres, float qv1d, float& rho, float& s15) {
+__device__ __forceinline__ void idle_record(const KConst& ck, float temp, float pres, float qv1d, float& rho, float& s15) {
   const float qv = fmaxf(1.E-10f, qv1d);
   const float tempc = temp - 273.15f;
   const float ocp = 1.f / (KP_CP * (1.f + 0.887f * qv));
@@ -1446,7 +1446,7 @@ __device__ __forceinline__ void idle_record(float temp, float pres, float qv1d, 
 enum { WS_TTEN = 0, WS_QVTEN, WS_QCTEN, WS_QITEN, WS_QRTEN, WS_QSTEN, WS_QGTEN, WS_NITEN, WS_NRTEN, WS_NCTEN,
        WS_RR, WS_NR, WS_RI, WS_NI, WS_RS, WS_RG, WS_VTR, WS_VTNR, WS_VTI, WS_VTNI, WS_VTS, WS_VTG, WS_RHO, WS_S15, WS_NWFAT, WS_NIFAT, WS_N };
 template <bool RATES, bool AERO>
-__global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a) {
+__global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a, const __grid_constant__ KConst ck) {
   const int n = *a.sub_count, count = *a.work_count;
   const unsigned k1_list = (unsigned)a.cell_kstart[KC_ICE], k2_list = (unsigned)a.cell_kstart[KC_MIXNR];
   const int nz = a.nz;
@@ -1492,7 +1492,7 @@ __global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a) {
         } else {
           const long o = (long)k * ld + col;
           float rho, s15;
-          idle_record(a.f[F_T][o], a.p[o], a.f[F_QV][o], rho, s15);
+          idle_record(ck, a.f[F_T][o], a.p[o], a.f[F_QV][o], rho, s15);
 #pragma unroll
           for (int q = WS_TTEN; q <= WS_NCTEN; ++q) w[q * ps] = 0.0f;
           w[WS_RR * ps] = R1; w[WS_NR * ps] = R2; w[WS_RI * ps] = R1; w[WS_NI * ps] = R2; w[WS_RS * ps] = R1; w[WS_RG * ps] = R1;
@@ -1541,7 +1541,7 @@ __global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a) {
         const long st = (long)nz * ld;
         for (int r = 0; r < KIDMP_NRATES; ++r) rp[r * st] = 0.0f;
       }
-      finish_level<AERO>(a, sp, c, h, k, nz, o, dzp[k * dzs], a.f[F_T][o], a.f[F_QV][o], a.f[F_QC][o], a.f[F_QI][o], a.f[F_QR][o],
+      finish_level<AERO>(ck, a, sp, c, h, k, nz, o, dzp[k * dzs], a.f[F_T][o], a.f[F_QV][o], a.f[F_QC][o], a.f[F_QI][o], a.f[F_QR][o],
                    a.f[F_QS][o], a.f[F_QG][o], a.f[F_NI][o], a.f[F_NR][o], a.p[o]);
     }
     // ppt is overwritten with this step's amounts: rain, ice, snow, graupel (I:55-58, I:162-177)
@@ -1557,7 +1557,7 @@ __global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a) {
 #define K2_MINB 20
 #endif
 template <bool RATES, bool AERO>
-__global__ void __launch_bounds__(32, K2_MINB) k_finish(StepArgs a) {
+__global__ void __launch_bounds__(32, K2_MINB) k_finish(StepArgs a, const __grid_constant__ KConst ck) {
   const int slot = blockIdx.x * 32 + threadIdx.x;
   const int count = *a.work_count;
   if (slot >= count) return;
@@ -1632,7 +1632,7 @@ __global__ void __launch_bounds__(32, K2_MINB) k_finish(StepArgs a) {
       h.tt = 0.f; h.qvt = 0.f; h.qct = 0.f; h.qit = 0.f; h.qrt = 0.f; h.qst = 0.f; h.qgt = 0.f; h.nit = 0.f; h.nrt = 0.f; h.nct = 0.f;
       h.rr = R1; h.nr = R2; h.ri = R1; h.ni = R2; h.rs = R1; h.rg = R1;
       h.nwfat = 0.f; h.nifat = 0.f;
-      idle_record(t1d, pres, qv1d, h.rho, h.s15);
+      idle_record(ck, t1d, pres, qv1d, h.rho, h.s15);
       if (RATES) {                                        // an idle cell: every process rate is zero
         float* rp = a.rates + o;
         const long st = (long)nz * ld;
@@ -1647,7 +1647,7 @@ __global__ void __launch_bounds__(32, K2_MINB) k_finish(StepArgs a) {
         if (v_s > 1.E-3f) sp.top_s = nz;
       }
     }
-    finish_level<AERO>(a, sp, c, h, k, nz, o, dzp[k * dzs], t1d, qv1d, qc1d, qi1d, qr1d, qs1d, qg1d, ni1d, nr1d, pres);
+    finish_level<AERO>(ck, a, sp, c, h, k, nz, o, dzp[k * dzs], t1d, qv1d, qc1d, qi1d, qr1d, qs1d, qg1d, ni1d, nr1d, pres);
   }
   // ppt is overwritten with this step's amounts: rain, ice, snow, graupel (I:55-58, I:162-177)
   a.ppt[col] = c.ppt_r; a.ppt[ld + col] = c.ppt_i; a.ppt[2 * ld + col] = c.ppt_s; a.ppt[3 * ld + col] = c.ppt_g;

@@ -19,8 +19,6 @@
 
 namespace kidmp {
 
-__constant__ KConst ck;
-
 // The f64 logarithm / exponential / power stay out of line (kidmp_math.cuh): ~130 call sites, and in line they made a
 // kernel whose instruction fetch was the limit (profiles/r01; still 6 % slower in line under the lockstep barriers).
 // The small helpers below are in line again since the lockstep blocks share their instruction-cache lines: measured
@@ -69,7 +67,7 @@ __device__ __forceinline__ int decade_guess(float x) {
 // When x / 10.**n0 is well inside [1, 10) no other candidate can match (x / 10.**(n0-1) is ten times larger, x / 10.**(n0+1)
 // ten times smaller, and a division is off by half an ulp at most), so the search of the reference is only walked,
 // in its own order, when the quotient is within 1e-5 of a decade boundary or the guess is a decade off.
-KIDMP_HELPER int decade_idx_f(float x, int n2, int ntb) {
+KIDMP_HELPER int decade_idx_f(const KConst& ck, float x, int n2, int ntb) {
   const int n0 = decade_guess(x);
   const float q0 = x / ck.p10[n0 + 32];
   int n = n0;
@@ -86,7 +84,7 @@ KIDMP_HELPER int decade_idx_f(float x, int n2, int ntb) {
   const int idx = (int)qn + 9 * (n - n2);
   return max(1, min(idx, ntb));
 }
-KIDMP_HELPER int decade_idx_d(double x, int n2, int ntb) {
+KIDMP_HELPER int decade_idx_d(const KConst& ck, double x, int n2, int ntb) {
   const int n0 = decade_guess((float)x);
   const double q0 = x / (double)ck.p10[n0 + 32];
   int n = n0;
@@ -105,15 +103,15 @@ KIDMP_HELPER int decade_idx_d(double x, int n2, int ntb) {
 }
 
 // rain number from mass at a clamped median volume diameter, M:1452-1454
-KIDMP_HELPER float nr_from_mvd(float rr, float mvd_r) {
+KIDMP_HELPER float nr_from_mvd(const KConst& ck, float rr, float mvd_r) {
   const double lamr = (double)((3.0f + 0.0f + 0.672f) / mvd_r);
   return (float)((double)(ck.crg[1] * ck.org3 * rr) * cube_d(lamr) / (double)ck.am_r);
 }
 // lamr = (am_r*crg(3)*org2*nr/rr)**obmr, M:1457
-KIDMP_HELPER double rain_lam(float nr, float rr) {
+KIDMP_HELPER double rain_lam(const KConst& ck, float nr, float rr) {
   return (double)pow_f(ck.am_r * ck.crg[2] * ck.org2 * nr / rr, ck.obmr);
 }
-KIDMP_HELPER double ice_lam(float ni, float ri) {   // M:1429
+KIDMP_HELPER double ice_lam(const KConst& ck, float ni, float ri) {   // M:1429
   return (double)pow_f(ck.am_i * ck.cig[1] * ck.oig1 * ni / ri, ck.obmi);
 }
 
@@ -128,10 +126,9 @@ __device__ __forceinline__ double graupel_n0_exp(float xslw1, float rg) {
   return fmax((double)KP_GONV_MIN, fmin(N0_exp, (double)KP_GONV_MAX));
 }
 KIDMP_HELPER double graupel_n0_lo() { return graupel_n0_exp(0.01f, R1); }
-__device__ double g_n0_lo;                                 // graupel_n0_lo(), evaluated once at init by k_n0_lo
-__global__ void k_n0_lo() { g_n0_lo = graupel_n0_lo(); }
-KIDMP_HELPER void graupel_n0(bool above_k0, bool L_qr, bool L_qg, float mvd_r, float rg, double n0_lo, double& N0_min,
-                             double& ilamg, double& N0_g) {
+__global__ void k_n0_lo(double* n0_lo) { *n0_lo = graupel_n0_lo(); }      // KConst::n0_lo, evaluated once by kidmp_init
+KIDMP_HELPER void graupel_n0(const KConst& ck, bool above_k0, bool L_qr, bool L_qg, float mvd_r, float rg, double n0_lo,
+                             double& N0_min, double& ilamg, double& N0_g) {
   const bool slw = above_k0 && L_qr && mvd_r > 100.E-6f;
   double N0_exp = n0_lo;
   if (slw || rg > 5.E-5f) {
@@ -331,8 +328,8 @@ struct HandOff {              // what S1..S13 leave for a level (SC_* order)
 };
 // AERO: is_aerosol_aware = .true.: the droplet number and the two aerosol numbers are state (a.nc, a.nwfa, a.nifa, M:3626-3647)
 template <bool AERO = false>
-__device__ __forceinline__ void finish_level(const StepArgs& a, const SedParams& p, SedCarry& c, const HandOff& h, int k, int nz,
-                                             long g, float dzk, float t1d, float qv1d, float qc1d, float qi1d, float qr1d,
+__device__ __forceinline__ void finish_level(const KConst& ck, const StepArgs& a, const SedParams& p, SedCarry& c, const HandOff& h,
+                                             int k, int nz, long g, float dzk, float t1d, float qv1d, float qc1d, float qi1d, float qr1d,
                                              float qs1d, float qg1d, float ni1d, float nr1d, float pres) {
   float tt = h.tt, qvt = h.qvt, qct = h.qct, qit = h.qit, qrt = h.qrt, qst = h.qst, qgt = h.qgt, nit = h.nit, nrt = h.nrt, nct = h.nct;
   const float rho = h.rho, s15 = h.s15, rr = h.rr, nr = h.nr, ri = h.ri, ni = h.ni, rs = h.rs, rg = h.rg;
@@ -423,7 +420,7 @@ __device__ __forceinline__ void finish_level(const StepArgs& a, const SedParams&
   if (qi1d <= KP_R1) {
     qi1d = 0.0f; ni1d = 0.0f;
   } else {
-    double lami = ice_lam(ni1d, qi1d);
+    double lami = ice_lam(ck, ni1d, qi1d);
     const double ilami = (double)1.f / lami;
     const float xDi = (float)((double)(3.f + 0.f + 1.f) * ilami);
     if (xDi < 5.E-6f) lami = (double)(ck.cie[1] / 5.E-6f);
@@ -435,11 +432,11 @@ __device__ __forceinline__ void finish_level(const StepArgs& a, const SedParams&
   if (qr1d <= KP_R1) {
     qr1d = 0.0f; nr1d = 0.0f;
   } else {
-    const double lamr = rain_lam(nr1d, qr1d);
+    const double lamr = rain_lam(ck, nr1d, qr1d);
     float mvd_r = (float)((double)(3.0f + 0.f + 0.672f) / lamr);
     if (mvd_r > 2.5E-3f) mvd_r = 2.5E-3f;
     else if (mvd_r < KP_D0R * 0.75f) mvd_r = KP_D0R * 0.75f;
-    nr1d = nr_from_mvd(qr1d, mvd_r);
+    nr1d = nr_from_mvd(ck, qr1d, mvd_r);
   }
   qs1d = qs1d + qst * p.DT;
   if (qs1d <= KP_R1) qs1d = 0.0f;

@@ -71,7 +71,8 @@ enum { F_TPI = 0, F_TPG, F_TNI, F_TNR, F_N };        // qrfz
 enum { C_TPI = 0, C_TNI, C_N };                      // qcfz
 enum { I_TPS = 0, I_TNI, I_TPI_IDE, I_N };           // iaus
 
-// constants written by the host part of init (M:381-670) and read by every kernel
+// constants written by the host part of init (M:381-670): one copy per handle, a __grid_constant__ parameter `ck` of
+// every kernel that reads them
 struct KConst {
   float Nt_c, Sc3, D0i, xm0s, xm0g, rho_not;
   float am_r, am_g, am_i, oRv, lfus, olfus;
@@ -92,6 +93,7 @@ struct KConst {
   float n0r_fac, n0g_fac, lamg_fac, dcg_fac[15];
   double Dr1, Ds1, lnDr, lnDs;                      // Dr(1), Ds(1), DLOG(Dr(nbr)/Dr(1)), DLOG(Ds(nbs)/Ds(1))
   double t_Nc1;                                     // t_Nc(1), M:668
+  double n0_lo;                                     // graupel_n0_lo() as the device computes it (k_n0_lo, run by kidmp_init)
   const double* tnc_wev;                            // [NBINS][NTB_C][NBINS] (idx_d fastest), table_dropEvap M:4400-4439; NULL until an aerosol-aware step asks for it
   // device tables
   const double* racg;   // [N_RACG][G_N]

@@ -65,7 +65,7 @@ __global__ void k_wrf_gather(WrfArgs a) {
 // M:4857-4868 cloud droplet shape parameter and g_ratio
 __device__ __constant__ float c_g_ratio[15] = {24, 60, 120, 210, 336, 504, 720, 990, 1320, 1716, 2184, 2730, 3360, 4080, 4896};
 
-__global__ void k_wrf_scatter(WrfArgs a, float Nt_c) {
+__global__ void k_wrf_scatter(WrfArgs a, const __grid_constant__ KConst ck) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x, k = blockIdx.y, j = blockIdx.z;
   if (i >= a.t.ni) return;
   const long dst = a.t.at(i, k, j), src = a.t.plane(i, k, j);
@@ -81,7 +81,7 @@ __global__ void k_wrf_scatter(WrfArgs a, float Nt_c) {
     float re_qc = 2.49E-6f, re_qi = 4.99E-6f, re_qs = 9.99E-6f;          // M:1112-1114
     const float rho = 0.622f * p1d / (KP_R * t1d * (qv1d + 0.622f));
     const float rc = fmaxf(KP_R1, qc1d * rho);
-    const float nc = a.nc_plane ? fmaxf(KP_R2, a.nc_plane[src] * rho) : Nt_c;       // M:4874-4875
+    const float nc = a.nc_plane ? fmaxf(KP_R2, a.nc_plane[src] * rho) : ck.Nt_c;    // M:4874-4875
     const float ri = fmaxf(KP_R1, qi1d * rho);
     const float ni = fmaxf(KP_R2, ni1d * rho);
     const float rs = fmaxf(KP_R1, qs1d * rho);
