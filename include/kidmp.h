@@ -101,6 +101,24 @@ int kidmp_step_device(kidmp_handle* h, long ncol, int nz, float dt,
                       float* const d_fields[KIDMP_NFIELDS], const float* d_p, const float* d_dz,
                       float* d_ppt, void* stream);
 
+/* Per-column cloud droplet number of the plain scheme (is_aerosol_aware = .false.).  The reference has one droplet number per
+ * run, Nt_c = set_Nc * 1e6 (M:381); these entries take one set_Nc [cm^-3] per column instead: column c is stepped with
+ * Nt_c = set_nc[c] * 1e6f (f32, as M:381), so it comes out bit for bit as a handle made with set_Nc = set_nc[c] would step it
+ * (set_Nc feeds nothing but Nt_c, and the lookup tables do not depend on it).  One handle, one table build and one launch
+ * sequence serve a domain of mixed droplet numbers (land and ocean) or a sweep of set_Nc values.  Every value must be finite
+ * and > 0, as kidmp_init requires of set_Nc.  set_nc == NULL: the handle's set_Nc, exactly as the entry without _nc.
+ *   kidmp_step_nc          kidmp_step with set_nc[ncol] on the host.  Every value is checked before anything is copied or
+ *                          launched; a bad one fails the call and leaves every array as it was.  All of kidmp_step's paths:
+ *                          both layouts, the chunk pipeline (each chunk takes its slice), multi-device handles (each device
+ *                          its column range), the handle's process-rate buffer.
+ *   kidmp_step_device_nc   kidmp_step_device with d_set_nc[ncol] on the device, enqueued on `stream`.  The values are not
+ *                          checked (as no other device input is); they are read when the step runs, also when the step is
+ *                          replayed from a captured CUDA graph. */
+int kidmp_step_nc(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
+                  const float* p, const float* dz, const float* set_nc, float* ppt);
+int kidmp_step_device_nc(kidmp_handle* h, long ncol, int nz, float dt, float* const d_fields[KIDMP_NFIELDS],
+                         const float* d_p, const float* d_dz, const float* d_set_nc, float* d_ppt, void* stream);
+
 /* Aerosol-aware step (is_aerosol_aware = .true., M:28, with dustyIce = homogIce = .true., M:30-31): the second half of
  * SURVEY.md section 8f-4.  Device pointers like kidmp_step_device; in addition the cloud droplet number nc and the numbers
  * of water-friendly and ice-friendly aerosols nwfa, nifa [kg^-1] are prognostic (INOUT, [nz][ncol]; mp_gt_driver's
@@ -198,6 +216,15 @@ int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const ki
                             float dt_in);
 int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t,
                                    const kidmp_wrf_aerosols* ae, float dt_in, void* stream);
+/* The plain-scheme tile entries with a droplet number per column (see kidmp_step_nc): set_nc2d is an (i,j) array of the memory
+ * box, read only at the tile's 2-D cells (i0+i, j0+j); column (i,j) is stepped with Nt_c = set_nc2d(i0+i, j0+j) * 1e6f, and
+ * re_cloud follows it.  kidmp_mp_gt_driver_tile_nc takes it on the host and checks every value it reads (finite, > 0) before
+ * anything is copied or launched; kidmp_mp_gt_driver_tile_device_nc takes it on the device, unchecked.  NULL: the handle's
+ * set_Nc.  Otherwise as kidmp_mp_gt_driver_tile / _device with ae = NULL. */
+int kidmp_mp_gt_driver_tile_nc(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const float* set_nc2d,
+                               float dt_in);
+int kidmp_mp_gt_driver_tile_device_nc(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t,
+                                      const float* d_set_nc2d, float dt_in, void* stream);
 
 /* Tuning knobs; results do not depend on them.
  * "chunk": columns per launch of the step kernels (default 1 048 576, or the KIDMP_CHUNK environment variable): the work

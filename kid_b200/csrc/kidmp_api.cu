@@ -7,6 +7,7 @@
 #include <cstring>
 #include <cstdarg>
 #include <cstdint>
+#include <cmath>
 #include <string>
 #include <vector>
 #include <map>
@@ -86,6 +87,7 @@ struct kidmp_handle {
   cudaEvent_t ev_done = nullptr;                          // end of the last step, on whatever stream it ran
   bool last_on_own_stream = true;
   double* d_diag = nullptr;
+  float* d_set_nc = nullptr; size_t set_nc_floats = 0;   // per-column set_Nc of kidmp_step_nc on the resident state
   float* d_rates = nullptr;                               // caller's device buffer (kidmp_set_rates_buffer) ...
   bool rates_on = false; float* d_rates_own = nullptr;    // ... or the handle's own, [36][nz][ncol] of the resident state (kidmp_enable_rates)
   float* d_kid = nullptr; size_t kid_floats = 0;   // staging of the KiD (k,i) arrays
@@ -335,20 +337,20 @@ int ensure_work(kidmp_handle* h, long cols, int nz) {
 #ifndef KC_AERO_MIX_B
 #define KC_AERO_MIX_B 2
 #endif
-template <bool RATES, bool AERO>
+template <bool RATES, bool AERO, bool NCOL>
 void launch_cells(kidmp_handle* h, const StepArgs& a, int nsm, cudaStream_t s, cudaEvent_t n0_done) {
   auto mark = [&](int q) { if (h->timing) cudaEventRecord(h->ev_k[q + 1], s); };
   // (the aerosol-aware instantiations carry more live values: one block per SM less keeps them out of local memory)
   constexpr int WB = AERO ? KC_AERO_WARM_B : KC_WARM_B, IB = AERO ? KC_AERO_ICE_B : KC_ICE_B, MB = AERO ? KC_AERO_MIX_B : KC_MIXNR_B,
                 FB = AERO ? KC_AERO_MIX_B : KC_FULL_B;
-  k_cells<KC_WARM, KC_WARM_T, WB, KC_WARM_BARS, RATES, AERO><<<nsm * WB, KC_WARM_T, 0, s>>>(a, h->kc);
+  k_cells<KC_WARM, KC_WARM_T, WB, KC_WARM_BARS, RATES, AERO, NCOL><<<nsm * WB, KC_WARM_T, 0, s>>>(a, h->kc);
   mark(KT_WARM);
-  k_cells<KC_ICE, KC_ICE_T, IB, KC_ICE_BARS, RATES, AERO><<<nsm * IB, KC_ICE_T, 0, s>>>(a, h->kc);
+  k_cells<KC_ICE, KC_ICE_T, IB, KC_ICE_BARS, RATES, AERO, NCOL><<<nsm * IB, KC_ICE_T, 0, s>>>(a, h->kc);
   mark(KT_ICE);
   if (n0_done) cudaStreamWaitEvent(s, n0_done, 0);     // only the classes with graupel read the intercept minima of k_n0_sweep
-  k_cells<KC_MIXNR, KC_MIXNR_T, MB, KC_MIXNR_BARS, RATES, AERO><<<nsm * MB, KC_MIXNR_T, 0, s>>>(a, h->kc);
+  k_cells<KC_MIXNR, KC_MIXNR_T, MB, KC_MIXNR_BARS, RATES, AERO, NCOL><<<nsm * MB, KC_MIXNR_T, 0, s>>>(a, h->kc);
   mark(KT_MIXNR);
-  k_cells<KC_FULL, KC_FULL_T, FB, KC_FULL_BARS, RATES, AERO><<<nsm * FB, KC_FULL_T, 0, s>>>(a, h->kc);
+  k_cells<KC_FULL, KC_FULL_T, FB, KC_FULL_BARS, RATES, AERO, NCOL><<<nsm * FB, KC_FULL_T, 0, s>>>(a, h->kc);
   mark(KT_FULL);
 }
 
@@ -416,6 +418,7 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
     if (a0.dz_col) a.dz_col = a0.dz_col + c0;
     if (a0.rates) a.rates = a0.rates + c0;
     if (a0.nc) { a.nc = a0.nc + c0; a.nwfa = a0.nwfa + c0; a.nifa = a0.nifa + c0; a.w = a0.w + c0; }
+    if (a0.set_nc) a.set_nc = a0.set_nc + c0;
     const long ngroups = (a.ncol + 31) / 32, lblocks = (a.ncol + LIST_TILE - 1) / LIST_TILE;
     a.scratch = w.d_scratch; a.scratch_b = w.d_scratch + (size_t)w.cols * w.nz * SC_HALF; a.cellidx = w.d_cellidx; a.cls = w.d_cls; a.colflag = w.d_colflag;
     a.work_count = w.d_work; a.work_list = w.d_work + 8;
@@ -458,19 +461,26 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
       mark(KT_LISTS); mark(KT_N0);
     }
     cudaEvent_t n0_done = serial ? nullptr : w.ev_n0_done;
-    const bool aero = a.nc != nullptr;                  // (an aerosol-aware step has no process-rate buffer: checked by its entry point)
-    if (aero) launch_cells<false, true>(h, a, h->nsm, s, n0_done);
-    else if (a.rates) launch_cells<true, false>(h, a, h->nsm, s, n0_done);
-    else launch_cells<false, false>(h, a, h->nsm, s, n0_done);
+    // (an aerosol-aware step has no process-rate buffer and no per-column droplet number: checked by the entry points)
+    const bool aero = a.nc != nullptr, per_col = a.set_nc != nullptr;
+    if (aero) launch_cells<false, true, false>(h, a, h->nsm, s, n0_done);
+    else if (per_col && a.rates) launch_cells<true, false, true>(h, a, h->nsm, s, n0_done);
+    else if (per_col) launch_cells<false, false, true>(h, a, h->nsm, s, n0_done);
+    else if (a.rates) launch_cells<true, false, false>(h, a, h->nsm, s, n0_done);
+    else launch_cells<false, false, false>(h, a, h->nsm, s, n0_done);
     k_carries<<<(unsigned)((a.ncol + 63) / 64), 64, 0, s>>>(a, h->kc);
     mark(KT_CARRIES);
     // the columns with sedimentation sub-steps on the second stream, the others on this one: disjoint columns
     fork(w.ev_fork, s, x);
     const unsigned sgrid = (unsigned)(ngroups < h->nsm * 16 ? ngroups : h->nsm * 16);
     if (aero) k_substeps<false, true><<<sgrid, 32, 0, x>>>(a, h->kc);
+    else if (per_col && a.rates) k_substeps<true, false, true><<<sgrid, 32, 0, x>>>(a, h->kc);
+    else if (per_col) k_substeps<false, false, true><<<sgrid, 32, 0, x>>>(a, h->kc);
     else if (a.rates) k_substeps<true, false><<<sgrid, 32, 0, x>>>(a, h->kc); else k_substeps<false, false><<<sgrid, 32, 0, x>>>(a, h->kc);
     mark(KT_SUBSTEPS);
     if (aero) k_finish<false, true><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
+    else if (per_col && a.rates) k_finish<true, false, true><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
+    else if (per_col) k_finish<false, false, true><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
     else if (a.rates) k_finish<true, false><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
     else k_finish<false, false><<<(unsigned)ngroups, 32, 0, s>>>(a, h->kc);
     mark(KT_FINISH);
@@ -561,7 +571,9 @@ int get_field(kidmp_handle* h, int layout, const float* src, float* dst) {
 #include <thread>
 extern "C" {
 static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* const fields[KIDMP_NFIELDS], const float* p,
-                          const float* dz, float* ppt, long hld);
+                          const float* dz, const float* set_nc, float* ppt, long hld);
+static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS], const float* p,
+                     const float* dz, const float* set_nc, float* ppt);
 }
 struct MultiCtx {
   std::vector<kidmp_handle*> dev;
@@ -594,7 +606,7 @@ template <class F> int on_all(kidmp_handle* h, F fn) {
 }
 
 int multi_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS], const float* p,
-               const float* dz, float* ppt) {
+               const float* dz, const float* set_nc, float* ppt) {
   MultiCtx* m = h->multi;
   const int n = (int)m->dev.size();
   for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "step: field %d is null", q);
@@ -608,11 +620,12 @@ int multi_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* 
     float* f[KIDMP_NFIELDS];
     if (layout == KIDMP_COL_FASTEST) {                // a column range of [nz][ncol] arrays: pitched copies
       for (int q = 0; q < KIDMP_NFIELDS; ++q) f[q] = fields[q] + c0;
-      return step_pipelined(c, c1 - c0, nz, dt, f, p + c0, dz, ppt ? ppt + c0 : nullptr, ncol);
+      return step_pipelined(c, c1 - c0, nz, dt, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, ppt ? ppt + c0 : nullptr, ncol);
     }
     for (int q = 0; q < KIDMP_NFIELDS; ++q) f[q] = fields[q] + (size_t)c0 * nz;   // KiD's (k,i) arrays: a range of columns is contiguous
     std::vector<float> pp(ppt ? (size_t)(c1 - c0) * 4 : 0);
-    if (kidmp_step(c, c1 - c0, nz, dt, layout, f, p + (size_t)c0 * nz, dz, ppt ? pp.data() : nullptr)) return 1;
+    if (step_host(c, c1 - c0, nz, dt, layout, f, p + (size_t)c0 * nz, dz, set_nc ? set_nc + c0 : nullptr, ppt ? pp.data() : nullptr))
+      return 1;
     if (ppt) for (int q = 0; q < 4; ++q) memcpy(ppt + (size_t)q * ncol + c0, pp.data() + (size_t)q * (c1 - c0), (size_t)(c1 - c0) * 4);
     return 0;
   });
@@ -890,6 +903,7 @@ int kidmp_finalize(kidmp_handle* h) {
   if (h->d_diag) cudaFree(h->d_diag);
   if (h->d_kid) cudaFree(h->d_kid);
   if (h->h_kid) cudaFreeHost(h->h_kid);
+  if (h->d_set_nc) cudaFree(h->d_set_nc);
   free_work(h->ws);
   for (cudaEvent_t e : {h->ws.ev_fork, h->ws.ev_join, h->ws.ev_lists_done, h->ws.ev_n0_done}) if (e) cudaEventDestroy(e);
   if (h->ws.aux) cudaStreamDestroy(h->ws.aux);
@@ -1165,6 +1179,24 @@ int kidmp_step_resident(kidmp_handle* h, float dt) {
   return 0;
 }
 
+static int ensure_dev(kidmp_handle* h, float** p, size_t* have, size_t need);
+
+// The host entries that take per-column set_Nc read every value before anything is copied or launched: each must be a valid
+// set_Nc of kidmp_init (finite, > 0).  n values at stride 1, or the (i,j) cells of a tile (2-D array of memory width ni_m).
+static int check_set_nc(kidmp_handle* h, const char* who, const float* v, long n) {
+  for (long c = 0; c < n; ++c)
+    if (!(v[c] > 0.f) || !std::isfinite(v[c])) return fail(h, "%s: set_nc[%ld] = %g, must be finite and positive", who, c, (double)v[c]);
+  return 0;
+}
+static int check_set_nc2d(kidmp_handle* h, const char* who, const float* v, const kidmp_wrf_tile* t, long ni_m) {
+  for (int j = t->j0; j < t->j0 + t->nj; ++j)
+    for (int i = t->i0; i < t->i0 + t->ni; ++i) {
+      const float x = v[i + ni_m * j];
+      if (!(x > 0.f) || !std::isfinite(x)) return fail(h, "%s: set_nc2d(%d,%d) = %g, must be finite and positive", who, i, j, (double)x);
+    }
+  return 0;
+}
+
 int kidmp_download(kidmp_handle* h, int layout, float* const fields[KIDMP_NFIELDS], float* ppt) {
   if (h && h->multi) return multi_copy(h, layout, fields, nullptr, nullptr, ppt, false);
   if (!h || !h->d_state) return h ? fail(h, "download before state_alloc") : 1;
@@ -1182,8 +1214,9 @@ int kidmp_download(kidmp_handle* h, int layout, float* const fields[KIDMP_NFIELD
 // SMs work at the same time.  Columns are independent, so chunking does not change any result.
 // `hld`: columns of the caller's host arrays (their row stride): a multi-device handle gives every device a range of columns
 // of the same arrays.
+// `set_nc`: per-column set_Nc of the ncol columns (host, contiguous) or NULL; each chunk takes its slice.
 static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* const fields[KIDMP_NFIELDS],
-                          const float* p, const float* dz, float* ppt, long hld) {
+                          const float* p, const float* dz, const float* set_nc, float* ppt, long hld) {
   // (no larger than a launch chunk: then every pipeline chunk is one launch of launch_step, whose column flags k_scatter_host reads)
   const long chunk = h->pipe_chunk < h->chunk_cols ? h->pipe_chunk : h->chunk_cols;
   const int NB = 3;
@@ -1192,7 +1225,7 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
   if (!h->copy_in) CK(h, cudaStreamCreateWithFlags(&h->copy_in, cudaStreamNonBlocking));
   if (!h->copy_out) CK(h, cudaStreamCreateWithFlags(&h->copy_out, cudaStreamNonBlocking));
   const size_t cells = (size_t)chunk * nz;
-  const size_t per_buf = cells * (KIDMP_NFIELDS + 1) + (size_t)chunk * 4;
+  const size_t per_buf = cells * (KIDMP_NFIELDS + 1) + (size_t)chunk * 5;   // fields and p, ppt [4][chunk], set_nc [chunk]
   if (h->pipe_floats < per_buf * NB || h->pipe_nz != nz) {
     if (h->d_pipe) cudaFree(h->d_pipe);
     h->d_pipe = nullptr; h->pipe_floats = 0;
@@ -1235,6 +1268,7 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
     const long n = (ncol - c0 < chunk) ? (ncol - c0) : chunk;
     float* base = h->d_pipe + per_buf * b;
     float* d_ppt = base + cells * (KIDMP_NFIELDS + 1);
+    float* const d_set_nc = d_ppt + (size_t)chunk * 4;
     const size_t dpitch = (size_t)n * 4;
     if (it >= NB) CK(h, cudaStreamWaitEvent(h->copy_in, h->pipe_ev[b][2], 0));     // buffer drained by its D2H
     tmark(h->copy_in);
@@ -1242,6 +1276,7 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
       const float* src = (q < KIDMP_NFIELDS ? fields[q] : p) + c0;
       CK(h, cudaMemcpy2DAsync(base + cells * q, dpitch, src, hpitch, dpitch, nz, cudaMemcpyHostToDevice, h->copy_in));
     }
+    if (set_nc) CK(h, cudaMemcpyAsync(d_set_nc, set_nc + c0, (size_t)n * 4, cudaMemcpyHostToDevice, h->copy_in));
     CK(h, cudaEventRecord(h->pipe_ev[b][0], h->copy_in));
     tmark(h->copy_in);
     CK(h, cudaStreamWaitEvent(h->stream, h->pipe_ev[b][0], 0));
@@ -1250,6 +1285,7 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
     a.ncol = n; a.ld = n; a.nz = nz; a.dt = dt;
     for (int q = 0; q < KIDMP_NFIELDS; ++q) a.f[q] = base + cells * q;
     a.p = base + cells * KIDMP_NFIELDS; a.dz = h->d_pipe_dz; a.ppt = d_ppt;
+    if (set_nc) a.set_nc = d_set_nc;
     if (launch_step(h, a, h->stream)) return 1;
     tmark(h->stream);
     CK(h, cudaEventRecord(h->pipe_ev[b][1], h->stream));
@@ -1287,22 +1323,47 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
   return 0;
 }
 
-int kidmp_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
-               const float* p, const float* dz, float* ppt) {
-  if (!h) return 1;
+// kidmp_step and kidmp_step_nc; set_nc (host, [ncol], checked by the caller) or NULL
+static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
+                     const float* p, const float* dz, const float* set_nc, float* ppt) {
   if (ncol == 0) return 0;                               // `do i = 1, nx` with nx = 0 (I:54): nothing to do, nothing touched
   if (!fields || !p || !dz) return fail(h, "step: null pointer");
-  if (h->multi) return multi_step(h, ncol, nz, dt, layout, fields, p, dz, ppt);
+  if (h->multi) return multi_step(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ppt);
   // (with a process-rate buffer set the whole domain goes through the resident path: the buffer is [36][nz][ncol] of the domain)
   if (layout == KIDMP_COL_FASTEST && ncol >= 2 * h->pipe_chunk && nz >= 2 && nz <= 256 && dt > 0.f && !h->d_rates) {
     for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "step: field %d is null", q);
     DevGuard guard_(h->device);
-    return step_pipelined(h, ncol, nz, dt, fields, p, dz, ppt, ncol);
+    return step_pipelined(h, ncol, nz, dt, fields, p, dz, set_nc, ppt, ncol);
   }
   if (kidmp_state_alloc(h, ncol, nz)) return 1;
   if (kidmp_upload(h, layout, fields, p, dz)) return 1;
-  if (kidmp_step_resident(h, dt)) return 1;
+  if (!set_nc) {
+    if (kidmp_step_resident(h, dt)) return 1;
+  } else {
+    DevGuard guard_(h->device);
+    if (ensure_dev(h, &h->d_set_nc, &h->set_nc_floats, (size_t)ncol)) return 1;
+    // (a captured step reads the values through the pointer when it is replayed: the copy is ordered before it on the stream)
+    CK(h, cudaMemcpyAsync(h->d_set_nc, set_nc, (size_t)ncol * 4, cudaMemcpyHostToDevice, h->stream));
+    StepArgs a = resident_args(h, dt);
+    a.set_nc = h->d_set_nc;
+    CK(h, cudaEventRecord(h->ev0, h->stream));
+    if (launch_step(h, a, h->stream)) return 1;
+    CK(h, cudaEventRecord(h->ev1, h->stream));
+  }
   return kidmp_download(h, layout, fields, ppt);
+}
+
+int kidmp_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
+               const float* p, const float* dz, float* ppt) {
+  if (!h) return 1;
+  return step_host(h, ncol, nz, dt, layout, fields, p, dz, nullptr, ppt);
+}
+
+int kidmp_step_nc(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
+                  const float* p, const float* dz, const float* set_nc, float* ppt) {
+  if (!h) return 1;
+  if (set_nc && ncol > 0 && check_set_nc(h, "step_nc", set_nc, ncol)) return 1;
+  return step_host(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ppt);
 }
 
 int kidmp_column(kidmp_handle* h, int nz, float dt, float* qv, float* qc, float* qi, float* qr, float* qs, float* qg,
@@ -1319,13 +1380,18 @@ int kidmp_column(kidmp_handle* h, int nz, float dt, float* qv, float* qc, float*
 
 int kidmp_step_device(kidmp_handle* h, long ncol, int nz, float dt, float* const d_fields[KIDMP_NFIELDS],
                       const float* d_p, const float* d_dz, float* d_ppt, void* stream) {
+  return kidmp_step_device_nc(h, ncol, nz, dt, d_fields, d_p, d_dz, nullptr, d_ppt, stream);
+}
+
+int kidmp_step_device_nc(kidmp_handle* h, long ncol, int nz, float dt, float* const d_fields[KIDMP_NFIELDS],
+                         const float* d_p, const float* d_dz, const float* d_set_nc, float* d_ppt, void* stream) {
   if (!h) return 1;
   if (h->multi) return fail(h, "step_device: device pointers belong to one device; use a single-device handle per GPU");
   if (ncol == 0) return 0;
   if (!d_fields || !d_p || !d_dz || !d_ppt) return fail(h, "step_device: null pointer");
   DevGuard guard_(h->device);
   StepArgs a{};
-  a.ncol = ncol; a.ld = ncol; a.nz = nz; a.dt = dt; a.rates = h->d_rates;
+  a.ncol = ncol; a.ld = ncol; a.nz = nz; a.dt = dt; a.rates = h->d_rates; a.set_nc = d_set_nc;
   for (int q = 0; q < KIDMP_NFIELDS; ++q) { if (!d_fields[q]) return fail(h, "step_device: field %d is null", q); a.f[q] = d_fields[q]; }
   a.p = d_p; a.dz = d_dz; a.ppt = d_ppt;
   cudaStream_t s = stream ? (cudaStream_t)stream : h->stream;
@@ -1473,7 +1539,10 @@ static int ensure_dev(kidmp_handle* h, float** p, size_t* have, size_t need) {
 // The kernels of one call on device arrays that a.t addresses, on stream s: the tile into the resident planes, the step,
 // the planes back into the tile, the accumulators.  ae4: nc nwfa nifa w of an aerosol-aware call (else NULL), nwfa2d or NULL,
 // with their planes in h->d_aero.  The caller sets a.t, the tile's arrays and a.dz_col; a.f, a.p, a.ppt are set here.
-static int wrf_kernels(kidmp_handle* h, WrfArgs& a, float* const* ae4, const float* nwfa2d, float dt_in, cudaStream_t s) {
+// a.set_nc: per-column set_Nc of the tile's columns [ni*nj] (NULL: the handle's); set_nc2d, when given, is the (i,j) array that
+// a.t addresses, gathered into a.set_nc first.
+static int wrf_kernels(kidmp_handle* h, WrfArgs& a, float* const* ae4, const float* nwfa2d, const float* set_nc2d, float dt_in,
+                       cudaStream_t s) {
   const long ncol = (long)a.t.ni * a.t.nj;
   const size_t n = (size_t)ncol * a.t.nk;
   if (ae4 && ensure_wev_table(h)) return 1;
@@ -1486,9 +1555,11 @@ static int wrf_kernels(kidmp_handle* h, WrfArgs& a, float* const* ae4, const flo
   WrfBox t2 = a.t;                                      // the (i,j) arrays: a box of one level
   t2.nk = 1; t2.nk_m = 1; t2.k0 = 0;
   k_wrf_gather<<<g, b, 0, s>>>(a);
+  if (set_nc2d) { k_ikj_planes<<<g2, b, 0, s>>>(const_cast<float*>(set_nc2d), const_cast<float*>(a.set_nc), t2, 1); ++h->launches; }   // (read only)
   if (s == h->stream) CK(h, cudaEventRecord(h->ev0, s));
   StepArgs sa = resident_args(h, dt_in);
   sa.dz_col = a.dz_col;
+  sa.set_nc = a.set_nc;
   float* const d_ae = h->d_aero;                         // aerosol-aware run: 4 planes and the nwfa2d plane
   if (ae4) {
     for (int q = 0; q < 4; ++q) k_ikj_planes<<<g, b, 0, s>>>(ae4[q], d_ae + n * q, a.t, 1);
@@ -1527,20 +1598,24 @@ static void tile_rows(float* tile, float* mem, const kidmp_wrf_tile& t, long ni_
     }
 }
 
-int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const kidmp_wrf_aerosols* ae,
-                            float dt_in) {
-  if (!h) return 1;
-  if (h->multi) return kidmp_mp_gt_driver_tile(h->multi->dev[0], w, t, ae, dt_in) ? fail(h, "%s", h->multi->dev[0]->err.c_str()) : 0;   // one tile, one device
-  if (wrf_check(h, ae ? "mp_gt_driver_aero" : "mp_gt_driver", w, t, ae, dt_in)) return 1;
+// kidmp_mp_gt_driver_tile and kidmp_mp_gt_driver_tile_nc (set_nc2d: host (i,j) array of the memory box, or NULL; never with ae)
+static int wrf_tile_host(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const kidmp_wrf_aerosols* ae,
+                         const float* set_nc2d, float dt_in) {
+  if (h->multi) return wrf_tile_host(h->multi->dev[0], w, t, ae, set_nc2d, dt_in) ? fail(h, "%s", h->multi->dev[0]->err.c_str()) : 0;   // one tile, one device
+  const char* who = set_nc2d ? "mp_gt_driver_tile_nc" : ae ? "mp_gt_driver_aero" : "mp_gt_driver";
+  if (wrf_check(h, who, w, t, ae, dt_in)) return 1;
+  if (set_nc2d && check_set_nc2d(h, who, set_nc2d, t, w->ni)) return 1;
   const bool radii = w->re_cloud && w->re_ice && w->re_snow;
   const long ncol = (long)t->ni * t->nj;
   if (kidmp_state_alloc(h, ncol, t->nk)) return 1;
   DevGuard guard_(h->device);
   const size_t n = (size_t)ncol * t->nk, n2 = (size_t)ncol;
-  // device staging: 12 three-dimensional inputs, the per-column dz in step layout, 3 radii, 7 two-dimensional arrays
-  if (ensure_dev(h, &h->d_kid, &h->kid_floats, (12 + 1 + 3) * n + 7 * n2)) return 1;
-  // one pinned buffer, one copy each way (as kidmp_kid_interface): the tile of the 12 inputs, 7 accumulators, 4 aerosol arrays + nwfa2d
-  const size_t hfloats = 12 * n + 7 * n2 + (ae ? 4 * n + n2 : 0);
+  // device staging: 12 three-dimensional inputs, the per-column dz in step layout, 3 radii, 7 two-dimensional arrays, set_nc
+  const size_t nc2 = set_nc2d ? n2 : 0;
+  if (ensure_dev(h, &h->d_kid, &h->kid_floats, (12 + 1 + 3) * n + 7 * n2 + nc2)) return 1;
+  // one pinned buffer, one copy each way (as kidmp_kid_interface): the tile of the 12 inputs, 7 accumulators, 4 aerosol arrays + nwfa2d,
+  // set_nc
+  const size_t hfloats = 12 * n + 7 * n2 + (ae ? 4 * n + n2 : 0) + nc2;
   if (h->h_kid_floats < hfloats) {
     if (h->h_kid) cudaFreeHost(h->h_kid);
     h->h_kid = nullptr; h->h_kid_floats = 0;
@@ -1564,6 +1639,8 @@ int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const ki
     for (int q = 0; q < 4; ++q) tile_rows(h_ae + n * q, const_cast<float*>(in4[q]), *t, ni_m, nk_m, true);
     if (ae->nwfa2d) tile_rows(h_ae + 4 * n, const_cast<float*>(ae->nwfa2d), t2, ni_m, 1, true);
   }
+  float* const h_nc = h_ae + (ae ? 4 * n + n2 : 0);
+  if (set_nc2d) tile_rows(h_nc, const_cast<float*>(set_nc2d), t2, ni_m, 1, true);                  // (read only)
   // on the device the packed tile is a memory box of its own
   WrfArgs a{};
   a.t = WrfBox{t->ni, t->nk, t->nj, 0, 0, 0, t->ni, t->nk};
@@ -1577,11 +1654,13 @@ int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const ki
   if (w->snownc && w->snowncv) { a.snownc = d_2d + 3 * n2; a.snowncv = d_2d + 4 * n2; }
   if (w->graupelnc && w->graupelncv) { a.graupelnc = d_2d + 5 * n2; a.graupelncv = d_2d + 6 * n2; }
   float* const d_aet = ae ? h->d_aero + 4 * n + n2 : nullptr;
+  if (set_nc2d) a.set_nc = d_2d + 7 * n2;                // the packed tile's (i,j) cells are its columns, in step order
   CK(h, cudaMemcpyAsync(h->d_kid, h->h_kid, 12 * n * 4, cudaMemcpyHostToDevice, h->stream));
   CK(h, cudaMemcpyAsync(d_2d, h_2d, 7 * n2 * 4, cudaMemcpyHostToDevice, h->stream));
+  if (set_nc2d) CK(h, cudaMemcpyAsync(d_2d + 7 * n2, h_nc, n2 * 4, cudaMemcpyHostToDevice, h->stream));
   if (ae) CK(h, cudaMemcpyAsync(d_aet, h_ae, (4 * n + n2) * 4, cudaMemcpyHostToDevice, h->stream));
   float* const ae4[4] = {d_aet, d_aet + n, d_aet + 2 * n, d_aet + 3 * n};
-  if (wrf_kernels(h, a, ae ? ae4 : nullptr, ae && ae->nwfa2d ? d_aet + 4 * n : nullptr, dt_in, h->stream)) return 1;
+  if (wrf_kernels(h, a, ae ? ae4 : nullptr, ae && ae->nwfa2d ? d_aet + 4 * n : nullptr, nullptr, dt_in, h->stream)) return 1;
   CK(h, cudaMemcpyAsync(h->h_kid, h->d_kid, 9 * n * 4, cudaMemcpyDeviceToHost, h->stream));
   float* const h_re = h->h_kid + n * 9;               // pii, p, dz slots of the pinned buffer are free again
   if (radii) CK(h, cudaMemcpyAsync(h_re, d_re, 3 * n * 4, cudaMemcpyDeviceToHost, h->stream));
@@ -1603,16 +1682,26 @@ int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const ki
   return 0;
 }
 
-int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t,
-                                   const kidmp_wrf_aerosols* ae, float dt_in, void* stream) {
+int kidmp_mp_gt_driver_tile(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const kidmp_wrf_aerosols* ae,
+                            float dt_in) {
   if (!h) return 1;
+  return wrf_tile_host(h, w, t, ae, nullptr, dt_in);
+}
+int kidmp_mp_gt_driver_tile_nc(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const float* set_nc2d,
+                               float dt_in) {
+  if (!h) return 1;
+  return wrf_tile_host(h, w, t, nullptr, set_nc2d, dt_in);
+}
+
+static int wrf_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const kidmp_wrf_aerosols* ae,
+                           const float* d_set_nc2d, float dt_in, void* stream) {
   if (h->multi) return fail(h, "mp_gt_driver_tile_device: device pointers belong to one device; use a single-device handle per GPU");
-  if (wrf_check(h, "mp_gt_driver_tile_device", w, t, ae, dt_in)) return 1;
+  if (wrf_check(h, d_set_nc2d ? "mp_gt_driver_tile_device_nc" : "mp_gt_driver_tile_device", w, t, ae, dt_in)) return 1;
   const long ncol = (long)t->ni * t->nj;
   if (kidmp_state_alloc(h, ncol, t->nk)) return 1;
   DevGuard guard_(h->device);
   const size_t n = (size_t)ncol * t->nk, n2 = (size_t)ncol;
-  if (ensure_dev(h, &h->d_kid, &h->kid_floats, n)) return 1;          // the per-column dz in step layout
+  if (ensure_dev(h, &h->d_kid, &h->kid_floats, n + (d_set_nc2d ? n2 : 0))) return 1;   // the per-column dz in step layout, set_nc
   if (ae && ensure_dev(h, &h->d_aero, &h->aero_floats, 4 * n + n2)) return 1;
   WrfArgs a{};
   a.t = WrfBox{t->ni, t->nk, t->nj, t->i0, t->k0, t->j0, w->ni, w->nk};
@@ -1620,13 +1709,24 @@ int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, c
   for (int q = 0; q < 9; ++q) a.a3[q] = io[q];
   a.pii = w->pii; a.p3 = w->p; a.dz3 = w->dz;
   a.dz_col = h->d_kid;
+  if (d_set_nc2d) a.set_nc = h->d_kid + n;
   if (w->re_cloud && w->re_ice && w->re_snow) { a.re_cloud = w->re_cloud; a.re_ice = w->re_ice; a.re_snow = w->re_snow; }
   a.rainnc = w->rainnc; a.rainncv = w->rainncv; a.sr = w->sr;
   if (w->snownc && w->snowncv) { a.snownc = w->snownc; a.snowncv = w->snowncv; }
   if (w->graupelnc && w->graupelncv) { a.graupelnc = w->graupelnc; a.graupelncv = w->graupelncv; }
   cudaStream_t s = stream ? (cudaStream_t)stream : h->stream;
   float* const ae4[4] = {ae ? ae->nc : nullptr, ae ? ae->nwfa : nullptr, ae ? ae->nifa : nullptr, ae ? const_cast<float*>(ae->w) : nullptr};
-  return wrf_kernels(h, a, ae ? ae4 : nullptr, ae ? ae->nwfa2d : nullptr, dt_in, s);
+  return wrf_kernels(h, a, ae ? ae4 : nullptr, ae ? ae->nwfa2d : nullptr, d_set_nc2d, dt_in, s);
+}
+int kidmp_mp_gt_driver_tile_device(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t,
+                                   const kidmp_wrf_aerosols* ae, float dt_in, void* stream) {
+  if (!h) return 1;
+  return wrf_tile_device(h, w, t, ae, nullptr, dt_in, stream);
+}
+int kidmp_mp_gt_driver_tile_device_nc(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const float* d_set_nc2d,
+                                      float dt_in, void* stream) {
+  if (!h) return 1;
+  return wrf_tile_device(h, w, t, nullptr, d_set_nc2d, dt_in, stream);
 }
 
 int kidmp_set_option(kidmp_handle* h, const char* name, int value) {

@@ -21,6 +21,7 @@
 //                                levels.  Idle cells never had a hand-off record: their tendencies are zero and their
 //                                contents R1 / R2 by construction.
 // AERO (template parameter of k_cells, k_finish, k_substeps): is_aerosol_aware = .true., M:28 (kidmp_aero.cuh).
+// NCOL (the same three): the plain scheme with a droplet number per column (StepArgs::set_nc) instead of the handle's.
 // Pruning rule: a block is compiled out of a class kernel only when it cannot execute for any cell of the class, so
 // every class kernel computes bit for bit what the general code (KC_FULL) computes for the same cell.
 #pragma once
@@ -258,7 +259,9 @@ __global__ void __launch_bounds__(128) k_n0_sweep(StepArgs a, const __grid_const
 // classes with the long bodies; the short ones run free.
 // AERO: is_aerosol_aware = .true. (M:28): cloud droplet number, water-friendly and ice-friendly aerosol numbers are prognostic
 // (a.nc, a.nwfa, a.nifa), a.w feeds the droplet activation; every aerosol block is compiled out of the default kernels.
-template <int KC, int THREADS, int MINB, int BARS, bool RATES, bool AERO>
+// NCOL: the droplet number of the plain scheme is the cell's column's (Nt_c = a.set_nc[col] * 1e6f, M:381) instead of the
+// handle's ck.Nt_c; never with AERO, where the droplet number is prognostic.
+template <int KC, int THREADS, int MINB, int BARS, bool RATES, bool AERO, bool NCOL = false>
 __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a, const __grid_constant__ KConst ck) {
   using TR = CellTraits<KC>;
   constexpr bool LOCK = BARS != 0;
@@ -272,7 +275,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a, const __gri
   constexpr bool COMPACT = !AERO && (KC == KC_WARM || KC == KC_ICE);         // ... and the half that only k_finish reads (RecA)
   const float DT = a.dt;
   const float odt = 1.f / DT, odts = 1.f / DT;
-  const float Nt_c = ck.Nt_c;
+  const float Nt_c_h = ck.Nt_c;
   const bool iiwarm = ck.iiwarm != 0;
   const double n0_empty = ck.n0_lo;
 #define LOCKBAR(i) do { if (LOCK && ((BARS >> (i)) & 1)) { __syncwarp(); asm volatile("bar.sync 1, %0;" ::"r"(lock_threads) : "memory"); } } while (0)
@@ -289,6 +292,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_cells(StepArgs a, const __gri
     const unsigned slot = e & 0xffffffu;
     const long col = a.work_list[slot];
     const long o = (long)k * ld + col;
+    const float Nt_c = NCOL ? a.set_nc[col] * 1.e6f : Nt_c_h;
     LOCKBAR(0);
     const float t1d = a.f[F_T][o], qv1d = a.f[F_QV][o], pres = a.p[o];
     float qc1d = TR::C ? a.f[F_QC][o] : 0.0f, qi1d = TR::I ? a.f[F_QI][o] : 0.0f, qr1d = TR::R ? a.f[F_QR][o] : 0.0f,
@@ -1445,7 +1449,7 @@ __device__ __forceinline__ void idle_record(const KConst& ck, float temp, float 
 // does for the other columns.  Runs beside k_finish on a second stream: the two kernels own different columns.
 enum { WS_TTEN = 0, WS_QVTEN, WS_QCTEN, WS_QITEN, WS_QRTEN, WS_QSTEN, WS_QGTEN, WS_NITEN, WS_NRTEN, WS_NCTEN,
        WS_RR, WS_NR, WS_RI, WS_NI, WS_RS, WS_RG, WS_VTR, WS_VTNR, WS_VTI, WS_VTNI, WS_VTS, WS_VTG, WS_RHO, WS_S15, WS_NWFAT, WS_NIFAT, WS_N };
-template <bool RATES, bool AERO>
+template <bool RATES, bool AERO, bool NCOL = false>
 __global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a, const __grid_constant__ KConst ck) {
   const int n = *a.sub_count, count = *a.work_count;
   const unsigned k1_list = (unsigned)a.cell_kstart[KC_ICE], k2_list = (unsigned)a.cell_kstart[KC_MIXNR];
@@ -1516,7 +1520,8 @@ __global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a, const __grid_co
                                 nz, cs, s.n_g - 1, s.ksed_g, s.on_g, DT, sedi, 0.f, ppt_g);
     // last sub-step of every species + S15 + S16, one top-down sweep
     SedParams sp;
-    sp.DT = DT; sp.odt = odt; sp.on_r = s.on_r; sp.on_i = s.on_i; sp.on_s = s.on_s; sp.on_g = s.on_g; sp.Nt_c = ck.Nt_c;
+    sp.DT = DT; sp.odt = odt; sp.on_r = s.on_r; sp.on_i = s.on_i; sp.on_s = s.on_s; sp.on_g = s.on_g;
+    sp.Nt_c = NCOL ? a.set_nc[col] * 1.e6f : ck.Nt_c;
     sp.top_r = s.ksed_r; sp.top_i = s.ksed_i; sp.top_s = s.ksed_s; sp.top_g = s.ksed_g; sp.sedi = sedi; sp.iiwarm = iiwarm;
     SedCarry c;
     c.sr_up = 0.f; c.snr_up = 0.f; c.si_up = 0.f; c.sni_up = 0.f; c.ss_up = 0.f; c.sg_up = 0.f;
@@ -1556,7 +1561,7 @@ __global__ void __launch_bounds__(32, 16) k_substeps(StepArgs a, const __grid_co
 #ifndef K2_MINB
 #define K2_MINB 20
 #endif
-template <bool RATES, bool AERO>
+template <bool RATES, bool AERO, bool NCOL = false>
 __global__ void __launch_bounds__(32, K2_MINB) k_finish(StepArgs a, const __grid_constant__ KConst ck) {
   const int slot = blockIdx.x * 32 + threadIdx.x;
   const int count = *a.work_count;
@@ -1584,7 +1589,8 @@ __global__ void __launch_bounds__(32, K2_MINB) k_finish(StepArgs a, const __grid
   const float* const dzp = a.dz_col ? a.dz_col + col : a.dz;
   const long dzs = a.dz_col ? ld : 1;
   SedParams sp;
-  sp.DT = DT; sp.odt = odt; sp.on_r = s.on_r; sp.on_i = s.on_i; sp.on_s = s.on_s; sp.on_g = s.on_g; sp.Nt_c = ck.Nt_c;
+  sp.DT = DT; sp.odt = odt; sp.on_r = s.on_r; sp.on_i = s.on_i; sp.on_s = s.on_s; sp.on_g = s.on_g;
+  sp.Nt_c = NCOL ? a.set_nc[col] * 1.e6f : ck.Nt_c;
   sp.top_r = s.ksed_r; sp.top_i = s.ksed_i; sp.top_s = s.ksed_s; sp.top_g = s.ksed_g; sp.sedi = ck.l_sediment != 0; sp.iiwarm = iiwarm;
   SedCarry c;
   c.sr_up = 0.f; c.snr_up = 0.f; c.si_up = 0.f; c.sni_up = 0.f; c.ss_up = 0.f; c.sg_up = 0.f;

@@ -171,6 +171,9 @@ struct StepArgs {
   // aerosol-aware runs (is_aerosol_aware = .true., M:28): prognostic droplet number and aerosol numbers, vertical velocity
   float* nc; float* nwfa; float* nifa;   // [nz][ld] INOUT
   const float* w;                        // [nz][ld] IN
+  // per-column droplet number of the plain scheme: set_Nc [cm^-3] of every column, [ld]; Nt_c = set_nc[col] * 1e6f (M:381).
+  // NULL: ck.Nt_c everywhere.  Read only by the NCOL instantiations of k_cells, k_substeps and k_finish.
+  const float* set_nc;
   int nsm;                     // SMs of the device
   int no_simple;               // 1: every cloudy column goes through the counts of k_carries ("simple" option off: for A/B runs)
   int no_classes;              // 1: every busy cell goes to k_cells<KC_FULL> ("classes" option off: the class kernels' reference)

@@ -40,6 +40,7 @@ struct WrfArgs {
   float *rainnc, *rainncv, *sr, *snownc, *snowncv, *graupelnc, *graupelncv;   // (i,j); the last four may be NULL
   float *re_cloud, *re_ice, *re_snow;   // (i,k,j), all three or none (has_reqc, has_reqi, has_reqs, M:1110)
   const float* nc_plane;                // [nk][ni*nj] prognostic droplet number of an aerosol-aware run, else NULL (nc = Nt_c, M:4875)
+  const float* set_nc;                  // [ni*nj] set_Nc of every column of a per-column run (Nt_c = set_nc * 1e6f), else NULL
 };
 
 // one (i,k,j) array <-> one [k][col] plane of the step; x: i, y: k, z: j.  A 2-D (i,j) array is the box with nk = nk_m = 1.
@@ -81,7 +82,8 @@ __global__ void k_wrf_scatter(WrfArgs a, const __grid_constant__ KConst ck) {
     float re_qc = 2.49E-6f, re_qi = 4.99E-6f, re_qs = 9.99E-6f;          // M:1112-1114
     const float rho = 0.622f * p1d / (KP_R * t1d * (qv1d + 0.622f));
     const float rc = fmaxf(KP_R1, qc1d * rho);
-    const float nc = a.nc_plane ? fmaxf(KP_R2, a.nc_plane[src] * rho) : ck.Nt_c;    // M:4874-4875
+    const float nc = a.nc_plane ? fmaxf(KP_R2, a.nc_plane[src] * rho)                // M:4874-4875
+                   : a.set_nc ? a.set_nc[(long)j * a.t.ni + i] * 1.e6f : ck.Nt_c;
     const float ri = fmaxf(KP_R1, qi1d * rho);
     const float ni = fmaxf(KP_R2, ni1d * rho);
     const float rs = fmaxf(KP_R1, qs1d * rho);

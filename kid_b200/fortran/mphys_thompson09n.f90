@@ -140,6 +140,27 @@ module mphys_thompson09n
        real(c_float), value :: dt_in
        type(c_ptr), value :: stream
      end function kidmp_mp_gt_driver_tile_device
+     ! the plain scheme with a cloud droplet number per column: set_nc2d(ims:ime,jms:jme) holds set_Nc [cm^-3] of every column
+     ! (e.g. land and ocean values); only the tile's cells are read.  Host array, every value read must be finite and > 0 ...
+     integer(c_int) function kidmp_mp_gt_driver_tile_nc(handle, w, t, set_nc2d, dt_in) bind(C, name='kidmp_mp_gt_driver_tile_nc')
+       import :: c_int, c_ptr, c_float, kidmp_wrf_fields, kidmp_wrf_tile
+       type(c_ptr), value :: handle
+       type(kidmp_wrf_fields), intent(in) :: w
+       type(kidmp_wrf_tile), intent(in) :: t
+       real(c_float), intent(in) :: set_nc2d(*)
+       real(c_float), value :: dt_in
+     end function kidmp_mp_gt_driver_tile_nc
+     ! ... or device array (c_loc of device data), enqueued on `stream` like kidmp_mp_gt_driver_tile_device
+     integer(c_int) function kidmp_mp_gt_driver_tile_device_nc(handle, w, t, set_nc2d, dt_in, stream) &
+          bind(C, name='kidmp_mp_gt_driver_tile_device_nc')
+       import :: c_int, c_ptr, c_float, kidmp_wrf_fields, kidmp_wrf_tile
+       type(c_ptr), value :: handle
+       type(kidmp_wrf_fields), intent(in) :: w
+       type(kidmp_wrf_tile), intent(in) :: t
+       type(c_ptr), value :: set_nc2d
+       real(c_float), value :: dt_in
+       type(c_ptr), value :: stream
+     end function kidmp_mp_gt_driver_tile_device_nc
   end interface
 
   !Logical switches

@@ -51,6 +51,8 @@ SYMBOLS = {
     "kidmp_step_device": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.POINTER(C.c_void_p), C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p]),
     "kidmp_step_device_aero": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.POINTER(C.c_void_p)] + [C.c_void_p] * 9),
+    "kidmp_step_nc": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.c_int, _fpp, _fp, _fp, _fp, _fp]),
+    "kidmp_step_device_nc": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.POINTER(C.c_void_p)] + [C.c_void_p] * 5),
     "kidmp_set_rates_buffer": (C.c_int, [C.c_void_p, C.c_void_p]),
     "kidmp_rate_names": (C.c_char_p, []),
     "kidmp_enable_rates": (C.c_int, [C.c_void_p, C.c_int]),
@@ -105,6 +107,9 @@ SYMBOLS["kidmp_mp_gt_driver_tile"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields)
                                                 C.c_float])
 SYMBOLS["kidmp_mp_gt_driver_tile_device"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields), C.POINTER(WrfTile),
                                                        C.POINTER(WrfAerosols), C.c_float, C.c_void_p])
+SYMBOLS["kidmp_mp_gt_driver_tile_nc"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields), C.POINTER(WrfTile), _fp, C.c_float])
+SYMBOLS["kidmp_mp_gt_driver_tile_device_nc"] = (C.c_int, [C.c_void_p, C.POINTER(WrfFields), C.POINTER(WrfTile), C.c_void_p,
+                                                          C.c_float, C.c_void_p])
 SYMBOLS["kidmp_kid_interface"] = (C.c_int, [C.c_void_p, C.POINTER(KidColumns), C.c_float, C.c_float, C.c_float])
 HYD_PLANES = ("qc", "qr", "nr", "qi", "ni", "qs", "qg")
 
@@ -235,16 +240,23 @@ class Thompson:
         a["ppt"] = ppt4
         return a
 
-    def step(self, dt, state, p, dz, layout="col_fastest"):
+    def step(self, dt, state, p, dz, layout="col_fastest", set_nc=None):
         """Host arrays in, host arrays out (in place).  state: dict by FIELDS of float32 arrays,
-        (nz, ncol) for 'col_fastest' or (ncol, nz) for 'k_fastest'.  Returns ppt[4, ncol]."""
+        (nz, ncol) for 'col_fastest' or (ncol, nz) for 'k_fastest'.  Returns ppt[4, ncol].
+        set_nc: float32 (ncol,) set_Nc [cm^-3] of every column (plain scheme, kidmp_step_nc); None = the handle's set_Nc."""
         lay = K_FASTEST if layout == "k_fastest" else COL_FASTEST
         t = _f32c(state["t"])
         ncol, nz = (t.shape if lay == K_FASTEST else t.shape[::-1])
         arrs = [_f32c(state[k]) for k in FIELDS]
         ppt = np.zeros((4, ncol), np.float32)
-        self._ck(self._L.kidmp_step(self.h, ncol, nz, float(dt), lay, _ptrs(arrs), _f32c(p).ctypes.data_as(_fp),
-                                    np.ascontiguousarray(dz, np.float32).ctypes.data_as(_fp), ppt.ctypes.data_as(_fp)))
+        args = (self.h, ncol, nz, float(dt), lay, _ptrs(arrs), _f32c(p).ctypes.data_as(_fp),
+                np.ascontiguousarray(dz, np.float32).ctypes.data_as(_fp))
+        if set_nc is None:
+            self._ck(self._L.kidmp_step(*args, ppt.ctypes.data_as(_fp)))
+        else:
+            if np.shape(set_nc) != (ncol,):
+                raise ValueError("set_nc shape %r, expected (%d,)" % (np.shape(set_nc), ncol))
+            self._ck(self._L.kidmp_step_nc(*args, _f32c(set_nc).ctypes.data_as(_fp), ppt.ctypes.data_as(_fp)))
         return ppt
 
     def state_alloc(self, ncol, nz):
@@ -267,12 +279,17 @@ class Thompson:
         self._ck(self._L.kidmp_download(self.h, lay, fp, ppt.ctypes.data_as(_fp) if want_ppt else None))
         return ppt
 
-    def step_device(self, ncol, nz, dt, field_ptrs, p_ptr, dz_ptr, ppt_ptr, stream=None):
-        """Device pointers (ints, e.g. torch.Tensor.data_ptr()), COL_FASTEST layout; asynchronous."""
+    def step_device(self, ncol, nz, dt, field_ptrs, p_ptr, dz_ptr, ppt_ptr, stream=None, set_nc_ptr=None):
+        """Device pointers (ints, e.g. torch.Tensor.data_ptr()), COL_FASTEST layout; asynchronous.
+        set_nc_ptr: device float32 [ncol] set_Nc of every column (kidmp_step_device_nc), None = the handle's set_Nc."""
         fp = (C.c_void_p * NFIELDS)(*[C.c_void_p(int(x)) for x in field_ptrs])
-        self._ck(self._L.kidmp_step_device(self.h, int(ncol), int(nz), float(dt), fp, C.c_void_p(int(p_ptr)),
-                                           C.c_void_p(int(dz_ptr)), C.c_void_p(int(ppt_ptr)),
-                                           C.c_void_p(int(stream)) if stream else None))
+        s = C.c_void_p(int(stream)) if stream else None
+        if set_nc_ptr is None:
+            self._ck(self._L.kidmp_step_device(self.h, int(ncol), int(nz), float(dt), fp, C.c_void_p(int(p_ptr)),
+                                               C.c_void_p(int(dz_ptr)), C.c_void_p(int(ppt_ptr)), s))
+        else:
+            self._ck(self._L.kidmp_step_device_nc(self.h, int(ncol), int(nz), float(dt), fp, C.c_void_p(int(p_ptr)),
+                                                  C.c_void_p(int(dz_ptr)), C.c_void_p(int(set_nc_ptr)), C.c_void_p(int(ppt_ptr)), s))
 
     def step_device_aero(self, ncol, nz, dt, field_ptrs, nc_ptr, nwfa_ptr, nifa_ptr, p_ptr, w_ptr, dz_ptr, ppt_ptr, nwfa2d_ptr=None,
                          stream=None):
@@ -292,7 +309,7 @@ class Thompson:
         """kidmp_set_option: tuning knobs that do not change results ("chunk": columns per launch, "timing": 0 / 1)."""
         self._ck(self._L.kidmp_set_option(self.h, name.encode(), int(value)))
 
-    def mp_gt_driver(self, dt, f3, pii, p, dz, acc, radii=True, aerosols=None, tile=None):
+    def mp_gt_driver(self, dt, f3, pii, p, dz, acc, radii=True, aerosols=None, tile=None, set_nc=None):
         """mp_gt_driver (M:806-1143) through kidmp_mp_gt_driver.  f3: dict qv qc qr qi qs qg ni nr th of (nj, nk, ni)
         float32 arrays (C order = WRF's (i,k,j) Fortran order), updated in place; pii, p, dz the same shape; acc: dict
         rainnc rainncv sr [snownc snowncv graupelnc graupelncv] of (nj, ni) arrays, updated in place.
@@ -302,10 +319,20 @@ class Thompson:
         spare levels included), through kidmp_mp_gt_driver_tile; nothing outside the tile is read or written.
         radii: True = new zero arrays of the memory box's shape, returned (outside a tile they stay zero); a dict of
         re_cloud re_ice re_snow arrays = those, filled in place; False = no radii.
+        set_nc: (nj, ni) float32 set_Nc [cm^-3] of every column of the memory box (plain scheme, kidmp_mp_gt_driver_tile_nc;
+        read at the tile's cells only); None = the handle's set_Nc.
         Returns dict re_cloud re_ice re_snow (empty when radii is False)."""
         nj, nk, ni = f3["qv"].shape
         w, ae, re, keep = self._wrf_structs(f3, pii, p, dz, acc, radii, aerosols, (nj, nk, ni), lambda a: _f32c(a).ctypes.data_as(_fp))
-        if tile is not None:
+        if set_nc is not None:
+            if ae is not None:
+                raise ValueError("set_nc is for the plain scheme: not with aerosols")
+            if np.shape(set_nc) != (nj, ni):
+                raise ValueError("set_nc shape %r, expected %r" % (np.shape(set_nc), (nj, ni)))
+            t = WrfTile(*[int(x) for x in (tile if tile is not None else (0, ni, 0, nk, 0, nj))])
+            self._ck(self._L.kidmp_mp_gt_driver_tile_nc(self.h, C.byref(w), C.byref(t), _f32c(set_nc).ctypes.data_as(_fp),
+                                                        float(dt)))
+        elif tile is not None:
             t = WrfTile(*[int(x) for x in tile])
             self._ck(self._L.kidmp_mp_gt_driver_tile(self.h, C.byref(w), C.byref(t), C.byref(ae) if ae is not None else None,
                                                      float(dt)))
@@ -315,18 +342,28 @@ class Thompson:
             self._ck(self._L.kidmp_mp_gt_driver(self.h, C.byref(w), float(dt)))
         return re
 
-    def mp_gt_driver_device(self, dt, f3, pii, p, dz, acc, tile=None, radii=None, aerosols=None, stream=None):
+    def mp_gt_driver_device(self, dt, f3, pii, p, dz, acc, tile=None, radii=None, aerosols=None, stream=None, set_nc=None):
         """kidmp_mp_gt_driver_tile_device: the same step on device arrays (anything with data_ptr(), e.g. contiguous float32
         CUDA tensors of the shapes of mp_gt_driver), enqueued on `stream` (a torch.cuda.Stream, a cudaStream_t as int, or
         None = the handle's stream) without synchronising.  tile None = the whole memory box.  radii: dict re_cloud re_ice
-        re_snow of device arrays (filled inside the tile) or None."""
+        re_snow of device arrays (filled inside the tile) or None.  set_nc: (nj, ni) device array of set_Nc per column
+        (plain scheme, kidmp_mp_gt_driver_tile_device_nc), None = the handle's set_Nc."""
         nj, nk, ni = f3["qv"].shape
         w, ae, _, keep = self._wrf_structs(f3, pii, p, dz, acc, radii or False, aerosols, (nj, nk, ni),
                                            lambda a: C.cast(C.c_void_p(int(a.data_ptr())), _fp))
         t = WrfTile(*[int(x) for x in (tile if tile is not None else (0, ni, 0, nk, 0, nj))])
         s = getattr(stream, "cuda_stream", stream)
-        self._ck(self._L.kidmp_mp_gt_driver_tile_device(self.h, C.byref(w), C.byref(t), C.byref(ae) if ae is not None else None,
-                                                        float(dt), C.c_void_p(int(s)) if s else None))
+        s = C.c_void_p(int(s)) if s else None
+        if set_nc is not None:
+            if ae is not None:
+                raise ValueError("set_nc is for the plain scheme: not with aerosols")
+            if tuple(set_nc.shape) != (nj, ni) or not set_nc.is_contiguous() or str(set_nc.dtype) != "torch.float32":
+                raise ValueError("set_nc: float32 contiguous tensor of shape %r required" % ((nj, ni),))
+            self._ck(self._L.kidmp_mp_gt_driver_tile_device_nc(self.h, C.byref(w), C.byref(t), C.c_void_p(int(set_nc.data_ptr())),
+                                                               float(dt), s))
+        else:
+            self._ck(self._L.kidmp_mp_gt_driver_tile_device(self.h, C.byref(w), C.byref(t), C.byref(ae) if ae is not None else None,
+                                                            float(dt), s))
 
     @staticmethod
     def _wrf_structs(f3, pii, p, dz, acc, radii, aerosols, shape3, addr):
