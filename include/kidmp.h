@@ -78,7 +78,9 @@ int kidmp_column(kidmp_handle* h, int nz, float dt,
 
 /* the body of `do i = 1, nx` (I:54-246) for ncol independent columns: host arrays in, host
  * arrays out (H2D, kernels, D2H inside the call).  dz is one shared vector of nz (I:63).
- * Large KIDMP_COL_FASTEST domains flow through the device in chunks on three streams.  When the nine field arrays are
+ * Large KIDMP_COL_FASTEST domains flow through the device in chunks on three streams, unless process rates are kept (a
+ * buffer of kidmp_set_rates_buffer, or kidmp_enable_rates): then the whole domain goes through the resident state, the rates
+ * are those of the whole domain, and nothing travels back by the zero-copy path below.  When the nine field arrays are
  * PINNED host memory (cudaHostAlloc / cudaHostRegister), only the columns the step changed travel back - a clear-sky column
  * is returned bit for bit by the reference too (M:1540) - written by a kernel straight into the host arrays.
  * ncol = 0 (here, in kidmp_step_device and as kidmp_kid_columns::nx) is the empty loop of I:54: success, nothing touched. */
@@ -137,9 +139,17 @@ int kidmp_step_device_aero(kidmp_handle* h, long ncol, int nz, float dt, float* 
 int kidmp_set_rates_buffer(kidmp_handle* h, float* d_rates);
 const char* kidmp_rate_names(void);
 /* The same rates for a HOST caller (the Fortran shim's save_dg calls, M:2963-3120): kidmp_enable_rates(h, 1) makes the handle
- * keep its own [36][nz][ncol] buffer for the resident state (every entry point that steps the resident state fills it:
- * kidmp_kid_interface, kidmp_step_resident, kidmp_column ...; zero where no process ran), kidmp_get_rates copies it to
- * `rates`: [36][nz][ncol] for KIDMP_COL_FASTEST, [36][ncol][nz] (KiD's (k,i) order, plane by plane) for KIDMP_K_FASTEST. */
+ * keep its own [36][nz][ncol] buffer for the resident state (36*nz*ncol floats of device memory).  Every entry point that steps
+ * the resident state fills it, zero where no process ran: kidmp_step and kidmp_step_nc (with rates kept every kidmp_step
+ * domain goes through the resident state, see kidmp_step), kidmp_step_resident, kidmp_column, kidmp_kid_interface and the
+ * kidmp_mp_gt_driver entries without aerosols.  kidmp_get_rates copies the rates of the handle's LAST step to `rates`:
+ * [36][nz][ncol] for KIDMP_COL_FASTEST, [36][ncol][nz] (KiD's (k,i) order, plane by plane) for KIDMP_K_FASTEST, with ncol
+ * and nz of that step.  It fails when that step wrote no rates into this buffer (kidmp_step_device, a step with a buffer of
+ * kidmp_set_rates_buffer, a failed step), before the first step after kidmp_enable_rates or kidmp_state_alloc, and after
+ * kidmp_enable_rates(h, 0).  The aerosol-aware steps refuse to run while rates are kept or a buffer is set.
+ * A multi-device handle returns KIDMP_K_FASTEST only, laid out by its last stepping call: [36][ncol][nz] of that call's columns,
+ * whether it cut them over the devices or ran on the first device alone (kidmp_column, the WRF tiles, kidmp_kid_interface
+ * with nx below the device count). */
 int kidmp_enable_rates(kidmp_handle* h, int on);
 int kidmp_get_rates(kidmp_handle* h, int layout, float* rates);
 

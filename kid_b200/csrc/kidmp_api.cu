@@ -90,6 +90,7 @@ struct kidmp_handle {
   float* d_set_nc = nullptr; size_t set_nc_floats = 0;   // per-column set_Nc of kidmp_step_nc on the resident state
   float* d_rates = nullptr;                               // caller's device buffer (kidmp_set_rates_buffer) ...
   bool rates_on = false; float* d_rates_own = nullptr;    // ... or the handle's own, [36][nz][ncol] of the resident state (kidmp_enable_rates)
+  bool rates_valid = false;                               // the last step of this handle wrote d_rates_own (kidmp_get_rates refuses otherwise)
   float* d_kid = nullptr; size_t kid_floats = 0;   // staging of the KiD (k,i) arrays
   float* h_kid = nullptr; size_t h_kid_floats = 0; // pinned host twin of it
   float* d_pipe = nullptr; size_t pipe_floats = 0; int pipe_nz = 0; float* d_pipe_dz = nullptr;   // chunk pipeline of kidmp_step
@@ -358,9 +359,12 @@ void launch_cells(kidmp_handle* h, const StepArgs& a, int nsm, cudaStream_t s, c
 // stream (the work buffers are sized for one launch: 29 hand-off planes would otherwise grow with the domain).  Columns are
 // independent, so the chunking changes no result.
 int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
+  // (a step that does not fill the handle's own rate buffer leaves rates of an earlier step there: kidmp_get_rates refuses them)
+  h->rates_valid = false;
   if (a0.nz < 2 || a0.nz > 256) return fail(h, "nz=%d outside [2,256]", a0.nz);
   if (a0.ncol < 1) return fail(h, "ncol=%ld", a0.ncol);
   if (!(a0.dt > 0.f)) return fail(h, "dt must be positive");
+  const bool own_rates = a0.rates && a0.rates == h->d_rates_own;
   const long chunk = h->chunk_cols;
   const long cap = a0.ncol < chunk ? a0.ncol : chunk;
   const long nchunks = (a0.ncol + chunk - 1) / chunk;
@@ -391,6 +395,7 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
     h->timing_valid = false;
     CK(h, cudaEventRecord(h->ev_done, s));
     h->last_on_own_stream = (s == h->stream);
+    h->rates_valid = own_rates;
     return 0;
   }
   bool capturing = false;
@@ -507,12 +512,13 @@ int launch_step(kidmp_handle* h, const StepArgs& a0, cudaStream_t s) {
   CK(h, cudaGetLastError());
   CK(h, cudaEventRecord(h->ev_done, s));
   h->last_on_own_stream = (s == h->stream);
+  h->rates_valid = own_rates;
   return 0;
 }
 
 void free_state(kidmp_handle* h) {
   if (h->d_rates_own) cudaFree(h->d_rates_own);
-  h->d_rates_own = nullptr;
+  h->d_rates_own = nullptr; h->rates_valid = false;
   if (h->d_state) cudaFree(h->d_state);
   if (h->d_dz) cudaFree(h->d_dz);
   if (h->d_ppt) cudaFree(h->d_ppt);
@@ -532,10 +538,13 @@ StepArgs resident_args(kidmp_handle* h, float dt) {
   return a;
 }
 
-// host <-> device copy of one field with layout conversion
-int put_field(kidmp_handle* h, int layout, const float* src, float* dst) {
+// host <-> device copy of one field with layout conversion.  hld: row stride (columns) of a KIDMP_COL_FASTEST host array, which
+// may hold more columns than the resident state (a multi-device handle gives each device a column range of the caller's arrays)
+int put_field(kidmp_handle* h, int layout, const float* src, float* dst, long hld) {
   const size_t bytes = (size_t)h->ncol * h->nz * 4;
-  if (layout == KIDMP_COL_FASTEST || h->ncol == 1) {
+  if (layout == KIDMP_COL_FASTEST && hld != h->ncol) {
+    CK(h, cudaMemcpy2DAsync(dst, (size_t)h->ncol * 4, src, (size_t)hld * 4, (size_t)h->ncol * 4, h->nz, cudaMemcpyHostToDevice, h->stream));
+  } else if (layout == KIDMP_COL_FASTEST || h->ncol == 1) {
     CK(h, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, h->stream));
   } else {
     CK(h, cudaMemcpyAsync(h->d_stage, src, bytes, cudaMemcpyHostToDevice, h->stream));
@@ -545,9 +554,11 @@ int put_field(kidmp_handle* h, int layout, const float* src, float* dst) {
   }
   return 0;
 }
-int get_field(kidmp_handle* h, int layout, const float* src, float* dst) {
+int get_field(kidmp_handle* h, int layout, const float* src, float* dst, long hld) {
   const size_t bytes = (size_t)h->ncol * h->nz * 4;
-  if (layout == KIDMP_COL_FASTEST || h->ncol == 1) {
+  if (layout == KIDMP_COL_FASTEST && hld != h->ncol) {
+    CK(h, cudaMemcpy2DAsync(dst, (size_t)hld * 4, src, (size_t)h->ncol * 4, (size_t)h->ncol * 4, h->nz, cudaMemcpyDeviceToHost, h->stream));
+  } else if (layout == KIDMP_COL_FASTEST || h->ncol == 1) {
     CK(h, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->stream));
   } else {
     dim3 g((unsigned)((h->ncol + 31) / 32), (unsigned)((h->nz + 31) / 32)), b(32, 8);
@@ -573,7 +584,7 @@ extern "C" {
 static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* const fields[KIDMP_NFIELDS], const float* p,
                           const float* dz, const float* set_nc, float* ppt, long hld);
 static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS], const float* p,
-                     const float* dz, const float* set_nc, float* ppt);
+                     const float* dz, const float* set_nc, float* ppt, long hld);
 }
 struct MultiCtx {
   std::vector<kidmp_handle*> dev;
@@ -587,6 +598,10 @@ struct MultiCtx {
   const char* (*GetErrorString)(int) = nullptr;
   std::vector<double*> d_red;                        // [8] per device: the sums being reduced
   long ncol = 0; int nz = 0;                         // resident state: columns of the whole domain
+  // The last call that stepped: its columns, cut into ranges over devices [0, last_ndev) (0: none, or it failed).  The first-
+  // device entries (kidmp_column, the WRF tiles, kidmp_kid_interface with nx < ndev) step one range on device 0; kidmp_get_rates
+  // lays out the devices' rates by this.
+  long last_ncol = 0; int last_ndev = 0;
 };
 namespace {
 void shard(long ncol, int d, int n, long& c0, long& c1) { c0 = ncol * d / n; c1 = ncol * (d + 1) / n; }
@@ -611,7 +626,8 @@ int multi_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* 
   const int n = (int)m->dev.size();
   for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "step: field %d is null", q);
   if (ncol < 1 || nz < 2 || nz > 256 || !(dt > 0.f)) return fail(h, "step: ncol=%ld nz=%d dt=%g", ncol, nz, (double)dt);
-  return on_all(h, [&](int d) -> int {
+  m->last_ndev = 0;
+  const int rc = on_all(h, [&](int d) -> int {
     kidmp_handle* c = m->dev[d];
     long c0, c1;
     shard(ncol, d, n, c0, c1);
@@ -620,22 +636,29 @@ int multi_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* 
     float* f[KIDMP_NFIELDS];
     if (layout == KIDMP_COL_FASTEST) {                // a column range of [nz][ncol] arrays: pitched copies
       for (int q = 0; q < KIDMP_NFIELDS; ++q) f[q] = fields[q] + c0;
-      return step_pipelined(c, c1 - c0, nz, dt, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, ppt ? ppt + c0 : nullptr, ncol);
+      // (with rates kept the range goes through the device's resident state, which holds its rate buffer)
+      if (!c->rates_on)
+        return step_pipelined(c, c1 - c0, nz, dt, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, ppt ? ppt + c0 : nullptr, ncol);
+      return step_host(c, c1 - c0, nz, dt, layout, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, ppt ? ppt + c0 : nullptr, ncol);
     }
     for (int q = 0; q < KIDMP_NFIELDS; ++q) f[q] = fields[q] + (size_t)c0 * nz;   // KiD's (k,i) arrays: a range of columns is contiguous
     std::vector<float> pp(ppt ? (size_t)(c1 - c0) * 4 : 0);
-    if (step_host(c, c1 - c0, nz, dt, layout, f, p + (size_t)c0 * nz, dz, set_nc ? set_nc + c0 : nullptr, ppt ? pp.data() : nullptr))
+    if (step_host(c, c1 - c0, nz, dt, layout, f, p + (size_t)c0 * nz, dz, set_nc ? set_nc + c0 : nullptr, ppt ? pp.data() : nullptr,
+                  c1 - c0))
       return 1;
     if (ppt) for (int q = 0; q < 4; ++q) memcpy(ppt + (size_t)q * ncol + c0, pp.data() + (size_t)q * (c1 - c0), (size_t)(c1 - c0) * 4);
     return 0;
   });
+  if (!rc) { m->last_ncol = ncol; m->last_ndev = n; }
+  return rc;
 }
 
 int multi_kid_interface(kidmp_handle* h, const kidmp_kid_columns* k, float dt, float p0, float r_on_cp) {
   MultiCtx* m = h->multi;
   const int n = (int)m->dev.size();
   if (!k->ppt) return fail(h, "kid_interface: null array");
-  return on_all(h, [&](int d) -> int {
+  m->last_ndev = 0;
+  const int rc = on_all(h, [&](int d) -> int {
     long c0, c1;
     shard(k->nx, d, n, c0, c1);
     if (c1 <= c0) return 0;
@@ -657,6 +680,8 @@ int multi_kid_interface(kidmp_handle* h, const kidmp_kid_columns* k, float dt, f
     for (int q = 0; q < 4; ++q) memcpy(k->ppt + (size_t)q * k->nx + c0, pp.data() + (size_t)q * (c1 - c0), (size_t)(c1 - c0) * 4);
     return 0;
   });
+  if (!rc) { m->last_ncol = k->nx; m->last_ndev = n; }
+  return rc;
 }
 
 int multi_diag(kidmp_handle* h, double out[KIDMP_NDIAG]) {
@@ -740,12 +765,14 @@ int multi_state_alloc(kidmp_handle* h, long ncol, int nz) {
   MultiCtx* m = h->multi;
   const int n = (int)m->dev.size();
   if (ncol < n) return fail(h, "state_alloc: %ld columns over %d devices", ncol, n);
+  m->last_ndev = 0;
   for (int d = 0; d < n; ++d) {
     long c0, c1;
     shard(ncol, d, n, c0, c1);
     if (kidmp_state_alloc(m->dev[d], c1 - c0, nz)) return fail(h, "device %d: %s", m->dev[d]->device, m->dev[d]->err.c_str());
   }
   m->ncol = ncol; m->nz = nz;
+  m->last_ncol = ncol; m->last_ndev = n;              // (kidmp_step_resident steps these ranges)
   return 0;
 }
 int multi_copy(kidmp_handle* h, int layout, float* const fields[KIDMP_NFIELDS], const float* p, const float* dz, float* ppt, bool up) {
@@ -1081,6 +1108,7 @@ int kidmp_state_alloc(kidmp_handle* h, long ncol, int nz) {
   if (h->multi) return multi_state_alloc(h, ncol, nz);
   if (ncol < 1 || nz < 2 || nz > 256) return fail(h, "state_alloc: ncol=%ld nz=%d", ncol, nz);
   DevGuard guard_(h->device);
+  h->rates_valid = false;
   if (h->ncol == ncol && h->nz == nz && h->d_state) return 0;
   free_state(h);
   const size_t n = (size_t)ncol * nz;
@@ -1102,6 +1130,7 @@ int kidmp_enable_rates(kidmp_handle* h, int on) {
   }
   DevGuard guard_(h->device);
   h->rates_on = on != 0;
+  h->rates_valid = false;                               // (a buffer made here holds nothing until the next step fills it)
   if (!h->rates_on && h->d_rates_own) { CK(h, cudaEventSynchronize(h->ev_done)); cudaFree(h->d_rates_own); h->d_rates_own = nullptr; }
   if (h->rates_on && !h->d_rates_own && h->d_state)
     CK(h, cudaMalloc((void**)&h->d_rates_own, (size_t)h->ncol * h->nz * KIDMP_NRATES * 4));
@@ -1113,21 +1142,24 @@ int kidmp_get_rates(kidmp_handle* h, int layout, float* rates) {
   if (h->multi) {
     MultiCtx* m = h->multi;
     if (layout != KIDMP_K_FASTEST) return fail(h, "get_rates: a multi-device handle returns KIDMP_K_FASTEST rates");
-    const int n = (int)m->dev.size();
-    for (int d = 0; d < n; ++d) {
+    if (!m->last_ndev) return fail(h, "get_rates: kidmp_enable_rates and a step first");
+    // the devices that took part in the last stepping call, each its range of that call's columns
+    const long total = m->last_ncol;
+    for (int d = 0; d < m->last_ndev; ++d) {
       kidmp_handle* c = m->dev[d];
-      if (!c->d_rates_own) return fail(h, "get_rates: kidmp_enable_rates and a step first");
       long c0, c1;
-      shard(m->ncol ? m->ncol : c->ncol, d, n, c0, c1);
+      shard(total, d, m->last_ndev, c0, c1);
+      if (c1 <= c0) continue;
+      if (c->ncol != c1 - c0) return fail(h, "get_rates: device %d holds %ld columns, not the %ld of the last step", c->device, c->ncol, c1 - c0);
       std::vector<float> part((size_t)KIDMP_NRATES * c->ncol * c->nz);
-      if (kidmp_get_rates(c, layout, part.data())) return fail(h, "%s", c->err.c_str());
-      const long total = m->ncol ? m->ncol : c->ncol;
+      if (kidmp_get_rates(c, layout, part.data())) return fail(h, "device %d: %s", c->device, c->err.c_str());
       for (int r = 0; r < KIDMP_NRATES; ++r)
         memcpy(rates + ((size_t)r * total + c0) * c->nz, part.data() + (size_t)r * c->ncol * c->nz, (size_t)c->ncol * c->nz * 4);
     }
     return 0;
   }
-  if (!h->d_rates_own || !h->d_state) return fail(h, "get_rates: kidmp_enable_rates and a step on the resident state first");
+  if (!h->d_rates_own || !h->d_state || !h->rates_valid)
+    return fail(h, "get_rates: the last step of this handle wrote no rates (kidmp_enable_rates, then a step on the resident state)");
   DevGuard guard_(h->device);
   const size_t n = (size_t)h->ncol * h->nz;
   CK(h, cudaStreamWaitEvent(h->stream, h->ev_done, 0));
@@ -1146,24 +1178,43 @@ int kidmp_get_rates(kidmp_handle* h, int layout, float* rates) {
   return 0;
 }
 
+// kidmp_upload / kidmp_download of a single-device handle; hld: see put_field
+static int upload_host(kidmp_handle* h, int layout, const float* const fields[KIDMP_NFIELDS], const float* p, const float* dz, long hld) {
+  if (!h->d_state) return fail(h, "upload before state_alloc");
+  if (!fields || !p || !dz) return fail(h, "upload: null pointer");
+  DevGuard guard_(h->device);
+  for (int q = 0; q < KIDMP_NFIELDS; ++q) {
+    if (!fields[q]) return fail(h, "upload: field %d is null", q);
+    if (put_field(h, layout, fields[q], field_ptr(h, q), hld)) return 1;
+    if (layout != KIDMP_COL_FASTEST && h->ncol > 1) CK(h, cudaStreamSynchronize(h->stream));
+  }
+  if (put_field(h, layout, p, field_ptr(h, KIDMP_NFIELDS), hld)) return 1;
+  CK(h, cudaMemcpyAsync(h->d_dz, dz, (size_t)h->nz * 4, cudaMemcpyHostToDevice, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));
+  return 0;
+}
+static int download_host(kidmp_handle* h, int layout, float* const fields[KIDMP_NFIELDS], float* ppt, long hld) {
+  if (!h->d_state) return fail(h, "download before state_alloc");
+  DevGuard guard_(h->device);
+  if (fields)
+    for (int q = 0; q < KIDMP_NFIELDS; ++q)
+      if (fields[q] && get_field(h, layout, field_ptr(h, q), fields[q], hld)) return 1;
+  if (ppt && layout == KIDMP_COL_FASTEST && hld != h->ncol)
+    CK(h, cudaMemcpy2DAsync(ppt, (size_t)hld * 4, h->d_ppt, (size_t)h->ncol * 4, (size_t)h->ncol * 4, 4, cudaMemcpyDeviceToHost, h->stream));
+  else if (ppt)
+    CK(h, cudaMemcpyAsync(ppt, h->d_ppt, (size_t)h->ncol * 16, cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
 int kidmp_upload(kidmp_handle* h, int layout, const float* const fields[KIDMP_NFIELDS], const float* p, const float* dz) {
   if (h && h->multi) {
     if (!fields || !p || !dz) return fail(h, "upload: null pointer");
     for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "upload: field %d is null", q);
     return multi_copy(h, layout, const_cast<float* const*>(fields), p, dz, nullptr, true);
   }
-  if (!h || !h->d_state) return h ? fail(h, "upload before state_alloc") : 1;
-  if (!fields || !p || !dz) return fail(h, "upload: null pointer");
-  DevGuard guard_(h->device);
-  for (int q = 0; q < KIDMP_NFIELDS; ++q) {
-    if (!fields[q]) return fail(h, "upload: field %d is null", q);
-    if (put_field(h, layout, fields[q], field_ptr(h, q))) return 1;
-    if (layout != KIDMP_COL_FASTEST && h->ncol > 1) CK(h, cudaStreamSynchronize(h->stream));
-  }
-  if (put_field(h, layout, p, field_ptr(h, KIDMP_NFIELDS))) return 1;
-  CK(h, cudaMemcpyAsync(h->d_dz, dz, (size_t)h->nz * 4, cudaMemcpyHostToDevice, h->stream));
-  CK(h, cudaStreamSynchronize(h->stream));
-  return 0;
+  if (!h) return 1;
+  return upload_host(h, layout, fields, p, dz, h->ncol);
 }
 
 int kidmp_step_resident(kidmp_handle* h, float dt) {
@@ -1199,14 +1250,8 @@ static int check_set_nc2d(kidmp_handle* h, const char* who, const float* v, cons
 
 int kidmp_download(kidmp_handle* h, int layout, float* const fields[KIDMP_NFIELDS], float* ppt) {
   if (h && h->multi) return multi_copy(h, layout, fields, nullptr, nullptr, ppt, false);
-  if (!h || !h->d_state) return h ? fail(h, "download before state_alloc") : 1;
-  DevGuard guard_(h->device);
-  if (fields)
-    for (int q = 0; q < KIDMP_NFIELDS; ++q)
-      if (fields[q] && get_field(h, layout, field_ptr(h, q), fields[q])) return 1;
-  if (ppt) CK(h, cudaMemcpyAsync(ppt, h->d_ppt, (size_t)h->ncol * 16, cudaMemcpyDeviceToHost, h->stream));
-  CK(h, cudaStreamSynchronize(h->stream));
-  return 0;
+  if (!h) return 1;
+  return download_host(h, layout, fields, ppt, h->ncol);
 }
 
 // Large column-fastest domains: the columns are cut into chunks that flow through three streams
@@ -1323,20 +1368,22 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
   return 0;
 }
 
-// kidmp_step and kidmp_step_nc; set_nc (host, [ncol], checked by the caller) or NULL
+// kidmp_step and kidmp_step_nc; set_nc (host, [ncol], checked by the caller) or NULL.  hld: row stride (columns) of
+// KIDMP_COL_FASTEST host arrays and ppt, ncol unless a multi-device handle steps a column range of them on this device.
 static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
-                     const float* p, const float* dz, const float* set_nc, float* ppt) {
+                     const float* p, const float* dz, const float* set_nc, float* ppt, long hld) {
   if (ncol == 0) return 0;                               // `do i = 1, nx` with nx = 0 (I:54): nothing to do, nothing touched
   if (!fields || !p || !dz) return fail(h, "step: null pointer");
   if (h->multi) return multi_step(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ppt);
-  // (with a process-rate buffer set the whole domain goes through the resident path: the buffer is [36][nz][ncol] of the domain)
-  if (layout == KIDMP_COL_FASTEST && ncol >= 2 * h->pipe_chunk && nz >= 2 && nz <= 256 && dt > 0.f && !h->d_rates) {
+  // (with a process-rate buffer set or the handle's own kept, the whole domain goes through the resident path: the rates are
+  // [36][nz][ncol] of the domain)
+  if (layout == KIDMP_COL_FASTEST && ncol >= 2 * h->pipe_chunk && nz >= 2 && nz <= 256 && dt > 0.f && !h->d_rates && !h->rates_on) {
     for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "step: field %d is null", q);
     DevGuard guard_(h->device);
-    return step_pipelined(h, ncol, nz, dt, fields, p, dz, set_nc, ppt, ncol);
+    return step_pipelined(h, ncol, nz, dt, fields, p, dz, set_nc, ppt, hld);
   }
   if (kidmp_state_alloc(h, ncol, nz)) return 1;
-  if (kidmp_upload(h, layout, fields, p, dz)) return 1;
+  if (upload_host(h, layout, fields, p, dz, hld)) return 1;
   if (!set_nc) {
     if (kidmp_step_resident(h, dt)) return 1;
   } else {
@@ -1350,26 +1397,32 @@ static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, f
     if (launch_step(h, a, h->stream)) return 1;
     CK(h, cudaEventRecord(h->ev1, h->stream));
   }
-  return kidmp_download(h, layout, fields, ppt);
+  return download_host(h, layout, fields, ppt, hld);
 }
 
 int kidmp_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
                const float* p, const float* dz, float* ppt) {
   if (!h) return 1;
-  return step_host(h, ncol, nz, dt, layout, fields, p, dz, nullptr, ppt);
+  return step_host(h, ncol, nz, dt, layout, fields, p, dz, nullptr, ppt, ncol);
 }
 
 int kidmp_step_nc(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
                   const float* p, const float* dz, const float* set_nc, float* ppt) {
   if (!h) return 1;
   if (set_nc && ncol > 0 && check_set_nc(h, "step_nc", set_nc, ncol)) return 1;
-  return step_host(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ppt);
+  return step_host(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ppt, ncol);
 }
 
 int kidmp_column(kidmp_handle* h, int nz, float dt, float* qv, float* qc, float* qi, float* qr, float* qs, float* qg,
                  float* ni, float* nr, float* t, const float* p, const float* dz, float* ppt4) {
   if (!h) return 1;
-  if (h->multi) return kidmp_column(h->multi->dev[0], nz, dt, qv, qc, qi, qr, qs, qg, ni, nr, t, p, dz, ppt4) ? fail(h, "%s", h->multi->dev[0]->err.c_str()) : 0;
+  if (h->multi) {                                       // one column, the first device
+    MultiCtx* m = h->multi;
+    m->last_ndev = 0;
+    if (kidmp_column(m->dev[0], nz, dt, qv, qc, qi, qr, qs, qg, ni, nr, t, p, dz, ppt4)) return fail(h, "%s", m->dev[0]->err.c_str());
+    m->last_ncol = 1; m->last_ndev = 1;
+    return 0;
+  }
   if (!ppt4) return fail(h, "column: ppt4 is null");
   float* f[KIDMP_NFIELDS] = {qv, qc, qi, qr, qs, qg, ni, nr, t};
   float inc[4] = {0.f, 0.f, 0.f, 0.f};
@@ -1601,7 +1654,13 @@ static void tile_rows(float* tile, float* mem, const kidmp_wrf_tile& t, long ni_
 // kidmp_mp_gt_driver_tile and kidmp_mp_gt_driver_tile_nc (set_nc2d: host (i,j) array of the memory box, or NULL; never with ae)
 static int wrf_tile_host(kidmp_handle* h, const kidmp_wrf_fields* w, const kidmp_wrf_tile* t, const kidmp_wrf_aerosols* ae,
                          const float* set_nc2d, float dt_in) {
-  if (h->multi) return wrf_tile_host(h->multi->dev[0], w, t, ae, set_nc2d, dt_in) ? fail(h, "%s", h->multi->dev[0]->err.c_str()) : 0;   // one tile, one device
+  if (h->multi) {                                       // one tile, the first device
+    MultiCtx* m = h->multi;
+    m->last_ndev = 0;
+    if (wrf_tile_host(m->dev[0], w, t, ae, set_nc2d, dt_in)) return fail(h, "%s", m->dev[0]->err.c_str());
+    m->last_ncol = (long)t->ni * t->nj; m->last_ndev = 1;
+    return 0;
+  }
   const char* who = set_nc2d ? "mp_gt_driver_tile_nc" : ae ? "mp_gt_driver_aero" : "mp_gt_driver";
   if (wrf_check(h, who, w, t, ae, dt_in)) return 1;
   if (set_nc2d && check_set_nc2d(h, who, set_nc2d, t, w->ni)) return 1;
@@ -1826,7 +1885,13 @@ int kidmp_kid_interface(kidmp_handle* h, const kidmp_kid_columns* c, float dt, f
   if (!c) return fail(h, "kid_interface: null argument");
   if (c->nx == 0) return 0;                              // an empty domain is not an error (I:54)
   if (h->multi && c->nx >= (long)h->multi->dev.size()) return multi_kid_interface(h, c, dt, p0, r_on_cp);
-  if (h->multi) return kidmp_kid_interface(h->multi->dev[0], c, dt, p0, r_on_cp) ? fail(h, "%s", h->multi->dev[0]->err.c_str()) : 0;
+  if (h->multi) {                                       // fewer columns than devices: the first device
+    MultiCtx* m = h->multi;
+    m->last_ndev = 0;
+    if (kidmp_kid_interface(m->dev[0], c, dt, p0, r_on_cp)) return fail(h, "%s", m->dev[0]->err.c_str());
+    m->last_ncol = c->nx; m->last_ndev = 1;
+    return 0;
+  }
   if (!c->theta || !c->dtheta_adv || !c->dtheta_div || !c->exner || !c->qv || !c->dqv_adv || !c->dqv_div || !c->dz ||
       !c->dtheta_mphys || !c->dqv_mphys || !c->ppt)
     return fail(h, "kid_interface: null array");
