@@ -4,9 +4,13 @@
 // (profiles/r01): ~40-50 instructions each with no table.  These versions use the classic
 // reduce-to-a-table-node scheme (as in glibc / ARM optimized-routines; restated here from the
 // published method, not copied): 128-entry tables, degree-5 / degree-7 polynomials on |r| < 2^-7,
-// ~16 and ~24 instructions, error below 1 ulp of f64 (tests/test_fastmath.py checks 4e6 points
-// against libm).  They are only ever used under an f32 rounding or inside f64 rates that are
-// narrowed to f32 tendencies, so this is far inside the parity budget (DESIGN.md section 4).
+// ~16 and ~24 instructions.  Accuracy (tests/test_device_math.py, against long double / mpmath):
+//   exp   < 1 ulp of f64 for |x| < 704;
+//   log   < 1.5 ulp where |log x| > 0.1 (1.42 measured, 1.10 below |log x| = 700); near 1 the error is
+//         absolute, < 1.5e-17 where |log x| <= 0.1 (up to ~1e4 ulps of a result next to 0);
+//   exp(y*log(x))  < 3 (1 + |y log x|) ulp, plus |y| * 1.5e-17 relative where |log x| <= 0.1.
+// They are only ever used under an f32 rounding or inside f64 rates that are narrowed to f32
+// tendencies, so this is far inside the parity budget (DESIGN.md section 4).
 //
 // Arguments outside the fast range (x <= 0, inf, nan, subnormal for log; |x| >= 704 or nan for exp)
 // take the library function.

@@ -7,8 +7,9 @@
 //     + - * / sqrt rounds exactly like the Fortran expression it restates;
 //   * evaluate every transcendental whose result is stored as f32 in f64 and round once, which
 //     is within one f32 ulp of any faithful libm (gfortran calls glibc powf/expf/logf/log10f);
-//   * keep f64 where the reference has DOUBLE PRECISION, with x**y as exp(y*log(x)) (relative
-//     error ~1e-15, invisible once the rates are narrowed to the f32 tendencies) and the
+//   * keep f64 where the reference has DOUBLE PRECISION, with x**y as exp(y*log(x)) (error below
+//     3 (1 + |y log x|) ulp, see kidmp_fastmath.h; invisible once the rates are narrowed to the f32
+//     tendencies) and the
 //     PARAMETER exponents of the scheme (mu_r = mu_g = mu_i = 0, bm_r = bm_g = bm_i = 3,
 //     bv_r = bv_i = 1, M:56-111) strength-reduced to products and square roots.
 #pragma once

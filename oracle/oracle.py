@@ -73,6 +73,16 @@ def lib():
         L.kor_mp_gt_driver.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float] + [_fp] * 22
         L.kor_decade_index.restype = C.c_int
         L.kor_decade_index.argtypes = [C.c_float, C.c_int, C.c_int]
+        L.kor_decade_index_d.restype = C.c_int
+        L.kor_decade_index_d.argtypes = [C.c_double, C.c_int, C.c_int]
+        _ip = C.POINTER(C.c_int)
+        for name, args in (("kor_rslf_array", [_fp] * 3), ("kor_rsif_array", [_fp] * 3),
+                           ("kor_decade_index_array", [_fp, C.c_int, C.c_int, _ip]),
+                           ("kor_decade_index_d_array", [_dp, C.c_int, C.c_int, _ip]),
+                           ("kor_eff_aero_array", [_fp] * 5 + [C.c_char, _fp]), ("kor_ice_demott_array", [_fp] * 4),
+                           ("kor_ice_koop_array", [_fp] * 6), ("kor_activ_ncloud_array", [_fp] * 4)):
+            getattr(L, name).restype = None
+            getattr(L, name).argtypes = args + [C.c_long]
         _lib = L
     return _lib
 
@@ -286,3 +296,56 @@ def rslf(p, t):
 
 def rsif(p, t):
     return float(lib().kor_rsif(p, t))
+
+
+def decade_index(x, n2, ntb):
+    """M:1762-1774: the table index of an f32 value (decade offset n2, ntb nodes)."""
+    return int(lib().kor_decade_index(x, n2, ntb))
+
+
+def decade_index_d(x, n2, ntb):
+    """M:1824-1833: the same for an f64 value (the rain and graupel intercepts)."""
+    return int(lib().kor_decade_index_d(x, n2, ntb))
+
+
+def _array_call(fn, inputs, dtype, out_dtype, *scalars):
+    """fn(in_0, ..., *scalars, out, n) over 1-D arrays broadcast to one length; returns out."""
+    arrs = [np.ascontiguousarray(a, dtype) for a in np.broadcast_arrays(*[np.asarray(a) for a in inputs])]
+    n = arrs[0].size
+    out = np.empty(n, out_dtype)
+    ptr = _dp if dtype == np.float64 else _fp
+    optr = C.POINTER(C.c_int) if out_dtype == np.int32 else _fp
+    fn(*[a.ravel().ctypes.data_as(ptr) for a in arrs], *scalars, out.ctypes.data_as(optr), n)
+    return out
+
+
+def rslf_array(p, t):
+    return _array_call(lib().kor_rslf_array, (p, t), np.float32, np.float32)
+
+
+def rsif_array(p, t):
+    return _array_call(lib().kor_rsif_array, (p, t), np.float32, np.float32)
+
+
+def decade_index_array(x, n2, ntb):
+    return _array_call(lib().kor_decade_index_array, (x,), np.float32, np.int32, int(n2), int(ntb))
+
+
+def decade_index_d_array(x, n2, ntb):
+    return _array_call(lib().kor_decade_index_d_array, (x,), np.float64, np.int32, int(n2), int(ntb))
+
+
+def eff_aero_array(D, Da, visc, rhoa, temp, species):
+    return _array_call(lib().kor_eff_aero_array, (D, Da, visc, rhoa, temp), np.float32, np.float32, species.encode())
+
+
+def ice_demott_array(tempc, rho, nifa):
+    return _array_call(lib().kor_ice_demott_array, (tempc, rho, nifa), np.float32, np.float32)
+
+
+def ice_koop_array(temp, qv, qvs, naero, dt):
+    return _array_call(lib().kor_ice_koop_array, (temp, qv, qvs, naero, dt), np.float32, np.float32)
+
+
+def activ_ncloud_array(Tt, Ww, NCCN):
+    return _array_call(lib().kor_activ_ncloud_array, (Tt, Ww, NCCN), np.float32, np.float32)

@@ -85,6 +85,19 @@ float kor_gammln(float x);
 float kor_wgamma(float x);
 float kor_gammp(float a, float x);
 int   kor_decade_index(float x, int n2, int ntb);   // M:1762-1774 pattern
+int   kor_decade_index_d(double x, int n2, int ntb);   // M:1824-1833 (f64 argument)
+
+// array forms of the helpers above (out[i] = f(x[i], ...), i < n): one call for a sweep of millions of points
+void kor_rslf_array(const float* p, const float* t, float* out, long n);
+void kor_rsif_array(const float* p, const float* t, float* out, long n);
+void kor_decade_index_array(const float* x, int n2, int ntb, int* out, long n);
+void kor_decade_index_d_array(const double* x, int n2, int ntb, int* out, long n);
+void kor_eff_aero_array(const float* D, const float* Da, const float* visc, const float* rhoa, const float* temp,
+                        char species, float* out, long n);
+void kor_ice_demott_array(const float* tempc, const float* rho, const float* nifa, float* out, long n);
+void kor_ice_koop_array(const float* temp, const float* qv, const float* qvs, const float* naero, const float* dt,
+                        float* out, long n);
+void kor_activ_ncloud_array(const float* Tt, const float* Ww, const float* NCCN, float* out, long n);
 
 #ifdef __cplusplus
 }
