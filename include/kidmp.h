@@ -88,8 +88,8 @@ int kidmp_step(kidmp_handle* h, long ncol, int nz, float dt, int layout,
                float* const fields[KIDMP_NFIELDS], const float* p, const float* dz, float* ppt);
 
 /* device-resident state: upload once, step many times, download when needed.  One resident state per handle: the entry
- * points that take HOST arrays of another size (kidmp_step below the pipeline threshold, kidmp_column, kidmp_kid_interface,
- * kidmp_mp_gt_driver) re-allocate it.  Calls on one handle are serialised by the caller; a step enqueued on a caller's
+ * points that take HOST arrays of another size (kidmp_step and kidmp_step_aero below the pipeline threshold, kidmp_column,
+ * kidmp_kid_interface, kidmp_mp_gt_driver) re-allocate it.  Calls on one handle are serialised by the caller; a step enqueued on a caller's
  * stream (kidmp_step_device) is ordered against kidmp_diag and the next step of the same handle by an event. */
 int kidmp_state_alloc(kidmp_handle* h, long ncol, int nz);
 int kidmp_upload(kidmp_handle* h, int layout, const float* const fields[KIDMP_NFIELDS],
@@ -133,6 +133,18 @@ int kidmp_step_device_nc(kidmp_handle* h, long ncol, int nz, float dt, float* co
 int kidmp_step_device_aero(kidmp_handle* h, long ncol, int nz, float dt, float* const d_fields[KIDMP_NFIELDS], float* d_nc,
                            float* d_nwfa, float* d_nifa, const float* d_p, const float* d_w, const float* d_dz,
                            const float* d_nwfa2d, float* d_ppt, void* stream);
+/* The same aerosol-aware step on HOST arrays, in place: kidmp_step with the aerosol switch on.  nc, nwfa, nifa (INOUT) and w (IN)
+ * are laid out like the fields ([nz][ncol] for KIDMP_COL_FASTEST, (k,i) for KIDMP_K_FASTEST); nwfa2d is [ncol] in both layouts,
+ * or NULL; ppt [4][ncol] is overwritten.  Every column comes out bit for bit as kidmp_step_device_aero makes it from device copies
+ * of the same inputs (the nine fields, nc, nwfa, nifa, ppt), and kidmp_diag counts it the same way.  Every path of kidmp_step:
+ * small domains and KIDMP_K_FASTEST through the resident state, large KIDMP_COL_FASTEST domains through the chunk pipeline (each
+ * chunk carries the four aerosol planes and its slice of nwfa2d), only the changed columns back when the twelve INOUT arrays
+ * are pinned (with nwfa2d the lowest nwfa level comes back for every column: the emission changes it everywhere), multi-device
+ * handles (each device its column range).  A NULL array other than nwfa2d and ppt, nz outside [2, 256], dt <= 0, or process
+ * rates kept or a rate buffer set (on any device of the handle) fail the call before anything is copied or launched, every
+ * array left as it was.  ncol = 0: success, nothing touched. */
+int kidmp_step_aero(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS], float* nc,
+                    float* nwfa, float* nifa, const float* p, const float* w, const float* dz, const float* nwfa2d, float* ppt);
 
 /* optional per-level process-rate buffer (the 36 save_dg rates of M:2963-3120): device buffer
  * [36][nz][ncol] f32, NULL switches it off (default).  Names: kidmp_rate_names(). */
@@ -258,7 +270,8 @@ int kidmp_set_option(kidmp_handle* h, const char* name, int value);
 
 /* Multi-device handles (kidmp_config::ndev > 1).  kidmp_step, kidmp_kid_interface and the resident-state calls cut the
  * host arrays into one contiguous column range per device (columns are independent, I:54: no exchange on the data path) and
- * run the devices side by side; results are bit-identical to a single-device handle, column by column.  kidmp_column and
+ * run the devices side by side; results are bit-identical to a single-device handle, column by column.  So does kidmp_step_aero:
+ * every device builds its own drop-evaporation table on its first aerosol-aware step.  kidmp_column and
  * kidmp_mp_gt_driver[_aero,_tile] run on the first device.  The entry points that take or return DEVICE pointers
  * (kidmp_step_device, kidmp_mp_gt_driver_tile_device, kidmp_set_rates_buffer, kidmp_device_state, kidmp_stream) need a
  * single-device handle.  NCCL (libnccl.so.2, or the file
@@ -269,7 +282,7 @@ int kidmp_num_devices(const kidmp_handle* h);
 long kidmp_gpu_launches(const kidmp_handle* h);         /* kernels launched so far          */
 /* counts of the last launch of the step kernels in the last step (waits for it): 0 cloudy columns, 1 busy
  * cells, 2-5 busy cells of the warm / ice / mixed-without-rain / full cell kernels, 6 columns with sedimentation sub-steps,
- * 7 whether the last kidmp_step returned only the changed columns (pinned host arrays, see kidmp_step) */
+ * 7 whether the last kidmp_step or kidmp_step_aero returned only the changed columns (pinned host arrays, see kidmp_step) */
 int kidmp_step_stats(kidmp_handle* h, long out[8]);
 /* per-kernel device times of the last launch of the step kernels, after kidmp_set_option(h, "timing", 1): in that mode the
  * kernels of a launch run one after the other on one stream with a CUDA event after each group (normally two of them run

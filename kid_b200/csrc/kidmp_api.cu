@@ -580,11 +580,14 @@ int get_field(kidmp_handle* h, int layout, const float* src, float* dst, long hl
 }  // namespace
 #include <dlfcn.h>
 #include <thread>
+// the aerosol arrays of kidmp_step_aero on the host: nc, nwfa, nifa (INOUT) and w (IN) laid out like the fields, nwfa2d [ncol]
+// or NULL.  A pointer to it selects the aerosol-aware step; NULL is the plain scheme.
+struct AeroHost { float* nc; float* nwfa; float* nifa; const float* w; const float* nwfa2d; };
 extern "C" {
 static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* const fields[KIDMP_NFIELDS], const float* p,
-                          const float* dz, const float* set_nc, float* ppt, long hld);
+                          const float* dz, const float* set_nc, const AeroHost* ae, float* ppt, long hld);
 static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS], const float* p,
-                     const float* dz, const float* set_nc, float* ppt, long hld);
+                     const float* dz, const float* set_nc, const AeroHost* ae, float* ppt, long hld);
 }
 struct MultiCtx {
   std::vector<kidmp_handle*> dev;
@@ -621,7 +624,7 @@ template <class F> int on_all(kidmp_handle* h, F fn) {
 }
 
 int multi_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS], const float* p,
-               const float* dz, const float* set_nc, float* ppt) {
+               const float* dz, const float* set_nc, const AeroHost* ae, float* ppt) {
   MultiCtx* m = h->multi;
   const int n = (int)m->dev.size();
   for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "step: field %d is null", q);
@@ -634,16 +637,21 @@ int multi_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* 
     if (c1 <= c0) return 0;
     cudaSetDevice(c->device);
     float* f[KIDMP_NFIELDS];
+    // the aerosol planes of the range are laid out like the fields; nwfa2d is [ncol] in both layouts
+    const size_t o3 = layout == KIDMP_COL_FASTEST ? (size_t)c0 : (size_t)c0 * nz;
+    const AeroHost ar = ae ? AeroHost{ae->nc + o3, ae->nwfa + o3, ae->nifa + o3, ae->w + o3, ae->nwfa2d ? ae->nwfa2d + c0 : nullptr}
+                           : AeroHost{};
+    const AeroHost* const aer = ae ? &ar : nullptr;
     if (layout == KIDMP_COL_FASTEST) {                // a column range of [nz][ncol] arrays: pitched copies
       for (int q = 0; q < KIDMP_NFIELDS; ++q) f[q] = fields[q] + c0;
       // (with rates kept the range goes through the device's resident state, which holds its rate buffer)
       if (!c->rates_on)
-        return step_pipelined(c, c1 - c0, nz, dt, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, ppt ? ppt + c0 : nullptr, ncol);
-      return step_host(c, c1 - c0, nz, dt, layout, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, ppt ? ppt + c0 : nullptr, ncol);
+        return step_pipelined(c, c1 - c0, nz, dt, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, aer, ppt ? ppt + c0 : nullptr, ncol);
+      return step_host(c, c1 - c0, nz, dt, layout, f, p + c0, dz, set_nc ? set_nc + c0 : nullptr, aer, ppt ? ppt + c0 : nullptr, ncol);
     }
     for (int q = 0; q < KIDMP_NFIELDS; ++q) f[q] = fields[q] + (size_t)c0 * nz;   // KiD's (k,i) arrays: a range of columns is contiguous
     std::vector<float> pp(ppt ? (size_t)(c1 - c0) * 4 : 0);
-    if (step_host(c, c1 - c0, nz, dt, layout, f, p + (size_t)c0 * nz, dz, set_nc ? set_nc + c0 : nullptr, ppt ? pp.data() : nullptr,
+    if (step_host(c, c1 - c0, nz, dt, layout, f, p + (size_t)c0 * nz, dz, set_nc ? set_nc + c0 : nullptr, aer, ppt ? pp.data() : nullptr,
                   c1 - c0))
       return 1;
     if (ppt) for (int q = 0; q < 4; ++q) memcpy(ppt + (size_t)q * ncol + c0, pp.data() + (size_t)q * (c1 - c0), (size_t)(c1 - c0) * 4);
@@ -1260,8 +1268,12 @@ int kidmp_download(kidmp_handle* h, int layout, float* const fields[KIDMP_NFIELD
 // `hld`: columns of the caller's host arrays (their row stride): a multi-device handle gives every device a range of columns
 // of the same arrays.
 // `set_nc`: per-column set_Nc of the ncol columns (host, contiguous) or NULL; each chunk takes its slice.
+// `ae`: the aerosol arrays of an aerosol-aware step (row stride hld like the fields; nwfa2d contiguous) or NULL.  Each chunk then
+// carries four more planes in (nc, nwfa, nifa, w) and nwfa2d's slice, gets the surface emission after its step, and returns
+// twelve planes.
+int ensure_wev_table(kidmp_handle* h);
 static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* const fields[KIDMP_NFIELDS],
-                          const float* p, const float* dz, const float* set_nc, float* ppt, long hld) {
+                          const float* p, const float* dz, const float* set_nc, const AeroHost* ae, float* ppt, long hld) {
   // (no larger than a launch chunk: then every pipeline chunk is one launch of launch_step, whose column flags k_scatter_host reads)
   const long chunk = h->pipe_chunk < h->chunk_cols ? h->pipe_chunk : h->chunk_cols;
   const int NB = 3;
@@ -1269,8 +1281,13 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
   // serialise kernels that could run side by side)
   if (!h->copy_in) CK(h, cudaStreamCreateWithFlags(&h->copy_in, cudaStreamNonBlocking));
   if (!h->copy_out) CK(h, cudaStreamCreateWithFlags(&h->copy_out, cudaStreamNonBlocking));
+  if (ae && ensure_wev_table(h)) return 1;
   const size_t cells = (size_t)chunk * nz;
-  const size_t per_buf = cells * (KIDMP_NFIELDS + 1) + (size_t)chunk * 5;   // fields and p, ppt [4][chunk], set_nc [chunk]
+  // fields and p [, nc nwfa nifa w], ppt [4][chunk], set_nc [chunk] [, nwfa2d [chunk]].  The buffer grows when a call needs more
+  // than it holds (an aerosol-aware step after a plain one, or more levels); a plain step after an aerosol-aware one lays its
+  // planes out at the start of the larger buffer.
+  const int nplanes = KIDMP_NFIELDS + 1 + (ae ? 4 : 0);
+  const size_t per_buf = cells * nplanes + (size_t)chunk * (ae ? 6 : 5);
   if (h->pipe_floats < per_buf * NB || h->pipe_nz != nz) {
     if (h->d_pipe) cudaFree(h->d_pipe);
     h->d_pipe = nullptr; h->pipe_floats = 0;
@@ -1294,13 +1311,18 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
   // Pinned output arrays (cudaHostAlloc / cudaHostRegister: what a host that cares about transfer speed uses): only the
   // columns the step changed go back, written by a kernel straight into the host arrays (k_scatter_host); pageable arrays
   // get the whole chunk back with a copy.  KIDMP_ZEROCOPY=0 switches the first path off.
-  HostFields hf{};
+  // The INOUT arrays: the nine fields [, nc nwfa nifa]; on the device plane q < 9 is field q, p sits between them and nc.
+  float* const io[KIDMP_NFIELDS + 3] = {fields[0], fields[1], fields[2], fields[3], fields[4], fields[5], fields[6], fields[7],
+                                        fields[8], ae ? ae->nc : nullptr, ae ? ae->nwfa : nullptr, ae ? ae->nifa : nullptr};
+  const int nio = ae ? KIDMP_NFIELDS + 3 : KIDMP_NFIELDS;
+  HostFieldsAero hf{};
   bool zero_copy = !(getenv("KIDMP_ZEROCOPY") && atoi(getenv("KIDMP_ZEROCOPY")) == 0);
-  for (int q = 0; q < KIDMP_NFIELDS && zero_copy; ++q) {
+  for (int q = 0; q < nio && zero_copy; ++q) {
     cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, fields[q]) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) { zero_copy = false; cudaGetLastError(); }
+    if (cudaPointerGetAttributes(&at, io[q]) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) { zero_copy = false; cudaGetLastError(); }
     else hf.f[q] = (float*)at.devicePointer;
   }
+  const float* const in_ae[4] = {ae ? ae->nc : nullptr, ae ? ae->nwfa : nullptr, ae ? ae->nifa : nullptr, ae ? ae->w : nullptr};
   h->last_zero_copy = zero_copy;
   const size_t hpitch = (size_t)hld * 4, ppitch = (size_t)ncol * 4;
   // KIDMP_PIPE_TRACE=1: device timeline of every chunk (H2D, step kernels, return path) on stderr after the step
@@ -1312,16 +1334,18 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
     const int b = it % NB;
     const long n = (ncol - c0 < chunk) ? (ncol - c0) : chunk;
     float* base = h->d_pipe + per_buf * b;
-    float* d_ppt = base + cells * (KIDMP_NFIELDS + 1);
+    float* d_ppt = base + cells * nplanes;
     float* const d_set_nc = d_ppt + (size_t)chunk * 4;
+    float* const d_nwfa2d = d_set_nc + chunk;
     const size_t dpitch = (size_t)n * 4;
     if (it >= NB) CK(h, cudaStreamWaitEvent(h->copy_in, h->pipe_ev[b][2], 0));     // buffer drained by its D2H
     tmark(h->copy_in);
-    for (int q = 0; q <= KIDMP_NFIELDS; ++q) {
-      const float* src = (q < KIDMP_NFIELDS ? fields[q] : p) + c0;
+    for (int q = 0; q < nplanes; ++q) {
+      const float* src = (q < KIDMP_NFIELDS ? fields[q] : q == KIDMP_NFIELDS ? p : in_ae[q - KIDMP_NFIELDS - 1]) + c0;
       CK(h, cudaMemcpy2DAsync(base + cells * q, dpitch, src, hpitch, dpitch, nz, cudaMemcpyHostToDevice, h->copy_in));
     }
     if (set_nc) CK(h, cudaMemcpyAsync(d_set_nc, set_nc + c0, (size_t)n * 4, cudaMemcpyHostToDevice, h->copy_in));
+    if (ae && ae->nwfa2d) CK(h, cudaMemcpyAsync(d_nwfa2d, ae->nwfa2d + c0, (size_t)n * 4, cudaMemcpyHostToDevice, h->copy_in));
     CK(h, cudaEventRecord(h->pipe_ev[b][0], h->copy_in));
     tmark(h->copy_in);
     CK(h, cudaStreamWaitEvent(h->stream, h->pipe_ev[b][0], 0));
@@ -1331,22 +1355,35 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
     for (int q = 0; q < KIDMP_NFIELDS; ++q) a.f[q] = base + cells * q;
     a.p = base + cells * KIDMP_NFIELDS; a.dz = h->d_pipe_dz; a.ppt = d_ppt;
     if (set_nc) a.set_nc = d_set_nc;
+    if (ae) {
+      float* const d_ae = base + cells * (KIDMP_NFIELDS + 1);
+      a.nc = d_ae; a.nwfa = d_ae + cells; a.nifa = d_ae + 2 * cells; a.w = d_ae + 3 * cells;
+    }
     if (launch_step(h, a, h->stream)) return 1;
+    // what mp_gt_driver does after the call (M:1001), as kidmp_step_device_aero
+    if (ae && ae->nwfa2d) { k_nwfa_surface<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(a.nwfa, d_nwfa2d, n, dt); ++h->launches; }
     tmark(h->stream);
     CK(h, cudaEventRecord(h->pipe_ev[b][1], h->stream));
     CK(h, cudaStreamWaitEvent(h->copy_out, h->pipe_ev[b][1], 0));
     if (zero_copy) {
-      HostFields hc = hf;
-      for (int q = 0; q < KIDMP_NFIELDS; ++q) hc.f[q] += c0;
       StepArgs sa = a;
       sa.colflag = h->ws.d_colflag;                  // (this chunk's flags: it was one launch, and the next chunk's kernels follow on this stream)
-      k_scatter_host<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(sa, hc, hld);
+      if (ae) {
+        HostFieldsAero hc = hf;
+        for (int q = 0; q < nio; ++q) hc.f[q] += c0;
+        k_scatter_host_aero<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(sa, hc, hld, ae->nwfa2d ? 1 : 0);
+      } else {
+        HostFields hc;
+        for (int q = 0; q < KIDMP_NFIELDS; ++q) hc.f[q] = hf.f[q] + c0;
+        k_scatter_host<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(sa, hc, hld);
+      }
       ++h->launches;
       CK(h, cudaEventRecord(h->pipe_ev[b][1], h->stream));
       CK(h, cudaStreamWaitEvent(h->copy_out, h->pipe_ev[b][1], 0));
     } else
-      for (int q = 0; q < KIDMP_NFIELDS; ++q)
-        CK(h, cudaMemcpy2DAsync(fields[q] + c0, hpitch, base + cells * q, dpitch, dpitch, nz, cudaMemcpyDeviceToHost, h->copy_out));
+      for (int q = 0; q < nio; ++q)                  // (device plane q + 1 from nc on: p lies between)
+        CK(h, cudaMemcpy2DAsync(io[q] + c0, hpitch, base + cells * (q < KIDMP_NFIELDS ? q : q + 1), dpitch, dpitch, nz,
+                                cudaMemcpyDeviceToHost, h->copy_out));
     if (ppt) CK(h, cudaMemcpy2DAsync(h->h_ppt + c0, ppitch, d_ppt, dpitch, dpitch, 4, cudaMemcpyDeviceToHost, h->copy_out));
     CK(h, cudaEventRecord(h->pipe_ev[b][2], h->copy_out));
     tmark(h->stream);
@@ -1368,23 +1405,57 @@ static int step_pipelined(kidmp_handle* h, long ncol, int nz, float dt, float* c
   return 0;
 }
 
-// kidmp_step and kidmp_step_nc; set_nc (host, [ncol], checked by the caller) or NULL.  hld: row stride (columns) of
-// KIDMP_COL_FASTEST host arrays and ppt, ncol unless a multi-device handle steps a column range of them on this device.
+// The aerosol-aware step of kidmp_step_aero on the resident state, which the caller has allocated and uploaded: the four aerosol
+// planes (and nwfa2d) into h->d_aero as wrf_kernels lays them out, the step, the surface emission, nc nwfa nifa back.
+static int step_resident_aero(kidmp_handle* h, int layout, float dt, const AeroHost* ae, long hld) {
+  DevGuard guard_(h->device);
+  if (ensure_wev_table(h)) return 1;
+  const size_t n = (size_t)h->ncol * h->nz;
+  if (ensure_dev(h, &h->d_aero, &h->aero_floats, 4 * n + (size_t)h->ncol)) return 1;
+  CK(h, cudaStreamWaitEvent(h->stream, h->ev_done, 0));  // (the planes may still serve a WRF tile on a caller's stream)
+  float* const d = h->d_aero;
+  const float* const in4[4] = {ae->nc, ae->nwfa, ae->nifa, ae->w};
+  for (int q = 0; q < 4; ++q) {
+    if (put_field(h, layout, in4[q], d + n * q, hld)) return 1;
+    if (layout != KIDMP_COL_FASTEST && h->ncol > 1) CK(h, cudaStreamSynchronize(h->stream));   // (d_stage serves the next plane)
+  }
+  if (ae->nwfa2d) CK(h, cudaMemcpyAsync(d + 4 * n, ae->nwfa2d, (size_t)h->ncol * 4, cudaMemcpyHostToDevice, h->stream));
+  StepArgs a = resident_args(h, dt);
+  a.nc = d; a.nwfa = d + n; a.nifa = d + 2 * n; a.w = d + 3 * n;
+  CK(h, cudaEventRecord(h->ev0, h->stream));
+  if (launch_step(h, a, h->stream)) return 1;
+  if (ae->nwfa2d) {                                      // M:1001, as kidmp_step_device_aero
+    k_nwfa_surface<<<(unsigned)((h->ncol + 255) / 256), 256, 0, h->stream>>>(a.nwfa, d + 4 * n, h->ncol, dt);
+    ++h->launches;
+    CK(h, cudaEventRecord(h->ev_done, h->stream));
+  }
+  CK(h, cudaEventRecord(h->ev1, h->stream));
+  float* const out3[3] = {ae->nc, ae->nwfa, ae->nifa};
+  for (int q = 0; q < 3; ++q) if (get_field(h, layout, d + n * q, out3[q], hld)) return 1;
+  h->last_zero_copy = false;
+  return 0;
+}
+
+// kidmp_step, kidmp_step_nc and kidmp_step_aero; set_nc (host, [ncol], checked by the caller) or NULL; ae (checked by the
+// caller, never with set_nc) or NULL.  hld: row stride (columns) of KIDMP_COL_FASTEST host arrays and ppt, ncol unless a
+// multi-device handle steps a column range of them on this device.
 static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
-                     const float* p, const float* dz, const float* set_nc, float* ppt, long hld) {
+                     const float* p, const float* dz, const float* set_nc, const AeroHost* ae, float* ppt, long hld) {
   if (ncol == 0) return 0;                               // `do i = 1, nx` with nx = 0 (I:54): nothing to do, nothing touched
   if (!fields || !p || !dz) return fail(h, "step: null pointer");
-  if (h->multi) return multi_step(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ppt);
+  if (h->multi) return multi_step(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ae, ppt);
   // (with a process-rate buffer set or the handle's own kept, the whole domain goes through the resident path: the rates are
   // [36][nz][ncol] of the domain)
   if (layout == KIDMP_COL_FASTEST && ncol >= 2 * h->pipe_chunk && nz >= 2 && nz <= 256 && dt > 0.f && !h->d_rates && !h->rates_on) {
     for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "step: field %d is null", q);
     DevGuard guard_(h->device);
-    return step_pipelined(h, ncol, nz, dt, fields, p, dz, set_nc, ppt, hld);
+    return step_pipelined(h, ncol, nz, dt, fields, p, dz, set_nc, ae, ppt, hld);
   }
   if (kidmp_state_alloc(h, ncol, nz)) return 1;
   if (upload_host(h, layout, fields, p, dz, hld)) return 1;
-  if (!set_nc) {
+  if (ae) {
+    if (step_resident_aero(h, layout, dt, ae, hld)) return 1;
+  } else if (!set_nc) {
     if (kidmp_step_resident(h, dt)) return 1;
   } else {
     DevGuard guard_(h->device);
@@ -1403,14 +1474,14 @@ static int step_host(kidmp_handle* h, long ncol, int nz, float dt, int layout, f
 int kidmp_step(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
                const float* p, const float* dz, float* ppt) {
   if (!h) return 1;
-  return step_host(h, ncol, nz, dt, layout, fields, p, dz, nullptr, ppt, ncol);
+  return step_host(h, ncol, nz, dt, layout, fields, p, dz, nullptr, nullptr, ppt, ncol);
 }
 
 int kidmp_step_nc(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS],
                   const float* p, const float* dz, const float* set_nc, float* ppt) {
   if (!h) return 1;
   if (set_nc && ncol > 0 && check_set_nc(h, "step_nc", set_nc, ncol)) return 1;
-  return step_host(h, ncol, nz, dt, layout, fields, p, dz, set_nc, ppt, ncol);
+  return step_host(h, ncol, nz, dt, layout, fields, p, dz, set_nc, nullptr, ppt, ncol);
 }
 
 int kidmp_column(kidmp_handle* h, int nz, float dt, float* qv, float* qc, float* qi, float* qr, float* qs, float* qg,
@@ -1515,6 +1586,23 @@ int kidmp_step_device_aero(kidmp_handle* h, long ncol, int nz, float dt, float* 
   if (d_nwfa2d) { k_nwfa_surface<<<(unsigned)((ncol + 255) / 256), 256, 0, s>>>(d_nwfa, d_nwfa2d, ncol, dt); ++h->launches; CK(h, cudaEventRecord(h->ev_done, s)); }
   if (s == h->stream) CK(h, cudaEventRecord(h->ev1, s));
   return 0;
+}
+
+int kidmp_step_aero(kidmp_handle* h, long ncol, int nz, float dt, int layout, float* const fields[KIDMP_NFIELDS], float* nc,
+                    float* nwfa, float* nifa, const float* p, const float* w, const float* dz, const float* nwfa2d, float* ppt) {
+  if (!h) return 1;
+  if (ncol == 0) return 0;
+  // every check before anything is copied or launched: a refused call leaves every array as it was
+  if (ncol < 0) return fail(h, "step_aero: ncol=%ld", ncol);
+  if (!fields || !nc || !nwfa || !nifa || !p || !w || !dz) return fail(h, "step_aero: null pointer");
+  for (int q = 0; q < KIDMP_NFIELDS; ++q) if (!fields[q]) return fail(h, "step_aero: field %d is null", q);
+  if (nz < 2 || nz > 256) return fail(h, "step_aero: nz=%d outside [2,256]", nz);
+  if (!(dt > 0.f)) return fail(h, "step_aero: dt must be positive");
+  bool rates = h->d_rates || h->rates_on;
+  if (h->multi) for (kidmp_handle* c : h->multi->dev) rates = rates || c->d_rates || c->rates_on;
+  if (rates) return fail(h, "step_aero: the process-rate buffer is not available in an aerosol-aware step");
+  const AeroHost ae{nc, nwfa, nifa, w, nwfa2d};
+  return step_host(h, ncol, nz, dt, layout, fields, p, dz, nullptr, &ae, ppt, ncol);
 }
 
 int kidmp_set_rates_buffer(kidmp_handle* h, float* d_rates) {

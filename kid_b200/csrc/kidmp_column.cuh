@@ -514,6 +514,27 @@ __global__ void __launch_bounds__(128) k_scatter_host(StepArgs a, HostFields hf,
     for (int q = 0; q < KIDMP_NFIELDS; ++q) hf.f[q][ho] = a.f[q][o];
   }
 }
+// The same return path of an aerosol-aware step: the nine fields, then nc, nwfa, nifa (written by finish_level of the active
+// columns only, so an untouched column is unchanged in all twelve).  nwfa_row0: the surface emission (M:1001) added level 0 of
+// nwfa in every column after the step, so that row goes back for the untouched columns too.
+struct HostFieldsAero { float* f[KIDMP_NFIELDS + 3]; };
+__global__ void __launch_bounds__(128) k_scatter_host_aero(StepArgs a, HostFieldsAero hf, long hld, int nwfa_row0) {
+  const long col = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= a.ncol) return;
+  if (a.colflag[col] == -1) {
+    if (nwfa_row0) hf.f[KIDMP_NFIELDS + 1][col] = a.nwfa[col];
+    return;
+  }
+  const float* const src[KIDMP_NFIELDS + 3] = {a.f[0], a.f[1], a.f[2], a.f[3], a.f[4], a.f[5], a.f[6], a.f[7], a.f[8],
+                                               a.nc, a.nwfa, a.nifa};
+  const int nz = a.nz;
+#pragma unroll 2
+  for (int k = 0; k < nz; ++k) {
+    const long o = (long)k * a.ld + col, ho = (long)k * hld + col;
+#pragma unroll
+    for (int q = 0; q < KIDMP_NFIELDS + 3; ++q) hf.f[q][ho] = src[q][o];
+  }
+}
 
 // layout conversion between KiD's (k,i) arrays [col][nz] and the device layout [nz][ncol]
 __global__ void k_transpose(const float* __restrict__ src, float* __restrict__ dst, long ncol, int nz, int to_col_fastest) {

@@ -51,6 +51,7 @@ SYMBOLS = {
     "kidmp_step_device": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.POINTER(C.c_void_p), C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p]),
     "kidmp_step_device_aero": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.POINTER(C.c_void_p)] + [C.c_void_p] * 9),
+    "kidmp_step_aero": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.c_int, _fpp] + [_fp] * 8),
     "kidmp_step_nc": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.c_int, _fpp, _fp, _fp, _fp, _fp]),
     "kidmp_step_device_nc": (C.c_int, [C.c_void_p, C.c_long, C.c_int, C.c_float, C.POINTER(C.c_void_p)] + [C.c_void_p] * 5),
     "kidmp_set_rates_buffer": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -257,6 +258,27 @@ class Thompson:
             if np.shape(set_nc) != (ncol,):
                 raise ValueError("set_nc shape %r, expected (%d,)" % (np.shape(set_nc), ncol))
             self._ck(self._L.kidmp_step_nc(*args, _f32c(set_nc).ctypes.data_as(_fp), ppt.ctypes.data_as(_fp)))
+        return ppt
+
+    def step_aero(self, dt, state, aero, p, w, dz, layout="col_fastest", nwfa2d=None):
+        """kidmp_step_aero: the aerosol-aware step (is_aerosol_aware = .true.) on host arrays, in place.  state as in step;
+        aero: dict nc nwfa nifa of float32 arrays shaped like the fields, updated in place; w the same shape; nwfa2d: float32
+        (ncol,) surface emission or None.  Returns ppt[4, ncol]."""
+        lay = K_FASTEST if layout == "k_fastest" else COL_FASTEST
+        t = _f32c(state["t"])
+        ncol, nz = (t.shape if lay == K_FASTEST else t.shape[::-1])
+        for name, a in (("nc", aero["nc"]), ("nwfa", aero["nwfa"]), ("nifa", aero["nifa"]), ("w", w)):
+            if np.shape(a) != t.shape:
+                raise ValueError("%s shape %r, expected %r" % (name, np.shape(a), t.shape))
+        if nwfa2d is not None and np.shape(nwfa2d) != (ncol,):
+            raise ValueError("nwfa2d shape %r, expected (%d,)" % (np.shape(nwfa2d), ncol))
+        arrs = [_f32c(state[k]) for k in FIELDS]
+        ae = [_f32c(aero[k]) for k in ("nc", "nwfa", "nifa")]
+        P = lambda a: a.ctypes.data_as(_fp)
+        ppt = np.zeros((4, ncol), np.float32)
+        self._ck(self._L.kidmp_step_aero(self.h, ncol, nz, float(dt), lay, _ptrs(arrs), *[P(a) for a in ae], P(_f32c(p)), P(_f32c(w)),
+                                         P(np.ascontiguousarray(dz, np.float32)), P(_f32c(nwfa2d)) if nwfa2d is not None else None,
+                                         P(ppt)))
         return ppt
 
     def state_alloc(self, ncol, nz):
